@@ -11,6 +11,8 @@ CUDA events on the stream the kernel is launched on; `e2e` times the host-buffer
 (pb200_encrypt_batch: pinned host -> device, kernel, device -> host) by wall clock around the blocking call.
 Multi-GPU: units are independent, so each rank encrypts its own 2^16 units (weak scaling, no data-path
 collective); the time is the max over ranks.
+`--dump-outputs DIR` writes a fixed sample of the last timed step's ciphertexts (rank 0) to DIR/ciphertexts.npy, so that two
+builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -480,6 +482,19 @@ def leg_decrypt(cx, key, kd, g, n_bits, d_c, m_w, reps=2):
             "note": "m = L(c^lambda mod n^2) * mu mod n; round trip of the headline step's ciphertexts, every plaintext compared"}
 
 
+DUMP_ROWS = 8192
+
+
+def dump_ciphertexts(out_dir, c_w):
+    """DIR/ciphertexts.npy: DUMP_ROWS ciphertexts spread evenly over the batch (all of them when the batch is smaller), one row
+    per ciphertext in little-endian 32-bit limbs stored as float64, which holds every limb exactly (16 MiB at most, |n| = 4096)."""
+    import numpy as np
+    rows = np.unique(np.linspace(0, c_w.shape[0] - 1, min(DUMP_ROWS, c_w.shape[0])).astype(np.int64))
+    limbs = np.ascontiguousarray(c_w[rows], dtype="<u8").view("<u4")
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "ciphertexts.npy"), limbs.astype(np.float64))
+
+
 TALLY_TOTAL = 1 << 20
 TALLY_PARTS = 8            # the 2^20 ciphertexts are 8 fixed Philox streams, so the SET is the same for every GPU count
 
@@ -641,7 +656,13 @@ def main():
     ap.add_argument("--workload", default="encrypt", choices=["encrypt", "tally", "witness"],
                     help="encrypt: the BASELINE metric with every leg (default); tally: configs[2] alone; witness: the witness leg alone "
                          "at --n-bits / --units")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's ciphertexts to DIR/ciphertexts.npy (encrypt workload, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "encrypt"):
+        ap.error("--dump-outputs covers the encrypt workload of --impl ours")
     global N_BITS, METRIC
     N_BITS = args.n_bits
     METRIC = f"paillier_enc_per_s_n{N_BITS}"
@@ -707,6 +728,8 @@ def main():
     launches = lib.pb200_kernel_launches() - launches0
     (dev_ms,) = cx.max_over_ranks(sum(a.elapsed_time(b) for a, b in evs))
     value = world * units * args.steps / (dev_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_ciphertexts(args.dump_outputs, d_c.cpu().numpy().view(np.uint64))
 
     # ---- e2e: the host-buffer C-ABI call, pinned host memory, H2D + kernel + D2H inside the timed region
     import ctypes as C
