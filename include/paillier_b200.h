@@ -187,6 +187,28 @@ int pb200_key_set_private(pb200_key* key, const uint64_t* lambda_le, const uint6
 int pb200_decrypt_batch(pb200_key* key, const uint64_t* c_le, size_t count, uint64_t* m_out_le);
 int pb200_decrypt_batch_dev(pb200_key* key, const uint64_t* d_c_le, size_t count, uint64_t* d_m_out_le);
 
+/* ---- homomorphic scalar multiplication and the weighted tally -----------------------------------------------------------
+ * Multiplying a ciphertext by a plaintext: Dec(c^k mod n^2) = k * Dec(c) mod n, and prod c_i^(k_i) encrypts sum k_i m_i (weighted
+ * votes, "against" votes with k = n - 1, encrypted dot products with a plaintext vector).  Runs on the key's engine (block28: a
+ * fixed-window chain per ciphertext, as long as the longest scalar among the 32 or 64 ciphertexts of a CTA; simple64: LSB-first
+ * square-and-multiply); needs no private part and no per-key preparation.
+ *
+ * out_i = c_i^(k_i) mod n^2 (Dec(out_i) = k_i * Dec(c_i) mod n).  c: count * words_out words (any value, reduced mod n^2);
+ * k: count * PB200_WORDS(k_bits) words, 1 <= k_bits <= n_bits (a negative scalar -s is n - s); out: count * words_out, canonical.
+ * PB200_ERR_INVALID_ARG for null pointers, k_bits == 0 or k_bits > n_bits; PB200_ERR_RANGE (host variant) when some scalar has a
+ * bit at or above k_bits.  _dev: device pointers on the key's device, enqueued on the key's stream, no final synchronise, scalars
+ * are not range-checked (the host variant checks them against k_bits). */
+int pb200_scalar_mul_batch(pb200_key* key, const uint64_t* c_le, const uint64_t* k_le, uint32_t k_bits, size_t count, uint64_t* out_le);
+int pb200_scalar_mul_batch_dev(pb200_key* key, const uint64_t* d_c_le, const uint64_t* d_k_le, uint32_t k_bits, size_t count,
+                               uint64_t* d_out_le);
+/* prod c_i^(k_i) mod n^2 = Enc(sum k_i m_i); count == 0 gives 1 mod n^2.  Same arguments and checks as pb200_scalar_mul_batch;
+ * works in chunks of 2^18 ciphertexts (scalar products, then the tally's fold of each chunk, then the fold of the partials), so
+ * its temporary device memory is bounded (128 MB at |n| = 2048).  _dev: d_out receives words_out words on the device; enqueued
+ * on the key's stream, no final synchronise, scalars are not range-checked. */
+int pb200_tally_weighted(pb200_key* key, const uint64_t* c_le, const uint64_t* k_le, uint32_t k_bits, size_t count, uint64_t* out_le);
+int pb200_tally_weighted_dev(pb200_key* key, const uint64_t* d_c_le, const uint64_t* d_k_le, uint32_t k_bits, size_t count,
+                             uint64_t* d_out_le);
+
 /* ---- witness --------------------------------------------------------------------------------
  * Replaces: the witness generation inside BigUintChip::pow_mod_fixed_exp / mul_mod that
  * PaillierChip::encrypt drives (src/paillier.rs:51,55,57).  Every mul_mod(a, b, n^2) of the chain

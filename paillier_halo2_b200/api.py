@@ -350,6 +350,62 @@ class PaillierKey(CellMixin):
     def decrypt_dev(self, d_c: int, count: int, d_m: int) -> None:
         check(self._lib.pb200_decrypt_batch_dev(self._h, d_c, count, d_m), "pb200_decrypt_batch_dev")
 
+    # -- homomorphic scalar multiplication: Dec(c^k mod n^2) = k Dec(c) mod n, prod c_i^(k_i) = Enc(sum k_i m_i) --------------
+    def scalar_mul_words(self, c_w: np.ndarray, k_w: np.ndarray, k_bits: int) -> np.ndarray:
+        """c_w: (count, words_out) any values; k_w: (count, words(k_bits)) scalars below 2^k_bits -> (count, words_out) c^k mod n^2."""
+        c_w = np.ascontiguousarray(c_w, dtype="<u8").reshape(-1, self.words_out)
+        k_w = np.ascontiguousarray(k_w, dtype="<u8").reshape(-1, words(k_bits))
+        count = c_w.shape[0]
+        assert k_w.shape[0] == count
+        out = np.empty((count, self.words_out), dtype="<u8")
+        check(self._lib.pb200_scalar_mul_batch(self._h, _p(c_w), _p(k_w), k_bits, count, _p(out)), "pb200_scalar_mul_batch")
+        return out
+
+    def scalar_mul_dev(self, d_c: int, d_k: int, k_bits: int, count: int, d_out: int) -> None:
+        """Device-pointer variant (pb200_scalar_mul_batch_dev): enqueues on the key's stream, no synchronise, no range check."""
+        check(self._lib.pb200_scalar_mul_batch_dev(self._h, d_c, d_k, k_bits, count, d_out), "pb200_scalar_mul_batch_dev")
+
+    def _scalars(self, ks: Sequence[int]) -> Tuple[np.ndarray, int]:
+        """Scalars reduced mod n (a negative weight -s becomes n - s), their words and the declared width (largest bit length)."""
+        red = [int(k) % self.n for k in ks]
+        k_bits = max([1] + [k.bit_length() for k in red])
+        return ints_to_words(red, words(k_bits)), k_bits
+
+    def _ciphertexts(self, cs: Sequence[int], where: str) -> np.ndarray:
+        try:
+            return ints_to_words(cs, self.words_out)
+        except OverflowError:
+            raise Pb200Error(_lib.PB200_ERR_RANGE, where)
+
+    def scalar_mul(self, cs: Sequence[int], ks: Sequence[int]) -> List[int]:
+        """c_i^(k_i mod n) mod n^2 for every pair: the ciphertext of k_i * m_i mod n."""
+        assert len(cs) == len(ks)
+        if not len(cs):
+            return []
+        k_w, k_bits = self._scalars(ks)
+        return words_to_ints(self.scalar_mul_words(self._ciphertexts(cs, "scalar_mul"), k_w, k_bits))
+
+    def tally_weighted_words(self, c_w: np.ndarray, k_w: np.ndarray, k_bits: int) -> np.ndarray:
+        c_w = np.ascontiguousarray(c_w, dtype="<u8").reshape(-1, self.words_out)
+        k_w = np.ascontiguousarray(k_w, dtype="<u8").reshape(-1, words(k_bits))
+        count = c_w.shape[0]
+        assert k_w.shape[0] == count
+        out = np.empty(self.words_out, dtype="<u8")
+        check(self._lib.pb200_tally_weighted(self._h, _p(c_w) if count else None, _p(k_w) if count else None, k_bits, count, _p(out)),
+              "pb200_tally_weighted")
+        return out
+
+    def tally_weighted(self, cs: Sequence[int], ks: Sequence[int]) -> int:
+        """prod c_i^(k_i mod n) mod n^2: the ciphertext of sum k_i m_i mod n (weights may be negative)."""
+        assert len(cs) == len(ks)
+        k_w, k_bits = self._scalars(ks)
+        c_w = self._ciphertexts(cs, "tally_weighted") if len(cs) else np.empty((0, self.words_out), dtype="<u8")
+        return words_to_ints(self.tally_weighted_words(c_w, k_w, k_bits))[0]
+
+    def tally_weighted_dev(self, d_c: int, d_k: int, k_bits: int, count: int, d_out: int) -> None:
+        """Device-pointer variant (pb200_tally_weighted_dev): enqueues on the key's stream, no synchronise, no range check."""
+        check(self._lib.pb200_tally_weighted_dev(self._h, d_c, d_k, k_bits, count, d_out), "pb200_tally_weighted_dev")
+
     # -- witness ------------------------------------------------------------------------------
     def g_chain(self) -> List[Tuple[int, int]]:
         """Per-key records (q, rem) of the g-chain squarings, i < enc_bits."""

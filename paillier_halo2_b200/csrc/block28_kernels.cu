@@ -435,6 +435,81 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
     cta_end<C, ENG>(S);
 }
 
+// out = c^k mod n^2 with its own scalar k per lane: homomorphic scalar multiplication, Dec(c^k) = k Dec(c) mod n.  Fixed window of
+// w bits aligned to bit 0; the table x^0 .. x^(2^w - 1) lives in the CTA's scratch slot.  Every lane runs the same sequence of
+// multiplications (w squarings, then one multiplication by its own table entry; digit 0 multiplies by the stored 1), so control flow
+// never depends on the lane and the lanes of a CTA share every mulmod.  The chain is as long as the CTA's longest scalar.
+constexpr int SCALAR_MAXW = 5;
+static_assert((1 << SCALAR_MAXW) <= SCRATCH_ENTRIES, "the scalar window's table must fit the CTA's scratch slot");
+
+// smem per-lane value <- entry d (this lane's own) of a per-lane table in the [entry][blk][chunk][lane] layout
+template <class C>
+__device__ __forceinline__ void copy_from_global_lane(int4* buf, const int4* tab, int d, int role, int lane) {
+    const int4* e = tab + (size_t)d * C::VAL4;
+#pragma unroll
+    for (int c = 0; c < C::CH; c++) buf[(role * C::CH + c) * 32 + lane] = e[(role * C::CH + c) * 32 + lane];
+    __syncthreads();
+}
+
+template <class C, int ENG>
+__global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k_scalar(B28Dev K, const u64* __restrict__ c, const u64* __restrict__ k,
+                                                                       int k_words, int w, size_t count, u64* __restrict__ out,
+                                                                       int4* scratch, SlotPool pool) {
+    extern __shared__ int4 smem[];
+    __shared__ int s_slot[2];
+    __shared__ int s_bits;
+    constexpr int LG = View<C, ENG>::LG;
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = (threadIdx.x >> 5) % C::G, grp = (threadIdx.x >> 5) / C::G;      // grp: lane group (LG per CTA)
+    if (threadIdx.x == 0) { for (int g = 0; g < LG; g++) s_slot[g] = slot_acquire(pool); s_bits = 0; }
+    cta_begin<C, ENG>(S, smem, K);
+    const int slot = s_slot[grp];
+    size_t unit = (size_t)blockIdx.x * (32 * LG) + grp * 32 + lane;
+    const bool active = unit < count;
+    if (!active) unit = count - 1;
+    int4* tab = scratch + (size_t)slot * SCRATCH_ENTRIES * C::VAL4;
+    const u64* kw = k + unit * k_words;
+    // chain length: bits of the CTA's longest scalar (over both lane groups)
+    if (role == 0 && active) {
+        int b = 0;
+        for (int i = k_words - 1; i >= 0; i--) if (kw[i]) { b = 64 * i + 64 - __clzll((long long)kw[i]); break; }
+        if (b) atomicMax(&s_bits, b);
+    }
+    // table: tab[0] = 1, tab[1] = x, tab[e] = x^e (even e by squaring x^(e/2), odd e as x^(e-1) * x)
+    load_value<C>(S.V, c + unit * K.words_out, K.words_out, role, lane);
+    copy_to_global<C>(tab + C::VAL4, S.V, role, lane);
+    set_one<C>(S.B, role, lane);
+    copy_to_global<C>(tab, S.B, role, lane);
+    for (int e = 2; e < (1 << w); e++) {
+        if (e & 1) {
+            copy_from_global<C>(S.B, tab + C::VAL4, role, lane);
+            mm<C, false, ENG>(S, S.B, role, lane);
+        } else {
+            copy_from_global<C>(S.V, tab + (size_t)(e >> 1) * C::VAL4, role, lane);
+            mm<C, true, ENG>(S, nullptr, role, lane);
+        }
+        copy_to_global<C>(tab + (size_t)e * C::VAL4, S.V, role, lane);
+    }
+    __syncthreads();
+    const int nwin = (s_bits + w - 1) / w;
+    auto digit = [&](int i) -> int {
+        const int bit = i * w, wi = bit >> 6, sft = bit & 63;
+        u64 v = kw[wi] >> sft;
+        if (sft + w > 64 && wi + 1 < k_words) v |= kw[wi + 1] << (64 - sft);
+        return (int)(v & ((1u << w) - 1));
+    };
+    if (nwin == 0) set_one<C>(S.V, role, lane);                                        // every scalar of the CTA is 0
+    else copy_from_global_lane<C>(S.V, tab, digit(nwin - 1), role, lane);
+    for (int i = nwin - 2; i >= 0; i--) {
+        for (int s_ = 0; s_ < w; s_++) mm<C, true, ENG>(S, nullptr, role, lane);
+        copy_from_global_lane<C>(S.B, tab, digit(i), role, lane);
+        mm<C, false, ENG>(S, S.B, role, lane);
+    }
+    finalize<C, ENG>(S, K, out + unit * K.words_out, active, role, lane);
+    if (threadIdx.x == 0) for (int g = 0; g < LG; g++) slot_release(pool, s_slot[g]);
+    cta_end<C, ENG>(S);
+}
+
 // ---- tally: the N-ary fold of paillier_add_native (/root/reference/src/paillier.rs:94-97) in ONE launch per GPU -------------------
 // 1. every lane of every CTA folds a strided subset of the inputs (main loop, all lanes useful);
 // 2. the CTAs fold pairwise up a binary tree by "last arriver continues": a CTA stores its 32 lane values in its node slot, bumps
@@ -1059,12 +1134,14 @@ static Block28Key* create_cfg(const BigInt& n, const BigInt& g, uint32_t n_bits,
         CUK((cudaFuncSetAttribute(k_encrypt<C, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));
         CUK((cudaFuncSetAttribute(k_tally<C, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));
         CUK((cudaFuncSetAttribute(k_pow<C, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));
+        CUK((cudaFuncSetAttribute(k_scalar<C, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));
     }
     if constexpr (UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED) {
         CUK(u_image(std::integral_constant<int, 2>{}, &key->d_uconsts2));
         key->has_u2 = true;
         CUK((cudaFuncSetAttribute(k_encrypt<C, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 2>::SMEM_BYTES)));
         CUK((cudaFuncSetAttribute(k_pow<C, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 2>::SMEM_BYTES)));
+        CUK((cudaFuncSetAttribute(k_scalar<C, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 2>::SMEM_BYTES)));
     }
     block28_set_engine(key, -1);
     // sliding-window schedule for the exponent n
@@ -1189,6 +1266,41 @@ static cudaError_t pow_cfg(Block28Key* key, const u64* d_base, int base_words, s
     if (done) {}
     else if (key->eng >= 1) k_pow<C, 1><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, key->pow, d_base, base_words, count, d_out, key->d_scratch, pool);
     else k_pow<C, 0><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, key->pow, d_base, base_words, count, d_out, key->d_scratch, pool);
+    count_launch();
+    return cudaGetLastError();
+}
+
+// window width of the scalar chain for k_bits-bit scalars: the w <= SCALAR_MAXW with the fewest multiplications,
+// (2^w - 2) for the table + (ceil(k_bits / w) - 1) * (w + 1) for the chain (5 at 2048 bits, 3 at 32)
+static int scalar_window(uint32_t k_bits) {
+    int best = 1; uint64_t best_cost = ~0ull;
+    for (int w = 1; w <= SCALAR_MAXW; w++) {
+        const uint64_t cost = ((1u << w) - 2) + ((k_bits + w - 1) / w - 1) * (uint64_t)(w + 1);
+        if (cost < best_cost) { best = w; best_cost = cost; }
+    }
+    return best;
+}
+
+template <class C>
+static cudaError_t scalar_cfg(Block28Key* key, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out, cudaStream_t st) {
+    CUW(ensure_slots<C>(key, st));
+    CUW((cudaFuncSetAttribute(k_scalar<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
+    CUW((cudaFuncSetAttribute(k_scalar<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
+    const SlotPool pool{key->d_slot_masks, key->enc_per_sm};
+    const int kw = (int)((k_bits + 63) / 64), w = scalar_window(k_bits);
+    const size_t ctas = (count + 31) / 32;
+    bool done = false;
+    if constexpr (UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED) if (key->eng == 3 && key->has_u2) {
+        k_scalar<C, 3><<<(unsigned)((count + 63) / 64), 2 * C::THREADS, UL<C, 2>::SMEM_BYTES, st>>>(key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
+        done = true;
+    }
+    if constexpr (UL<C, 1>::SUPPORTED) if (!done && key->eng >= 2 && key->has_u) {
+        k_scalar<C, 2><<<(unsigned)ctas, C::THREADS, UL<C, 1>::SMEM_BYTES, st>>>(key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
+        done = true;
+    }
+    if (done) {}
+    else if (key->eng >= 1) k_scalar<C, 1><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
+    else k_scalar<C, 0><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
     count_launch();
     return cudaGetLastError();
 }
@@ -1436,6 +1548,14 @@ cudaError_t block28_pow(Block28Key* key, const u64* d_base, int base_words, size
     if (key->G == 8) return pow_cfg<Cfg2048>(key, d_base, base_words, count, d_out, st);
     if (key->BL == 14) return pow_cfg<Cfg3072>(key, d_base, base_words, count, d_out, st);
     return pow_cfg<Cfg4096>(key, d_base, base_words, count, d_out, st);
+}
+cudaError_t block28_scalar(Block28Key* key, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out, cudaStream_t st) {
+    if (!count) return cudaSuccess;
+    if (k_bits == 0) return cudaErrorInvalidValue;
+    if (key->G == 4) return scalar_cfg<Cfg1024>(key, d_c, d_k, k_bits, count, d_out, st);
+    if (key->G == 8) return scalar_cfg<Cfg2048>(key, d_c, d_k, k_bits, count, d_out, st);
+    if (key->BL == 14) return scalar_cfg<Cfg3072>(key, d_c, d_k, k_bits, count, d_out, st);
+    return scalar_cfg<Cfg4096>(key, d_c, d_k, k_bits, count, d_out, st);
 }
 
 static cudaError_t tally_dispatch(Block28Key* key, const u64* d_c, size_t count, u64* d_out, bool collective, cudaStream_t st) {

@@ -69,6 +69,7 @@ struct pb200_key {
     std::string fast_why;
     int engine = 0;                 // 0 auto, 1 simple64, 2 block28, 3 block28t, 4 block28u, 5 block28u2
     DevBuf in_a, in_b, out_a, out_b, scratch, offs;
+    DevBuf wt_chunk, wt_part;               // weighted tally: one chunk's scalar products, the per-chunk partial products
     std::string engine_name;
     // K4 cell expansion: per lookup_bits layout + device constants (n^2 limbs, word_max, q_acc, mod_acc), refresh spill vector
     struct CellCtx { CellLayout Y; u64* d_consts = nullptr; int* d_inc = nullptr; u64* d_mtab = nullptr; int n_out = 0; int n2_cells = 0; };
@@ -182,6 +183,7 @@ void pb200_key_destroy(pb200_key* k) {
     if (k->d_simple_n) cudaFree(k->d_simple_n);
     if (k->d_lambda) cudaFree(k->d_lambda);
     k->in_a.release(); k->in_b.release(); k->out_a.release(); k->out_b.release(); k->scratch.release(); k->offs.release();
+    k->wt_chunk.release(); k->wt_part.release();
     k->cin_a.release(); k->cin_b.release(); k->cin_q.release(); k->cin_r.release();
     if (k->pipe.ready) {
         if (k->pipe.copy) { cudaStreamSynchronize(k->pipe.copy); cudaStreamDestroy(k->pipe.copy); }
@@ -595,7 +597,7 @@ int pb200_decrypt_batch_dev(pb200_key* k, const uint64_t* d_c, size_t count, uin
     CU(k->scratch.reserve(count * k->words_out * sizeof(u64)));
     u64* d_x = (u64*)k->scratch.p;                               // x = c^lambda mod n^2
     if (use_fast(k)) CU(block28_pow(k->fast, (const u64*)d_c, (int)k->words_out, count, d_x, k->stream));
-    else CU(simple_pow(k->d_simple, (const u64*)d_c, (int)k->words_out, k->d_lambda, k->lambda_bits, count, d_x, k->d_flags, k->stream));
+    else CU(simple_pow(k->d_simple, (const u64*)d_c, (int)k->words_out, k->d_lambda, k->lambda_bits, 0, count, d_x, k->d_flags, k->stream));
     CU(simple_lfunc(k->d_simple_n, d_x, count, (u64*)d_m, k->d_flags, k->stream));
     return PB200_OK;
 } PB200_CATCH
@@ -612,6 +614,81 @@ int pb200_decrypt_batch(pb200_key* k, const uint64_t* c, size_t count, uint64_t*
     int rc = pb200_decrypt_batch_dev(k, (const uint64_t*)k->in_a.p, count, (uint64_t*)k->out_a.p);
     if (rc) return rc;
     CU(cudaMemcpyAsync(m_out, k->out_a.p, bout, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
+} PB200_CATCH
+
+// ---- homomorphic scalar multiplication and the weighted tally --------------------------------------------------------------
+static bool scalar_args_ok(const pb200_key* k, uint32_t k_bits) { return k && k_bits != 0 && k_bits <= k->n_bits; }
+static int check_scalars(const uint64_t* ks, uint32_t k_bits, size_t count) {
+    const uint32_t kw = PB200_WORDS(k_bits);
+    for (size_t u = 0; u < count; u++) if (!fits(ks + u * kw, kw, k_bits)) return PB200_ERR_RANGE;
+    return PB200_OK;
+}
+static int scalar_dev_impl(pb200_key* k, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out) {
+    if (!count) return PB200_OK;
+    if (use_fast(k)) CU(block28_scalar(k->fast, d_c, d_k, k_bits, count, d_out, k->stream));
+    else CU(simple_pow(k->d_simple, d_c, (int)k->words_out, d_k, (int)k_bits, (int)PB200_WORDS(k_bits), count, d_out, k->d_flags, k->stream));
+    return PB200_OK;
+}
+// chunks of at most 2^18 units: scalar products into wt_chunk, their tally into one slot of wt_part, then the tally of the partials
+// (128 MB of temporary memory at |n| = 2048 whatever the count)
+static const size_t WT_CHUNK = (size_t)1 << 18;
+static int tally_weighted_dev_impl(pb200_key* k, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out) {
+    if (!count) return tally_dev_impl(k, nullptr, 0, (uint64_t*)d_out, false);
+    const size_t wo = k->words_out, kw = PB200_WORDS(k_bits), chunks = (count + WT_CHUNK - 1) / WT_CHUNK;
+    CU(k->wt_chunk.reserve((count < WT_CHUNK ? count : WT_CHUNK) * wo * sizeof(u64)));
+    if (chunks > 1) CU(k->wt_part.reserve(chunks * wo * sizeof(u64)));
+    u64* prod = (u64*)k->wt_chunk.p;
+    for (size_t i = 0; i < chunks; i++) {
+        const size_t u0 = i * WT_CHUNK, n = count - u0 < WT_CHUNK ? count - u0 : WT_CHUNK;
+        int rc = scalar_dev_impl(k, d_c + u0 * wo, d_k + u0 * kw, k_bits, n, prod); if (rc) return rc;
+        u64* dst = chunks > 1 ? (u64*)k->wt_part.p + i * wo : d_out;                 // one chunk: its tally is the result
+        rc = tally_dev_impl(k, (const uint64_t*)prod, n, (uint64_t*)dst, false); if (rc) return rc;
+    }
+    if (chunks > 1) return tally_dev_impl(k, (const uint64_t*)k->wt_part.p, chunks, (uint64_t*)d_out, false);
+    return PB200_OK;
+}
+
+int pb200_scalar_mul_batch_dev(pb200_key* k, const uint64_t* d_c, const uint64_t* d_k, uint32_t k_bits, size_t count, uint64_t* d_out) try {
+    if (!scalar_args_ok(k, k_bits) || (count && (!d_c || !d_k || !d_out))) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    USE_DEVICE(k);
+    return scalar_dev_impl(k, (const u64*)d_c, (const u64*)d_k, k_bits, count, (u64*)d_out);
+} PB200_CATCH
+int pb200_scalar_mul_batch(pb200_key* k, const uint64_t* c, const uint64_t* ks, uint32_t k_bits, size_t count, uint64_t* out) try {
+    if (!scalar_args_ok(k, k_bits) || (count && (!c || !ks || !out))) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    int rc = check_scalars(ks, k_bits, count); if (rc) return rc;
+    USE_DEVICE(k);
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bc = count * k->words_out * sizeof(u64), bk = count * PB200_WORDS(k_bits) * sizeof(u64);
+    CU(k->in_a.reserve(bc)); CU(k->in_b.reserve(bk)); CU(k->out_a.reserve(bc));
+    CU(cudaMemcpyAsync(k->in_a.p, c, bc, cudaMemcpyHostToDevice, k->stream));
+    CU(cudaMemcpyAsync(k->in_b.p, ks, bk, cudaMemcpyHostToDevice, k->stream));
+    rc = scalar_dev_impl(k, (const u64*)k->in_a.p, (const u64*)k->in_b.p, k_bits, count, (u64*)k->out_a.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out, k->out_a.p, bc, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
+} PB200_CATCH
+int pb200_tally_weighted_dev(pb200_key* k, const uint64_t* d_c, const uint64_t* d_k, uint32_t k_bits, size_t count, uint64_t* d_out) try {
+    if (!scalar_args_ok(k, k_bits) || !d_out || (count && (!d_c || !d_k))) return PB200_ERR_INVALID_ARG;
+    USE_DEVICE(k);
+    return tally_weighted_dev_impl(k, (const u64*)d_c, (const u64*)d_k, k_bits, count, (u64*)d_out);
+} PB200_CATCH
+int pb200_tally_weighted(pb200_key* k, const uint64_t* c, const uint64_t* ks, uint32_t k_bits, size_t count, uint64_t* out) try {
+    if (!scalar_args_ok(k, k_bits) || !out || (count && (!c || !ks))) return PB200_ERR_INVALID_ARG;
+    int rc = check_scalars(ks, k_bits, count); if (rc) return rc;
+    USE_DEVICE(k);
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bc = count * k->words_out * sizeof(u64), bk = count * PB200_WORDS(k_bits) * sizeof(u64), bout = k->words_out * sizeof(u64);
+    CU(k->in_a.reserve(bc ? bc : 8)); CU(k->in_b.reserve(bk ? bk : 8)); CU(k->out_b.reserve(bout));
+    if (bc) CU(cudaMemcpyAsync(k->in_a.p, c, bc, cudaMemcpyHostToDevice, k->stream));
+    if (bk) CU(cudaMemcpyAsync(k->in_b.p, ks, bk, cudaMemcpyHostToDevice, k->stream));
+    rc = tally_weighted_dev_impl(k, (const u64*)k->in_a.p, (const u64*)k->in_b.p, k_bits, count, (u64*)k->out_b.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out, k->out_b.p, bout, cudaMemcpyDeviceToHost, k->stream));
     CU(cudaStreamSynchronize(k->stream));
     return take_flags(k);
 } PB200_CATCH

@@ -28,9 +28,11 @@ cudaError_t simple_tally(const SimpleConsts* dK, int k, const u64* d_c, size_t c
 cudaError_t repack_limbs(const u64* d_vals, size_t count, int words_per_value, int value_bits, int limb_bits,
                          u64* d_out, cudaStream_t st);
 // decryption pieces on the simple engine: x = base^e mod n^2 (exponent words on the device), and m = (x - 1) / n * mu mod n with
-// the constants of the modulus n (mu in their g slot); flag bit 3 when x != 1 (mod n)
-cudaError_t simple_pow(const SimpleConsts* dK, const u64* d_base, int base_words, const u64* d_e, int e_bits, size_t count, u64* d_out,
-                       int* d_flags, cudaStream_t st);
+// the constants of the modulus n (mu in their g slot); flag bit 3 when x != 1 (mod n).  e_stride = 0: one exponent for every unit
+// (decryption's lambda); e_stride > 0: unit u's exponent starts at word u * e_stride, and the base is reduced mod n^2 first (scalar
+// multiplication accepts any words_out-word value)
+cudaError_t simple_pow(const SimpleConsts* dK, const u64* d_base, int base_words, const u64* d_e, int e_bits, int e_stride, size_t count,
+                       u64* d_out, int* d_flags, cudaStream_t st);
 cudaError_t simple_lfunc(const SimpleConsts* dKn, const u64* d_x, size_t count, u64* d_m, int* d_flags, cudaStream_t st);
 
 // ---- block28 engine (block28_kernels.cu) ----------------------------------------------------
@@ -52,6 +54,9 @@ cudaError_t block28_tally(Block28Key*, const u64* d_c, size_t count, u64* d_out,
 // out = base^e mod n^2 for a per-key exponent e (sliding-window schedule built by block28_pow_prepare): the decryption's c^lambda
 cudaError_t block28_pow_prepare(Block28Key*, const BigInt& e, cudaStream_t st);
 cudaError_t block28_pow(Block28Key*, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st);
+// out_i = c_i^(k_i) mod n^2 with a scalar per unit (PB200_WORDS(k_bits) words each; c_i: words_out words, any value): fixed-window
+// chain per lane, window width chosen from k_bits; no per-key preparation
+cudaError_t block28_scalar(Block28Key*, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out, cudaStream_t st);
 // multi-GPU tally: one launch per GPU, partials exchanged through peer-mapped mailboxes inside the kernel (collective call)
 cudaError_t block28_tally_peer(Block28Key*, const u64* d_c, size_t count, u64* d_out, cudaStream_t st);
 cudaError_t block28_mailbox(Block28Key*, u64** d_mail, cudaStream_t st);

@@ -129,9 +129,12 @@ __global__ void k_simple_tally_final(const SimpleConsts* __restrict__ K, const u
 
 // ---- decryption (SURVEY.md 8f-4; the reference's README.md:5-22 states it, its code never implements it) ------------------------
 // x = base^e mod n^2, LSB-first square-and-multiply, exponent words from device memory: the always-available pow for keys the
-// block engine does not serve
+// block engine does not serve.  e_stride = 0: one exponent for all units (decryption); else unit u's own exponent at u * e_stride
+// words, and the base is reduced first (scalar multiplication takes any words_out-word value; squaring an unreduced one would
+// overflow the Barrett input)
 __global__ void __launch_bounds__(32) k_simple_pow(const SimpleConsts* __restrict__ K, const u64* __restrict__ base, int base_words,
-                                                   const u64* __restrict__ e, int e_bits, size_t count, u64* __restrict__ out, int* flags) {
+                                                   const u64* __restrict__ e, int e_bits, int e_stride, size_t count, u64* __restrict__ out,
+                                                   int* flags) {
     const size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (u >= count) return;
     const int k = K->k;
@@ -139,6 +142,11 @@ __global__ void __launch_bounds__(32) k_simple_pow(const SimpleConsts* __restric
     int bad = 0;
     set_one(acc, k);
     load_ext(sq, base + u * base_words, base_words, k);
+    if (e_stride) {
+        e += u * (size_t)e_stride;
+        bad |= mulmod_simple(K, q, t, sq, acc);
+        for (int j = 0; j < k; j++) sq[j] = t[j];
+    }
     for (int i = 0; i < e_bits; i++) {
         if (bit_at(e, i)) { bad |= mulmod_simple(K, q, t, acc, sq); for (int j = 0; j < k; j++) acc[j] = t[j]; }
         if (i + 1 < e_bits) { bad |= mulmod_simple(K, q, t, sq, sq); for (int j = 0; j < k; j++) sq[j] = t[j]; }
@@ -219,10 +227,11 @@ cudaError_t simple_tally(const SimpleConsts* dK, int k, const u64* d_c, size_t c
     k_simple_tally_final<<<1, 1, 0, st>>>(dK, p2, T2, d_out, d_flags); count_launch();
     return cudaGetLastError();
 }
-cudaError_t simple_pow(const SimpleConsts* dK, const u64* d_base, int base_words, const u64* d_e, int e_bits, size_t count, u64* d_out,
-                       int* d_flags, cudaStream_t st) {
+cudaError_t simple_pow(const SimpleConsts* dK, const u64* d_base, int base_words, const u64* d_e, int e_bits, int e_stride, size_t count,
+                       u64* d_out, int* d_flags, cudaStream_t st) {
     if (!count) return cudaSuccess;
-    k_simple_pow<<<(unsigned)((count + 31) / 32), 32, 0, st>>>(dK, d_base, base_words, d_e, e_bits, count, d_out, d_flags); count_launch();
+    k_simple_pow<<<(unsigned)((count + 31) / 32), 32, 0, st>>>(dK, d_base, base_words, d_e, e_bits, e_stride, count, d_out, d_flags);
+    count_launch();
     return cudaGetLastError();
 }
 cudaError_t simple_lfunc(const SimpleConsts* dKn, const u64* d_x, size_t count, u64* d_m, int* d_flags, cudaStream_t st) {

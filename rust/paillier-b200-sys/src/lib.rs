@@ -107,6 +107,11 @@ extern "C" {
     pub fn pb200_decrypt_batch(key: *mut pb200_key, c_le: *const u64, count: usize, m_out_le: *mut u64) -> c_int;
     pub fn pb200_decrypt_batch_dev(key: *mut pb200_key, d_c_le: *const u64, count: usize, d_m_out_le: *mut u64) -> c_int;
 
+    pub fn pb200_scalar_mul_batch(key: *mut pb200_key, c_le: *const u64, k_le: *const u64, k_bits: u32, count: usize, out_le: *mut u64) -> c_int;
+    pub fn pb200_scalar_mul_batch_dev(key: *mut pb200_key, d_c_le: *const u64, d_k_le: *const u64, k_bits: u32, count: usize, d_out_le: *mut u64) -> c_int;
+    pub fn pb200_tally_weighted(key: *mut pb200_key, c_le: *const u64, k_le: *const u64, k_bits: u32, count: usize, out_le: *mut u64) -> c_int;
+    pub fn pb200_tally_weighted_dev(key: *mut pb200_key, d_c_le: *const u64, d_k_le: *const u64, k_bits: u32, count: usize, d_out_le: *mut u64) -> c_int;
+
     pub fn pb200_encrypt_witness_batch(key: *mut pb200_key, m_le: *const u64, r_le: *const u64, count: usize, c_out_le: *mut u64,
                                        max_chunk_units: usize, sink: pb200_witness_sink_fn, user: *mut c_void) -> c_int;
     pub fn pb200_witness_records_for(key: *const pb200_key, m_le: *const u64) -> u64;
@@ -192,6 +197,29 @@ impl Key {
         }
         let mut out = vec![0u64; wo];
         let rc = unsafe { pb200_tally(self.raw, c.as_ptr(), c.len() / wo, out.as_mut_ptr()) };
+        if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// homomorphic scalar multiplication: `c` holds `count * words_out` words, `k` `count * ceil(k_bits / 64)` words (scalars below
+    /// 2^k_bits, 1 <= k_bits <= n_bits; a negative scalar -s is n - s); returns c_i^(k_i) mod n^2, whose plaintext is k_i * m_i mod n
+    pub fn scalar_mul_batch(&mut self, c: &[u64], k: &[u64], k_bits: u32) -> Result<Vec<u64>, i32> {
+        let (wo, kw) = (self.words_out(), ((k_bits as usize) + 63) / 64);
+        if wo == 0 || kw == 0 || c.len() % wo != 0 || k.len() != c.len() / wo * kw {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let mut out = vec![0u64; c.len()];
+        let rc = unsafe { pb200_scalar_mul_batch(self.raw, c.as_ptr(), k.as_ptr(), k_bits, c.len() / wo, out.as_mut_ptr()) };
+        if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// weighted tally: prod c_i^(k_i) mod n^2, the ciphertext of sum k_i * m_i mod n (same layout of `c` and `k` as scalar_mul_batch)
+    pub fn tally_weighted(&mut self, c: &[u64], k: &[u64], k_bits: u32) -> Result<Vec<u64>, i32> {
+        let (wo, kw) = (self.words_out(), ((k_bits as usize) + 63) / 64);
+        if wo == 0 || kw == 0 || c.len() % wo != 0 || k.len() != c.len() / wo * kw {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let mut out = vec![0u64; wo];
+        let rc = unsafe { pb200_tally_weighted(self.raw, c.as_ptr(), k.as_ptr(), k_bits, c.len() / wo, out.as_mut_ptr()) };
         if rc == PB200_OK { Ok(out) } else { Err(rc) }
     }
 }
