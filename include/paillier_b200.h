@@ -209,6 +209,32 @@ int pb200_tally_weighted(pb200_key* key, const uint64_t* c_le, const uint64_t* k
 int pb200_tally_weighted_dev(pb200_key* key, const uint64_t* d_c_le, const uint64_t* d_k_le, uint32_t k_bits, size_t count,
                              uint64_t* d_out_le);
 
+/* ---- encrypted matrix-vector product with a signed plaintext matrix ------------------------------------------------------
+ * Enc(W m) from Enc(m): private scoring with a linear model, multi-question ballots, PIR-style selection.  On a block28 engine a
+ * bucket (Pippenger) multi-exponentiation shared by all the ciphertexts of a row (about ceil(k_bits / c) multiplications per
+ * ciphertext and row, c <= 16), else per row and sign the weighted tally's chains (the "chain" method; simple64 keys always).
+ *
+ * out_r = P_r * N_r^(n-1) mod n^2 for r < rows, where
+ *   P_r = prod_{i: w_ri > 0} c_i^|w_ri| mod n^2,   N_r = prod_{i: w_ri < 0} c_i^|w_ri| mod n^2   (empty product = 1)
+ * so that Dec(out_r) = sum_i w_ri * Dec(c_i) mod n.  c: count * words_out words (any value, reduced mod n^2);
+ * w_mag: rows * count * PB200_WORDS(k_bits) words, row-major (entry (r, i) at (r * count + i) * PB200_WORDS(k_bits));
+ * w_neg: nullable, rows * count bytes, non-zero = that weight is negative;  out: rows * words_out words, canonical.
+ * A row without negative weights equals pb200_tally_weighted of that row bit for bit.  count == 0 gives 1 for every row, rows == 0
+ * does nothing.  PB200_ERR_INVALID_ARG for null pointers where data is needed, k_bits == 0 or k_bits > n_bits; PB200_ERR_RANGE
+ * (host variant) when a magnitude has a bit at or above k_bits.  Temporary device memory stays within 3 * 2^18 * 8 * words_out bytes
+ * (384 MB at |n| = 2048) whatever rows, count and k_bits (work proceeds in passes; the host variant's staged inputs come on top).
+ * _dev: device pointers, enqueued on the key's stream, no final synchronise, magnitudes are not range-checked; the sign step runs
+ * whenever d_w_neg is non-null.  The first call with negative weights prepares copies of n - 1 on the device (synchronises once). */
+int pb200_matvec(pb200_key* key, const uint64_t* c_le, size_t count, const uint64_t* w_mag_le, const uint8_t* w_neg,
+                 uint32_t k_bits, size_t rows, uint64_t* out_le);
+int pb200_matvec_dev(pb200_key* key, const uint64_t* d_c_le, size_t count, const uint64_t* d_w_mag_le, const uint8_t* d_w_neg,
+                     uint32_t k_bits, size_t rows, uint64_t* d_out_le);
+/* host only, no device needed: the plan pb200_matvec would use for a key of n_bits on a GPU of `sms` SMs running a block28 engine
+ * (the same planner; PB200_MATVEC_METHOD and PB200_MATVEC_PASS_ENTRIES apply).  out11: method (0 chain, 1 bucket), window width c,
+ * windows J, passes, bucket segments per window, then upper bounds for dense weights of the multiplications of accumulation,
+ * reduction, Horner and the sign step, the longest sequential chain of multiplications, and the temporary device bytes. */
+int pb200_matvec_plan(uint32_t n_bits, int sms, size_t rows, size_t count, uint32_t k_bits, int has_neg, uint64_t* out11);
+
 /* ---- witness --------------------------------------------------------------------------------
  * Replaces: the witness generation inside BigUintChip::pow_mod_fixed_exp / mul_mod that
  * PaillierChip::encrypt drives (src/paillier.rs:51,55,57).  Every mul_mod(a, b, n^2) of the chain

@@ -84,6 +84,9 @@ SYMBOLS = {
     "pb200_scalar_mul_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
     "pb200_tally_weighted": (C.c_int, [C.c_void_p, u64p, u64p, C.c_uint32, C.c_size_t, u64p]),
     "pb200_tally_weighted_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
+    "pb200_matvec": (C.c_int, [C.c_void_p, u64p, C.c_size_t, u64p, C.c_void_p, C.c_uint32, C.c_size_t, u64p]),
+    "pb200_matvec_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
+    "pb200_matvec_plan": (C.c_int, [C.c_uint32, C.c_int, C.c_size_t, C.c_size_t, C.c_uint32, C.c_int, u64p]),
     "pb200_encrypt_witness_batch": (C.c_int, [C.c_void_p, u64p, u64p, C.c_size_t, u64p, C.c_size_t, SINK_FN, C.c_void_p]),
     "pb200_witness_records_for": (C.c_uint64, [C.c_void_p, u64p]),
     "pb200_encrypt_witness_digest": (C.c_int, [C.c_void_p, u64p, u64p, C.c_size_t, u64p, u64p]),

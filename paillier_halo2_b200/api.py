@@ -406,6 +406,37 @@ class PaillierKey(CellMixin):
         """Device-pointer variant (pb200_tally_weighted_dev): enqueues on the key's stream, no synchronise, no range check."""
         check(self._lib.pb200_tally_weighted_dev(self._h, d_c, d_k, k_bits, count, d_out), "pb200_tally_weighted_dev")
 
+    # -- encrypted matrix-vector product: row r of the result encrypts sum_i W[r, i] * m_i mod n --------------------------------
+    def matvec_words(self, c_w: np.ndarray, w_mag_w: np.ndarray, w_neg: Optional[np.ndarray], k_bits: int) -> np.ndarray:
+        """c_w: (count, words_out) any values; w_mag_w: (rows, count, words(k_bits)) magnitudes below 2^k_bits; w_neg: None or
+        (rows, count), non-zero where the weight is negative -> (rows, words_out) canonical ciphertexts (pb200_matvec)."""
+        c_w = np.ascontiguousarray(c_w, dtype="<u8").reshape(-1, self.words_out)
+        count, kw = c_w.shape[0], words(k_bits)
+        w_mag_w = np.ascontiguousarray(w_mag_w, dtype="<u8")
+        rows = w_mag_w.shape[0]
+        assert w_mag_w.size == rows * count * kw
+        neg = None
+        if w_neg is not None:
+            neg = np.ascontiguousarray(w_neg, dtype=np.uint8)
+            assert neg.size == rows * count
+        out = np.empty((rows, self.words_out), dtype="<u8")
+        check(self._lib.pb200_matvec(self._h, _p(c_w) if count else None, count, _p(w_mag_w) if w_mag_w.size else None,
+                                     neg.ctypes.data_as(C.c_void_p) if neg is not None and neg.size else None, k_bits, rows,
+                                     _p(out) if rows else None), "pb200_matvec")
+        return out
+
+    def matvec_dev(self, d_c: int, count: int, d_w_mag: int, d_w_neg: Optional[int], k_bits: int, rows: int, d_out: int) -> None:
+        """Device-pointer variant (pb200_matvec_dev): enqueues on the key's stream, no synchronise, no range check; the sign step
+        runs whenever d_w_neg is given."""
+        check(self._lib.pb200_matvec_dev(self._h, d_c, count, d_w_mag, d_w_neg or None, k_bits, rows, d_out), "pb200_matvec_dev")
+
+    def matvec(self, cs: Sequence[int], W) -> List[int]:
+        """Enc(W m): W is a sequence of rows of Python ints (any sign) or a 2-D numpy integer array with one column per ciphertext.
+        Row r of the result is prod c_i^|W[r, i]| over the positive weights times (the same over the negative ones)^(n - 1)."""
+        mag, neg, k_bits = matvec_weights(W, len(cs))
+        c_w = self._ciphertexts(cs, "matvec") if len(cs) else np.empty((0, self.words_out), dtype="<u8")
+        return words_to_ints(self.matvec_words(c_w, mag, neg, k_bits)) if mag.shape[0] else []
+
     # -- witness ------------------------------------------------------------------------------
     def g_chain(self) -> List[Tuple[int, int]]:
         """Per-key records (q, rem) of the g-chain squarings, i < enc_bits."""
@@ -465,6 +496,49 @@ class PaillierKey(CellMixin):
         out = np.empty((len(vals), nl, 2), dtype="<u8")
         check(self._lib.pb200_repack_limbs(self._h, _p(v_w), len(vals), value_bits, limb_bits, _p(out)), "pb200_repack_limbs")
         return [[int(out[i, j, 0]) | (int(out[i, j, 1]) << 64) for j in range(nl)] for i in range(len(vals))]
+
+
+def matvec_weights(W, count: int) -> Tuple[np.ndarray, Optional[np.ndarray], int]:
+    """Weights -> (magnitude words (rows, count, words(k_bits)), signs (rows, count) uint8 or None, k_bits = largest bit length, >= 1).
+    A numpy integer array is converted without a Python loop; anything else is taken as rows of Python ints."""
+    if isinstance(W, np.ndarray) and W.dtype.kind in "iu":
+        if W.ndim != 2 or W.shape[1] != count:
+            raise ValueError("W must have one column per ciphertext")
+        if W.dtype.kind == "u":
+            mag, neg = W.astype(np.uint64), None
+        else:
+            w64 = W.astype(np.int64)
+            mag = np.abs(w64).astype(np.uint64)                   # |int64 min| wraps to 2^63 as uint64: exact
+            neg = (w64 < 0).astype(np.uint8)
+            if not neg.any():
+                neg = None
+        top = int(mag.max()) if mag.size else 0
+        return np.ascontiguousarray(mag.reshape(W.shape[0], count, 1), dtype="<u8"), neg, max(1, top.bit_length())
+    rows = [list(r) for r in W]
+    if any(len(r) != count for r in rows):
+        raise ValueError("every row of W needs one weight per ciphertext")
+    flat = [int(v) for r in rows for v in r]
+    k_bits = max([1] + [abs(v).bit_length() for v in flat])
+    mag = ints_to_words([abs(v) for v in flat], words(k_bits)).reshape(len(rows), count, words(k_bits))
+    neg = np.array([v < 0 for v in flat], dtype=np.uint8).reshape(len(rows), count) if any(v < 0 for v in flat) else None
+    return mag, neg, k_bits
+
+
+MATVEC_PLAN_FIELDS = ("method", "c", "windows", "passes", "segments", "acc_mulmods", "reduce_mulmods", "horner_mulmods", "sign_mulmods",
+                      "chain", "temp_bytes")
+
+
+def matvec_budget(n_bits: int) -> int:
+    """Temporary device memory a matvec stays within (pb200_matvec): 3 * 2^18 ciphertexts of words_out words."""
+    return 3 * (1 << 18) * 8 * words(2 * n_bits)
+
+
+def matvec_plan(n_bits: int, sms: int, rows: int, count: int, k_bits: int, has_neg: bool) -> dict:
+    """The plan pb200_matvec would use on a block28 engine (pb200_matvec_plan, host only): method 0 chain / 1 bucket, window width c,
+    windows, passes, bucket segments per window, dense-weight mulmod upper bounds, longest sequential chain, temporary bytes."""
+    out = np.zeros(11, dtype="<u8")
+    check(_lib.load().pb200_matvec_plan(n_bits, sms, rows, count, k_bits, int(bool(has_neg)), _p(out)), "pb200_matvec_plan")
+    return dict(zip(MATVEC_PLAN_FIELDS, (int(v) for v in out)))
 
 
 def chip_order(m: int, n: int, g_chain: Sequence[Tuple[int, int]], unit_records: Sequence[Tuple[int, int]]):

@@ -15,6 +15,7 @@
 #include <vector>
 #include <cstring>
 #include <cstdlib>
+#include <algorithm>
 
 namespace pb200 {
 using namespace b28;
@@ -645,6 +646,217 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_tally(B28D
     fold_lanes<C, ENG>(S, width, role, lane);
     finalize<C, ENG>(S, K, out, lane == 0, role, lane);
     cta_end<C, ENG>(S);
+}
+
+// ---- matvec: bucket (Pippenger) multi-exponentiation, DESIGN.md §9b ------------------------------------------------------------
+// The engine kernels below run the tally's CTA shape (32 lanes, ENG 0 / 1 / 4).  Values between them are either canonical words
+// (words_out u64, read with load_value, written by finalize) or lazy digits (ENTRY4 int4 per value, gather_entry / scatter_entry).
+template <class C>
+__device__ __forceinline__ void scatter_one(int4* entry, int role) {
+#pragma unroll
+    for (int c = 0; c < C::CH; c++) entry[role * C::CH + c] = make_int4(role == 0 && c == 0 ? 1 : 0, 0, 0, 0);
+}
+
+// Reduce-by-key of a key-sorted list: out[key] = product of the values with that key (lazy digits).  Lane l takes the slice
+// [l * ls, (l + 1) * ls) and multiplies every value of it into its accumulator, restarting at 1 on a key change (one multiplication
+// per entry on every lane, padding multiplies by 1).  Runs that start and end inside the slice are complete and stored; the first and
+// the last run of a slice may continue into a neighbour, so they go to the carry list as pieces 2l and 2l + 1 (a slice of one run
+// emits it and a 1), which is again key-sorted and is folded by the next launch.  A launch whose list fits one slice stores every run.
+// Level 0 gathers its values from words (src + idx[t] * src_words), later levels from the lazy pieces of the previous one.
+// n: *d_n entries when d_n is set (counted on the device), else n_fixed; *d_n_next: entries of the carry list (0 when complete).
+template <class C, int ENG>
+__global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_bucket_fold(B28Dev K, const unsigned* __restrict__ keys, const unsigned* __restrict__ idx,
+                                                                            const u64* __restrict__ src, int src_words, const int4* __restrict__ src_lazy,
+                                                                            const unsigned* __restrict__ d_n, size_t n_fixed, int ls, int4* __restrict__ out,
+                                                                            unsigned* __restrict__ keys_next, int4* __restrict__ vals_next, unsigned* __restrict__ d_n_next) {
+    extern __shared__ int4 smem[];
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
+    const size_t n = d_n ? *d_n : n_fixed;
+    const size_t lanes = (n + ls - 1) / ls;
+    const bool last = lanes <= 1;
+    if (blockIdx.x == 0 && threadIdx.x == 0) *d_n_next = last ? 0u : (unsigned)(2 * lanes);
+    if ((size_t)blockIdx.x * 32 >= lanes) return;                                   // the whole CTA is past the list
+    cta_begin<C, ENG>(S, smem, K);
+    const size_t l = (size_t)blockIdx.x * 32 + lane, a = l * ls;
+    const bool active = l < lanes;
+    unsigned cur = active ? keys[a] : 0u;
+    bool head = true;
+    set_one<C>(S.V, role, lane);
+    for (int it = 0; it < ls; it++) {
+        const size_t t = a + it;
+        const bool real = active && t < n;
+        const unsigned kt = real ? keys[t] : cur;
+        const bool brk = kt != cur;
+        if (brk) {                                                                      // the run ending at t is finished
+            if (head && !last) { scatter_entry<C>(vals_next + 2 * l * C::ENTRY4, S.V, role, lane); if (role == 0) keys_next[2 * l] = cur; }
+            else scatter_entry<C>(out + (size_t)cur * C::ENTRY4, S.V, role, lane);
+            head = false; cur = kt;
+        }
+        set_one_where<C>(S.V, brk, role, lane);
+        const size_t ts = real ? t : n - 1;
+        if (src) load_value<C>(S.B, src + (size_t)idx[ts] * src_words, src_words, role, lane);
+        else gather_entry<C>(S.B, src_lazy + ts * C::ENTRY4, role, lane);
+        set_one_where<C>(S.B, !real, role, lane);
+        mm<C, false, ENG>(S, S.B, role, lane);
+    }
+    if (active) {
+        if (last) scatter_entry<C>(out + (size_t)cur * C::ENTRY4, S.V, role, lane);
+        else {
+            scatter_entry<C>(vals_next + (2 * l + 1) * C::ENTRY4, S.V, role, lane);
+            if (head) scatter_one<C>(vals_next + 2 * l * C::ENTRY4, role);
+            if (role == 0) { keys_next[2 * l + 1] = cur; if (head) keys_next[2 * l] = cur; }
+        }
+    }
+    cta_end<C, ENG>(S);
+}
+
+// Buckets B_1 .. B_(2^c - 1) of a set -> per segment [a, a + lseg): T = prod B_d^(d - a + 1) and A = prod B_d, as running products from
+// the top (A *= B_d, T *= A: two multiplications per bucket, buckets past 2^c - 1 are 1).  One lane per (set, segment); the set's
+// W = prod B_d^d is then prod_s T_s * A_s^(a_s - 1), with a_exp[unit] = a - 1 the scalar of k_scalar.  T rests in the CTA's scratch
+// while A is multiplied and the other way round.
+template <class C, int ENG>
+__global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_bucket_reduce(B28Dev K, const int4* __restrict__ buckets, int c, int nseg, int lseg,
+                                                                              size_t units, u64* __restrict__ t_out, u64* __restrict__ a_out,
+                                                                              u64* __restrict__ a_exp, int4* scratch) {
+    extern __shared__ int4 smem[];
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
+    cta_begin<C, ENG>(S, smem, K);
+    size_t unit = (size_t)blockIdx.x * 32 + lane;
+    const bool active = unit < units;
+    if (!active) unit = units - 1;
+    const size_t set = unit / nseg;
+    const int a = 1 + (int)(unit % nseg) * lseg, dmax = (1 << c) - 1;
+    const int4* bk = buckets + (set << c) * C::ENTRY4;
+    int4* sa = scratch + (size_t)blockIdx.x * 2 * C::VAL4;
+    int4* stt = sa + C::VAL4;
+    set_one<C>(S.V, role, lane);
+    copy_to_global<C>(sa, S.V, role, lane);                                             // A = 1, T = 1 (in V)
+    for (int it = lseg - 1; it >= 0; it--) {
+        const int d = a + it;
+        copy_to_global<C>(stt, S.V, role, lane);
+        copy_from_global<C>(S.V, sa, role, lane);
+        gather_entry<C>(S.B, bk + (size_t)(d <= dmax ? d : dmax) * C::ENTRY4, role, lane);
+        set_one_where<C>(S.B, d > dmax, role, lane);
+        mm<C, false, ENG>(S, S.B, role, lane);                                          // A *= B_d
+        copy_to_global<C>(sa, S.V, role, lane);
+#pragma unroll
+        for (int ch = 0; ch < C::CH; ch++) S.B[(role * C::CH + ch) * 32 + lane] = S.V[(role * C::CH + ch) * 32 + lane];
+        __syncthreads();
+        copy_from_global<C>(S.V, stt, role, lane);
+        mm<C, false, ENG>(S, S.B, role, lane);                                          // T *= A
+    }
+    finalize<C, ENG>(S, K, t_out + unit * K.words_out, active, role, lane);
+    copy_from_global<C>(S.V, sa, role, lane);
+    finalize<C, ENG>(S, K, a_out + unit * K.words_out, active, role, lane);
+    if (active && threadIdx.x < 32) a_exp[unit] = (u64)(a - 1);
+    cta_end<C, ENG>(S);
+}
+
+// x_u <- x_u^(2^(c * jg)) * prod_jl W_(u, jl)^(2^(c * jl)) (Horner over a group of windows, most significant first), one lane per
+// (sign, row); x and W canonical, x updated in place
+template <class C, int ENG>
+__global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_horner(B28Dev K, u64* x, const u64* __restrict__ w, size_t units, int jg, int c) {
+    extern __shared__ int4 smem[];
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
+    cta_begin<C, ENG>(S, smem, K);
+    size_t unit = (size_t)blockIdx.x * 32 + lane;
+    const bool active = unit < units;
+    if (!active) unit = units - 1;
+    load_value<C>(S.V, x + unit * K.words_out, K.words_out, role, lane);
+    for (int jl = jg - 1; jl >= 0; jl--) {
+        for (int s_ = 0; s_ < c; s_++) mm<C, true, ENG>(S, nullptr, role, lane);
+        load_value<C>(S.B, w + (unit * jg + jl) * K.words_out, K.words_out, role, lane);
+        mm<C, false, ENG>(S, S.B, role, lane);
+    }
+    finalize<C, ENG>(S, K, x + unit * K.words_out, active, role, lane);
+    cta_end<C, ENG>(S);
+}
+
+// lazy digits -> canonical words, one lane per value
+template <class C, int ENG>
+__global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_lazy_canon(B28Dev K, const int4* __restrict__ in, size_t count, u64* __restrict__ out) {
+    extern __shared__ int4 smem[];
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
+    cta_begin<C, ENG>(S, smem, K);
+    size_t unit = (size_t)blockIdx.x * 32 + lane;
+    const bool active = unit < count;
+    if (!active) unit = count - 1;
+    gather_entry<C>(S.V, in + unit * C::ENTRY4, role, lane);
+    finalize<C, ENG>(S, K, out + unit * K.words_out, active, role, lane);
+    cta_end<C, ENG>(S);
+}
+
+// Digits of one pass (rows [r0, r0 + rb), ciphertexts [i0, i0 + nc), windows [j0, j0 + jg)), one thread per (row, ciphertext): every
+// non-zero c-bit digit d becomes one entry with key ((sign * rb + row) * jg + window) * 2^c + d and value i - i0.  keys == nullptr:
+// histogram into cursor; else scatter to the positions cursor holds (its exclusive scan), order inside a bucket arbitrary.
+__global__ void k_mv_digits(const u64* __restrict__ w, const uint8_t* __restrict__ neg, size_t count, int kw, size_t r0, size_t rb, size_t i0,
+                            size_t nc, int c, int j0, int jg, unsigned* __restrict__ cursor, unsigned* __restrict__ keys, unsigned* __restrict__ idx) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= rb * nc) return;
+    const size_t r = t / nc, i = t - r * nc, e = (r0 + r) * count + i0 + i;
+    const u64* m = w + e * kw;
+    const unsigned sgn = neg && neg[e] ? 1u : 0u;
+    for (int jl = 0; jl < jg; jl++) {
+        const int bit = (j0 + jl) * c, wi = bit >> 6, sft = bit & 63;
+        u64 v = m[wi] >> sft;
+        if (sft + c > 64 && wi + 1 < kw) v |= m[wi + 1] << (64 - sft);
+        const unsigned d = (unsigned)(v & ((1ull << c) - 1));
+        if (!d) continue;
+        const unsigned key = (((sgn * (unsigned)rb + (unsigned)r) * (unsigned)jg + (unsigned)jl) << c) + d;
+        const unsigned p = atomicAdd(cursor + key, 1u);
+        if (keys) { keys[p] = key; idx[p] = (unsigned)i; }
+    }
+}
+
+// in-place exclusive scan of n counters, one CTA of 1024 threads (each a contiguous slice); *total = the sum
+__global__ void __launch_bounds__(1024) k_mv_scan(unsigned* v, size_t n, unsigned* total) {
+    __shared__ unsigned s[1024];
+    const int tid = threadIdx.x;
+    const size_t per = (n + 1023) / 1024, b = tid * per, e = b + per < n ? b + per : n;
+    unsigned sum = 0;
+    for (size_t i = b; i < e; i++) sum += v[i];
+    s[tid] = sum;
+    __syncthreads();
+    for (int off = 1; off < 1024; off <<= 1) {
+        const unsigned x = tid >= off ? s[tid - off] : 0u;
+        __syncthreads();
+        s[tid] += x;
+        __syncthreads();
+    }
+    unsigned run = s[tid] - sum;
+    for (size_t i = b; i < e; i++) { const unsigned x = v[i]; v[i] = run; run += x; }
+    if (tid == 1023) *total = s[1023];
+}
+
+// n lazy values (e4 int4 each) <- 1
+__global__ void k_mv_one_lazy(int4* p, size_t n, int e4) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < n * e4) p[t] = make_int4(t % e4 == 0 ? 1 : 0, 0, 0, 0);
+}
+// n canonical values (wo words each) <- 1
+__global__ void k_mv_one_words(u64* p, size_t n, int wo) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < n * wo) p[t] = t % wo == 0 ? 1 : 0;
+}
+// entry lists of the per-set fold: set s owns per = 2m (+ 1) entries, values at s*m + l (l < m), sets*m + s*m + l - m (l < 2m),
+// 2*sets*m + s (l = 2m) of a [T | A' | W] block
+__global__ void k_mv_block_entries(unsigned* keys, unsigned* idx, size_t sets, int m, int per) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= sets * per) return;
+    const size_t s = t / per; const int l = (int)(t - s * per);
+    keys[t] = (unsigned)s;
+    idx[t] = (unsigned)(l < m ? s * m + l : l < 2 * m ? sets * m + s * m + (l - m) : 2 * sets * m + s);
+}
+// the magnitudes of one sign (the others 0): chain method
+__global__ void k_mv_mask(const u64* __restrict__ w, const uint8_t* __restrict__ neg, size_t n, int kw, int sgn, u64* __restrict__ out) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n * kw) return;
+    const int s = neg && neg[t / kw] ? 1 : 0;
+    out[t] = s == sgn ? w[t] : 0;
 }
 
 
@@ -1722,6 +1934,247 @@ cudaError_t block28_add(Block28Key* key, const u64* d_c1, const u64* d_c2, int c
     if (key->G == 8) return add_cfg<Cfg2048>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st);
     if (key->BL == 14) return add_cfg<Cfg3072>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st);
     return add_cfg<Cfg4096>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st);
+}
+
+// ---- matvec: planner and driver (DESIGN.md §9b) ---------------------------------------------------------------------------------
+static size_t cdiv(size_t a, size_t b) { return (a + b - 1) / b; }
+// multiplications of k_scalar's chain for k_bits-bit scalars (table, windows, finalize)
+static uint64_t scalar_chain(uint32_t k_bits) {
+    const int w = scalar_window(k_bits);
+    return ((1u << w) - 2) + ((k_bits + w - 1) / w - 1) * (uint64_t)(w + 1) + 1;
+}
+// slice length of a k_bucket_fold launch over n entries: one wave of lanes, at least 8 entries (the carry list shrinks 4x per level)
+static int fold_ls(size_t n, size_t lanes) { const size_t l = cdiv(n, lanes); return (int)(l < 8 ? 8 : l); }
+// mulmods (upper bound) and sequential chain of the fold of n entries, every carry level included
+static void fold_cost(size_t n, size_t lanes, uint64_t* work, uint64_t* chain) {
+    for (;;) {
+        const int ls = fold_ls(n, lanes);
+        const size_t l = cdiv(n, (size_t)ls);
+        *work += (uint64_t)l * ls + l; *chain += (uint64_t)ls + 1;
+        if (l <= 1) break;
+        n = 2 * l;
+    }
+}
+static size_t fold_lanes0(size_t n, size_t lanes) { return cdiv(n, (size_t)fold_ls(n, lanes)); }
+
+struct MvShape { size_t e_bytes = 0, wo = 0, lanes = 0; bool ok = false; };
+template <class C>
+static MvShape mv_shape_cfg(uint32_t n_bits, int sms) {
+    MvShape s; s.e_bytes = (size_t)C::ENTRY4 * 16; s.wo = (2 * (size_t)n_bits + 63) / 64; s.lanes = (size_t)sms * C::CTAS_PER_SM * 32; s.ok = true;
+    return s;
+}
+static MvShape mv_shape(uint32_t n_bits, int sms) {
+    if (covers<Cfg1024>(n_bits)) return mv_shape_cfg<Cfg1024>(n_bits, sms);
+    if (covers<Cfg2048>(n_bits)) return mv_shape_cfg<Cfg2048>(n_bits, sms);
+    if (covers<Cfg3072>(n_bits)) return mv_shape_cfg<Cfg3072>(n_bits, sms);
+    if (covers<Cfg4096>(n_bits)) return mv_shape_cfg<Cfg4096>(n_bits, sms);
+    return MvShape();
+}
+
+// the bucket method's arena, carved in this order (every piece 256-byte aligned)
+struct MvLayout {
+    size_t hist, keys, idx, skeys, sidx, ckeys[2], cvals[2], cnt, buckets, vals, aseg, scal, rscr, wlazy, x, nprime, total;
+};
+static MvLayout mv_layout(const MatvecPlan& P, const MvShape& S) {
+    const size_t sp = P.rb * P.nsign * P.jg, nkeys = sp << P.c, ents = P.rb * P.jg * P.nc, units = sp * P.nseg;
+    const size_t sents = std::max(sp * (2 * (size_t)P.nseg + 1), 2 * P.rb);
+    const size_t carry = 2 * std::max(fold_lanes0(ents, S.lanes), fold_lanes0(sents, S.lanes));
+    const size_t vb = S.wo * 8;
+    MvLayout L; size_t o = 0;
+    auto take = [&](size_t bytes) { const size_t at = o; o += (bytes + 255) & ~(size_t)255; return at; };
+    L.hist = take(nkeys * 4); L.keys = take(ents * 4); L.idx = take(ents * 4); L.skeys = take(sents * 4); L.sidx = take(sents * 4);
+    for (int i = 0; i < 2; i++) { L.ckeys[i] = take(carry * 4); L.cvals[i] = take(carry * S.e_bytes); }
+    L.cnt = take(64 * 4); L.buckets = take(nkeys * S.e_bytes); L.vals = take((2 * units + sp) * vb); L.aseg = take(units * vb);
+    L.scal = take(units * 8); L.rscr = take(cdiv(units, 32) * 64 * S.e_bytes); L.wlazy = take(std::max(sp, P.rb) * S.e_bytes);
+    L.x = take(P.rb * P.nsign * vb); L.nprime = take(P.rb * vb);
+    L.total = o;
+    return L;
+}
+
+size_t matvec_budget(uint32_t n_bits) { return ((size_t)3 << 18) * 8 * ((2 * (size_t)n_bits + 63) / 64); }
+
+MatvecPlan matvec_plan(uint32_t n_bits, int sms, size_t rows, size_t count, uint32_t k_bits, bool has_neg, bool bucket_ok) {
+    const MvShape S = mv_shape(n_bits, sms > 0 ? sms : 1);
+    const size_t budget = matvec_budget(n_bits), wo = (2 * (size_t)n_bits + 63) / 64, kw = (k_bits + 63) / 64, kwn = (n_bits + 63) / 64;
+    const size_t lanes = S.ok ? S.lanes : (size_t)(sms > 0 ? sms : 1) * 64;
+    const int nsign = has_neg ? 2 : 1;
+    const char* force = getenv("PB200_MATVEC_METHOD");
+    size_t pe = (size_t)1 << 24;
+    if (const char* e = getenv("PB200_MATVEC_PASS_ENTRIES")) { const long long v = atoll(e); if (v >= 1 && (size_t)v < pe) pe = (size_t)v; }
+    auto waves = [&](size_t u) -> uint64_t { return cdiv(u ? u : 1, lanes); };
+    if (!rows || !count) { MatvecPlan z; z.nsign = nsign; return z; }                    // nothing to multiply: every row is 1
+    // chain: per row and sign, chunks of 2^18 ciphertexts (masked scalars, scalar products, tally); sign step per block of rows
+    MatvecPlan ch;
+    {
+        const size_t chunk = std::min(count, (size_t)1 << 18), chunks = cdiv(count, (size_t)1 << 18), rbc = std::min(rows, (size_t)4096);
+        const uint64_t sk = scalar_chain(k_bits), sn = scalar_chain(n_bits);
+        ch.method = 0; ch.nsign = nsign; ch.rb = rbc; ch.nc = chunk; ch.passes = rows * nsign * chunks;
+        ch.acc = (uint64_t)rows * nsign * count * sk;
+        ch.red = (uint64_t)rows * nsign * (count + 2 * chunks);
+        ch.sign = has_neg ? (uint64_t)rows * (sn + 2) : 0;
+        ch.chain = ch.passes * (sk + 8) + (has_neg ? cdiv(rows, rbc) * sn + rows * 8 : 0);
+        ch.bytes = (chunk * (kw + wo) + (4 + 2 * rbc) * wo + rbc * kwn) * 8;
+        if (!S.ok || !bucket_ok || (force && !strcmp(force, "chain"))) return ch;
+    }
+    const uint64_t slots_chain = (uint64_t)rows * nsign * cdiv(count, (size_t)1 << 18) * (waves(std::min(count, (size_t)1 << 18)) * (scalar_chain(k_bits) + 1) + 8) +
+                                 (has_neg ? cdiv(rows, ch.rb) * waves(ch.rb) * scalar_chain(n_bits) + rows * 8 : 0);
+    MatvecPlan best; uint64_t best_slots = ~0ull;
+    for (int c = 1; c <= 16 && c <= (int)k_bits; c++) {
+        MatvecPlan p; p.method = 1; p.c = c; p.J = (int)cdiv(k_bits, c); p.nsign = nsign;
+        p.nc = std::min(count, pe);
+        const size_t q = std::max((size_t)1, pe / p.nc);
+        p.jg = std::min((size_t)p.J, q); p.rb = std::min(rows, std::max((size_t)1, q / p.jg));
+        uint64_t slots = 0; bool fit = false;
+        for (;;) {
+            // segment length: one wave of reduce lanes where possible, fewest slots
+            const size_t sp = p.rb * nsign * p.jg, nb = ((size_t)1 << c) - 1;
+            uint64_t rs_best = ~0ull;
+            for (size_t ls = 1; ls <= nb; ls <<= 1) {
+                const size_t nseg = cdiv(nb, ls), units = sp * nseg;
+                uint64_t w = 0, fch = 0; fold_cost(sp * (2 * nseg + 1), lanes, &w, &fch);
+                const uint64_t rs = waves(units) * (2 * ls + 2 + scalar_chain(c)) + fch;
+                if (rs < rs_best) { rs_best = rs; p.lseg = (int)ls; p.nseg = (int)nseg; }
+            }
+            p.bytes = mv_layout(p, S).total + (has_neg ? p.rb * kwn * 8 : 0);              // + the sign step's copies of n - 1
+            if (p.bytes <= budget) { fit = true; break; }
+            if (p.rb > 1) p.rb = cdiv(p.rb, 2);
+            else if (p.jg > 1) p.jg = cdiv(p.jg, 2);
+            else if (p.nc > 1) p.nc = cdiv(p.nc, 2);
+            else break;
+        }
+        if (!fit) continue;
+        const size_t sp = p.rb * nsign * p.jg, units = sp * p.nseg, blocks = cdiv(rows, p.rb), groups = cdiv(p.J, p.jg), chunks = cdiv(count, p.nc);
+        p.passes = blocks * groups * chunks;
+        uint64_t fw = 0, fc = 0, sw = 0, sc = 0, cw = 0, cc = 0;
+        fold_cost(p.rb * p.jg * p.nc, lanes, &fw, &fc);
+        fold_cost(sp * (2 * (size_t)p.nseg + 1), lanes, &sw, &sc);
+        fold_cost(2 * p.rb, lanes, &cw, &cc);
+        const uint64_t sn = scalar_chain(n_bits), s_c = scalar_chain(c);
+        p.acc = p.passes * fw;
+        p.red = p.passes * ((uint64_t)units * (2 * p.lseg + 2) + units * s_c + sw + sp);
+        p.horner = (uint64_t)blocks * groups * p.rb * nsign * p.jg * (c + 1) + blocks * p.rb * nsign;
+        p.sign = has_neg ? (uint64_t)blocks * p.rb * sn + blocks * cw : 0;
+        const uint64_t pass_chain = fc + 2 * p.lseg + 2 + s_c + sc + 1, group_chain = (uint64_t)p.jg * (c + 1) + 1;
+        p.chain = p.passes * pass_chain + blocks * groups * group_chain + (has_neg ? blocks * (sn + cc) : 0);
+        slots = p.passes * (fc + waves(units) * (2 * p.lseg + 2 + s_c) + sc + 1) +
+                blocks * groups * waves(p.rb * nsign) * group_chain + (has_neg ? blocks * (waves(p.rb) * sn + cc) : 0);
+        if (slots < best_slots) { best_slots = slots; best = p; }
+    }
+    if (!best.method) return ch;
+    if (force && !strcmp(force, "bucket")) return best;
+    return best_slots < slots_chain ? best : ch;
+}
+
+#define MV_LAUNCH(KERN, grid, ...) do {                                                                                             \
+    if (eng == 4) { if constexpr (UL<C, 1>::SUPPORTED) {                                                                            \
+        CUW((cudaFuncSetAttribute(KERN<C, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));           \
+        KERN<C, 4><<<(unsigned)(grid), C::THREADS, UL<C, 1>::SMEM_BYTES, st>>>(__VA_ARGS__); } }                                     \
+    else if (eng == 1) {                                                                                                             \
+        CUW((cudaFuncSetAttribute(KERN<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));                  \
+        KERN<C, 1><<<(unsigned)(grid), C::THREADS, C::SMEM_BYTES, st>>>(__VA_ARGS__); }                                              \
+    else {                                                                                                                           \
+        CUW((cudaFuncSetAttribute(KERN<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));                  \
+        KERN<C, 0><<<(unsigned)(grid), C::THREADS, C::SMEM_BYTES, st>>>(__VA_ARGS__); }                                              \
+    count_launch(); CUW(cudaGetLastError()); } while (0)
+
+// k_bucket_fold over an entry list, level after level until the carry list is empty.  n_dev: the entry count is *cnt (device);
+// else n_ub exactly.  Level l reads its count from cnt[l] and writes the next one to cnt[l + 1].
+template <class C>
+static cudaError_t mv_fold(Block28Key* key, int eng, const unsigned* keys, const unsigned* idx, const u64* src, bool n_dev, size_t n_ub,
+                           int4* out, const MvLayout& L, unsigned char* A, size_t lanes, cudaStream_t st) {
+    unsigned* cnt = (unsigned*)(A + L.cnt);
+    int lv = 0, ls = fold_ls(n_ub, lanes);
+    size_t ln = cdiv(n_ub, (size_t)ls);
+    MV_LAUNCH(k_bucket_fold, cdiv(ln, 32), key->dev, keys, idx, src, key->dev.words_out, (const int4*)nullptr, n_dev ? cnt : nullptr, n_ub, ls,
+              out, (unsigned*)(A + L.ckeys[0]), (int4*)(A + L.cvals[0]), cnt + 1);
+    while (ln > 1) {
+        const size_t n = 2 * ln;
+        ls = fold_ls(n, lanes); ln = cdiv(n, (size_t)ls); lv++;
+        const int i = (lv - 1) & 1;
+        MV_LAUNCH(k_bucket_fold, cdiv(ln, 32), key->dev, (const unsigned*)(A + L.ckeys[i]), (const unsigned*)nullptr, (const u64*)nullptr, 0,
+                  (const int4*)(A + L.cvals[i]), cnt + lv, n, ls, out, (unsigned*)(A + L.ckeys[i ^ 1]), (int4*)(A + L.cvals[i ^ 1]), cnt + lv + 1);
+        if (lv >= 62) return cudaErrorInvalidValue;
+    }
+    return cudaSuccess;
+}
+
+template <class C>
+static cudaError_t matvec_cfg(Block28Key* key, const MatvecPlan& P, const u64* d_c, size_t count, const u64* d_w, uint32_t k_bits,
+                              const uint8_t* d_neg, size_t rows, u64* d_out, unsigned char* A, const u64* d_nm1, cudaStream_t st) {
+    CUW(ensure_slots<C>(key, st));
+    const MvShape S = mv_shape_cfg<C>(key->n_bits, key->sms);
+    const MvLayout L = mv_layout(P, S);
+    const int eng = key->eng >= 2 && key->has_u ? 4 : key->eng;
+    const int c = P.c, kw = (int)((k_bits + 63) / 64), wo = key->dev.words_out;
+    const size_t vb = (size_t)wo;                                   // u64 per canonical value
+    u64* vals = (u64*)(A + L.vals); u64* x = (u64*)(A + L.x);
+    for (size_t r0 = 0; r0 < rows; r0 += P.rb) {
+        const size_t rb = std::min(P.rb, rows - r0), xs = rb * P.nsign;
+        k_mv_one_words<<<(unsigned)cdiv(xs * wo, 256), 256, 0, st>>>(x, xs, wo); count_launch();
+        for (size_t g = cdiv(P.J, P.jg); g-- > 0;) {
+            const int j0 = (int)(g * P.jg), jg = (int)std::min(P.jg, (size_t)P.J - j0);
+            const size_t sp = xs * jg, units = sp * P.nseg, nkeys = sp << c;
+            u64* w_acc = vals + 2 * units * vb;                                              // the W block of [T | A' | W]
+            k_mv_one_words<<<(unsigned)cdiv(sp * wo, 256), 256, 0, st>>>(w_acc, sp, wo); count_launch();
+            for (size_t i0 = 0; i0 < count; i0 += P.nc) {
+                const size_t nc = std::min(P.nc, count - i0), th = rb * nc;
+                unsigned* hist = (unsigned*)(A + L.hist);
+                CUW(cudaMemsetAsync(hist, 0, nkeys * 4, st));
+                k_mv_digits<<<(unsigned)cdiv(th, 256), 256, 0, st>>>(d_w, d_neg, count, kw, r0, rb, i0, nc, c, j0, jg, hist, nullptr, nullptr);
+                k_mv_scan<<<1, 1024, 0, st>>>(hist, nkeys, (unsigned*)(A + L.cnt));
+                k_mv_digits<<<(unsigned)cdiv(th, 256), 256, 0, st>>>(d_w, d_neg, count, kw, r0, rb, i0, nc, c, j0, jg, hist,
+                                                                    (unsigned*)(A + L.keys), (unsigned*)(A + L.idx));
+                k_mv_one_lazy<<<(unsigned)cdiv(nkeys * C::ENTRY4, 256), 256, 0, st>>>((int4*)(A + L.buckets), nkeys, C::ENTRY4);
+                count_launch(4);
+                CUW(cudaGetLastError());
+                CUW(mv_fold<C>(key, eng, (const unsigned*)(A + L.keys), (const unsigned*)(A + L.idx), d_c + i0 * wo, true, rb * jg * nc,
+                               (int4*)(A + L.buckets), L, A, S.lanes, st));
+                MV_LAUNCH(k_bucket_reduce, cdiv(units, 32), key->dev, (const int4*)(A + L.buckets), c, P.nseg, P.lseg, units, vals,
+                          (u64*)(A + L.aseg), (u64*)(A + L.scal), (int4*)(A + L.rscr));
+                CUW(scalar_cfg<C>(key, (const u64*)(A + L.aseg), (const u64*)(A + L.scal), (uint32_t)c, units, vals + units * vb, st));
+                const int per = 2 * P.nseg + 1;
+                k_mv_block_entries<<<(unsigned)cdiv(sp * per, 256), 256, 0, st>>>((unsigned*)(A + L.skeys), (unsigned*)(A + L.sidx), sp, P.nseg, per);
+                count_launch(); CUW(cudaGetLastError());
+                CUW(mv_fold<C>(key, eng, (const unsigned*)(A + L.skeys), (const unsigned*)(A + L.sidx), vals, false, sp * per,
+                               (int4*)(A + L.wlazy), L, A, S.lanes, st));
+                MV_LAUNCH(k_lazy_canon, cdiv(sp, 32), key->dev, (const int4*)(A + L.wlazy), sp, w_acc);
+            }
+            MV_LAUNCH(k_horner, cdiv(xs, 32), key->dev, x, (const u64*)w_acc, xs, jg, c);
+        }
+        u64* out = d_out + r0 * vb;
+        if (P.nsign == 1) { CUW(cudaMemcpyAsync(out, x, rb * vb * 8, cudaMemcpyDeviceToDevice, st)); continue; }
+        // sign step: N^(n-1) next to P, then the fold of the pairs (P_r, N_r^(n-1))
+        u64* np = (u64*)(A + L.nprime);
+        CUW(scalar_cfg<C>(key, x + rb * vb, d_nm1, key->n_bits, rb, np, st));
+        CUW(cudaMemcpyAsync(x + rb * vb, np, rb * vb * 8, cudaMemcpyDeviceToDevice, st));
+        k_mv_block_entries<<<(unsigned)cdiv(2 * rb, 256), 256, 0, st>>>((unsigned*)(A + L.skeys), (unsigned*)(A + L.sidx), rb, 1, 2);
+        count_launch(); CUW(cudaGetLastError());
+        CUW(mv_fold<C>(key, eng, (const unsigned*)(A + L.skeys), (const unsigned*)(A + L.sidx), x, false, 2 * rb, (int4*)(A + L.wlazy), L, A,
+                       S.lanes, st));
+        MV_LAUNCH(k_lazy_canon, cdiv(rb, 32), key->dev, (const int4*)(A + L.wlazy), rb, out);
+    }
+    return cudaSuccess;
+}
+#undef MV_LAUNCH
+
+cudaError_t block28_matvec(Block28Key* key, const MatvecPlan& P, const u64* d_c, size_t count, const u64* d_w, uint32_t k_bits, const uint8_t* d_neg,
+                           size_t rows, u64* d_out, void* arena, const u64* d_nm1, cudaStream_t st) {
+    if (!rows || !count || P.method != 1) return cudaErrorInvalidValue;
+    unsigned char* A = (unsigned char*)arena;
+    if (key->G == 4) return matvec_cfg<Cfg1024>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
+    if (key->G == 8) return matvec_cfg<Cfg2048>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
+    if (key->BL == 14) return matvec_cfg<Cfg3072>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
+    return matvec_cfg<Cfg4096>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
+}
+cudaError_t matvec_mask(const u64* d_w, const uint8_t* d_neg, size_t n, int kw, int sgn, u64* d_out, cudaStream_t st) {
+    if (!n) return cudaSuccess;
+    k_mv_mask<<<(unsigned)cdiv(n * kw, 256), 256, 0, st>>>(d_w, d_neg, n, kw, sgn, d_out); count_launch();
+    return cudaGetLastError();
+}
+cudaError_t matvec_ones(u64* d_out, size_t n, int wo, cudaStream_t st) {
+    if (!n) return cudaSuccess;
+    k_mv_one_words<<<(unsigned)cdiv(n * wo, 256), 256, 0, st>>>(d_out, n, wo); count_launch();
+    return cudaGetLastError();
 }
 
 }  // namespace pb200

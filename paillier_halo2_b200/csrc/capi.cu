@@ -70,6 +70,8 @@ struct pb200_key {
     int engine = 0;                 // 0 auto, 1 simple64, 2 block28, 3 block28t, 4 block28u, 5 block28u2
     DevBuf in_a, in_b, out_a, out_b, scratch, offs;
     DevBuf wt_chunk, wt_part;               // weighted tally: one chunk's scalar products, the per-chunk partial products
+    DevBuf mv_arena, mv_neg, mv_nm1;        // matvec: temporary memory of the plan, staged signs, copies of n - 1 for the sign step
+    size_t mv_nm1_units = 0;
     std::string engine_name;
     // K4 cell expansion: per lookup_bits layout + device constants (n^2 limbs, word_max, q_acc, mod_acc), refresh spill vector
     struct CellCtx { CellLayout Y; u64* d_consts = nullptr; int* d_inc = nullptr; u64* d_mtab = nullptr; int n_out = 0; int n2_cells = 0; };
@@ -184,6 +186,7 @@ void pb200_key_destroy(pb200_key* k) {
     if (k->d_lambda) cudaFree(k->d_lambda);
     k->in_a.release(); k->in_b.release(); k->out_a.release(); k->out_b.release(); k->scratch.release(); k->offs.release();
     k->wt_chunk.release(); k->wt_part.release();
+    k->mv_arena.release(); k->mv_neg.release(); k->mv_nm1.release();
     k->cin_a.release(); k->cin_b.release(); k->cin_q.release(); k->cin_r.release();
     if (k->pipe.ready) {
         if (k->pipe.copy) { cudaStreamSynchronize(k->pipe.copy); cudaStreamDestroy(k->pipe.copy); }
@@ -691,6 +694,110 @@ int pb200_tally_weighted(pb200_key* k, const uint64_t* c, const uint64_t* ks, ui
     CU(cudaMemcpyAsync(out, k->out_b.p, bout, cudaMemcpyDeviceToHost, k->stream));
     CU(cudaStreamSynchronize(k->stream));
     return take_flags(k);
+} PB200_CATCH
+
+// ---- matvec: out_r = P_r * N_r^(n-1), P_r / N_r the products of c_i^|w_ri| over the positive / negative weights ---------------
+// `units` copies of n - 1 (the sign step's scalar), prepared once per key
+static int mv_nm1(pb200_key* k, size_t units) {
+    if (k->mv_nm1_units >= units) return PB200_OK;
+    const size_t kwn = PB200_WORDS(k->n_bits);
+    std::vector<u64> h(units * kwn);
+    const BigInt nm1 = BigInt::sub(k->n, BigInt(1));
+    for (size_t u = 0; u < units; u++) nm1.to_u64_le(h.data() + u * kwn, (uint32_t)kwn);
+    CU(k->mv_nm1.reserve(h.size() * sizeof(u64)));
+    CU(cudaMemcpyAsync(k->mv_nm1.p, h.data(), h.size() * sizeof(u64), cudaMemcpyHostToDevice, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    k->mv_nm1_units = units;
+    return PB200_OK;
+}
+// chain method: per row and sign, the weighted tally of the masked magnitudes (chunks of 2^18 ciphertexts, partials folded into the
+// row's value); then per block of rows N^(n-1) in one scalar launch and P * N^(n-1) by a tally of the pair
+static int matvec_chain(pb200_key* k, const MatvecPlan& P, const u64* d_c, size_t count, const u64* d_w, uint32_t k_bits, const uint8_t* d_neg,
+                        size_t rows, u64* d_out) {
+    const size_t wo = k->words_out, kw = PB200_WORDS(k_bits), CH = WT_CHUNK, chunk = count < CH ? count : CH, rbc = P.rb;
+    CU(k->mv_arena.reserve((chunk * kw + (4 + 2 * rbc) * wo) * sizeof(u64)));
+    u64* masked = (u64*)k->mv_arena.p;
+    u64* acc = masked + chunk * kw;                   // [running product, chunk partial]
+    u64* pair = acc + 2 * wo;                         // [P_r, N_r^(n-1)]
+    u64* nb = pair + 2 * wo;                          // N of the row block
+    u64* np = nb + rbc * wo;                          // N^(n-1) of the row block
+    int rc;
+    for (size_t r0 = 0; r0 < rows; r0 += rbc) {
+        const size_t rb = rows - r0 < rbc ? rows - r0 : rbc;
+        for (size_t r = 0; r < rb; r++)
+            for (int sgn = 0; sgn < P.nsign; sgn++) {
+                u64* dst = sgn ? nb + r * wo : d_out + (r0 + r) * wo;
+                for (size_t i0 = 0; i0 < count; i0 += CH) {
+                    const size_t n = count - i0 < CH ? count - i0 : CH, e = (r0 + r) * count + i0;
+                    CU(matvec_mask(d_w + e * kw, d_neg ? d_neg + e : nullptr, n, (int)kw, sgn, masked, k->stream));
+                    if (!i0) { rc = tally_weighted_dev_impl(k, d_c, masked, k_bits, n, dst); if (rc) return rc; continue; }
+                    rc = tally_weighted_dev_impl(k, d_c + i0 * wo, masked, k_bits, n, acc + wo); if (rc) return rc;
+                    CU(cudaMemcpyAsync(acc, dst, wo * sizeof(u64), cudaMemcpyDeviceToDevice, k->stream));
+                    rc = tally_dev_impl(k, acc, 2, dst, false); if (rc) return rc;
+                }
+            }
+        if (P.nsign == 1) continue;
+        rc = scalar_dev_impl(k, nb, (const u64*)k->mv_nm1.p, k->n_bits, rb, np); if (rc) return rc;
+        for (size_t r = 0; r < rb; r++) {
+            u64* out = d_out + (r0 + r) * wo;
+            CU(cudaMemcpyAsync(pair, out, wo * sizeof(u64), cudaMemcpyDeviceToDevice, k->stream));
+            CU(cudaMemcpyAsync(pair + wo, np + r * wo, wo * sizeof(u64), cudaMemcpyDeviceToDevice, k->stream));
+            rc = tally_dev_impl(k, pair, 2, out, false); if (rc) return rc;
+        }
+    }
+    return PB200_OK;
+}
+static int matvec_dev_impl(pb200_key* k, const u64* d_c, size_t count, const u64* d_w, const uint8_t* d_neg, uint32_t k_bits, size_t rows,
+                           u64* d_out) {
+    if (!rows) return PB200_OK;
+    if (!count) { CU(matvec_ones(d_out, rows, (int)k->words_out, k->stream)); return PB200_OK; }
+    const MatvecPlan P = matvec_plan(k->n_bits, k->sms, rows, count, k_bits, d_neg != nullptr, use_fast(k));
+    if (P.nsign == 2) { int rc = mv_nm1(k, P.rb); if (rc) return rc; }
+    if (P.method == 0) return matvec_chain(k, P, d_c, count, d_w, k_bits, d_neg, rows, d_out);
+    CU(k->mv_arena.reserve(P.bytes));                 // the plan's bytes include the copies of n - 1 (held in mv_nm1): a small margin
+    CU(block28_matvec(k->fast, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, k->mv_arena.p, (const u64*)k->mv_nm1.p, k->stream));
+    return PB200_OK;
+}
+static bool matvec_args_ok(const pb200_key* k, const void* c, size_t count, const void* w, uint32_t k_bits, size_t rows, const void* out) {
+    return scalar_args_ok(k, k_bits) && (!rows || out) && (!rows || !count || (c && w));
+}
+int pb200_matvec_dev(pb200_key* k, const uint64_t* d_c, size_t count, const uint64_t* d_w, const uint8_t* d_neg, uint32_t k_bits, size_t rows,
+                     uint64_t* d_out) try {
+    if (!matvec_args_ok(k, d_c, count, d_w, k_bits, rows, d_out)) return PB200_ERR_INVALID_ARG;
+    if (!rows) return PB200_OK;
+    USE_DEVICE(k);
+    return matvec_dev_impl(k, (const u64*)d_c, count, (const u64*)d_w, d_neg, k_bits, rows, (u64*)d_out);
+} PB200_CATCH
+int pb200_matvec(pb200_key* k, const uint64_t* c, size_t count, const uint64_t* w, const uint8_t* neg, uint32_t k_bits, size_t rows,
+                 uint64_t* out) try {
+    if (!matvec_args_ok(k, c, count, w, k_bits, rows, out)) return PB200_ERR_INVALID_ARG;
+    if (!rows) return PB200_OK;
+    int rc = check_scalars(w, k_bits, rows * count); if (rc) return rc;
+    bool any_neg = false;
+    if (neg) for (size_t e = 0; e < rows * count && !any_neg; e++) any_neg = neg[e] != 0;
+    USE_DEVICE(k);
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bc = count * k->words_out * sizeof(u64), bw = rows * count * PB200_WORDS(k_bits) * sizeof(u64), bo = rows * k->words_out * sizeof(u64);
+    CU(k->in_a.reserve(bc ? bc : 8)); CU(k->in_b.reserve(bw ? bw : 8)); CU(k->out_a.reserve(bo));
+    if (bc) CU(cudaMemcpyAsync(k->in_a.p, c, bc, cudaMemcpyHostToDevice, k->stream));
+    if (bw) CU(cudaMemcpyAsync(k->in_b.p, w, bw, cudaMemcpyHostToDevice, k->stream));
+    if (any_neg) {                                    // rows without a negative weight give P_r * 1^(n-1) = P_r: only stage signs when some exist
+        CU(k->mv_neg.reserve(rows * count));
+        CU(cudaMemcpyAsync(k->mv_neg.p, neg, rows * count, cudaMemcpyHostToDevice, k->stream));
+    }
+    rc = matvec_dev_impl(k, (const u64*)k->in_a.p, count, (const u64*)k->in_b.p, any_neg ? (const uint8_t*)k->mv_neg.p : nullptr, k_bits, rows,
+                         (u64*)k->out_a.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out, k->out_a.p, bo, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
+} PB200_CATCH
+int pb200_matvec_plan(uint32_t n_bits, int sms, size_t rows, size_t count, uint32_t k_bits, int has_neg, uint64_t* out11) try {
+    if (!out11 || n_bits == 0 || k_bits == 0 || k_bits > n_bits || sms < 1) return PB200_ERR_INVALID_ARG;
+    const MatvecPlan P = matvec_plan(n_bits, sms, rows, count, k_bits, has_neg != 0, true);
+    const uint64_t v[11] = {(uint64_t)P.method, (uint64_t)P.c, (uint64_t)P.J, P.passes, (uint64_t)P.nseg, P.acc, P.red, P.horner, P.sign, P.chain, P.bytes};
+    for (int i = 0; i < 11; i++) out11[i] = v[i];
+    return PB200_OK;
 } PB200_CATCH
 
 // ---- witness --------------------------------------------------------------------------------

@@ -57,6 +57,25 @@ cudaError_t block28_pow(Block28Key*, const u64* d_base, int base_words, size_t c
 // out_i = c_i^(k_i) mod n^2 with a scalar per unit (PB200_WORDS(k_bits) words each; c_i: words_out words, any value): fixed-window
 // chain per lane, window width chosen from k_bits; no per-key preparation
 cudaError_t block28_scalar(Block28Key*, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out, cudaStream_t st);
+// matvec (pb200_matvec): the planner's choice for one call.  method 0 = chain (per row and sign: scalar products + tally), 1 = bucket.
+// Bucket passes cover rb rows x jg windows x nc ciphertexts (both signs); mulmod counts are upper bounds for dense weights.
+struct MatvecPlan {
+    int method = 0, c = 0, J = 0, nseg = 0, lseg = 0, nsign = 1;
+    size_t rb = 0, jg = 0, nc = 0;
+    uint64_t passes = 0, acc = 0, red = 0, horner = 0, sign = 0, chain = 0, bytes = 0;
+};
+// temporary device memory every matvec stays within: 3 * 2^18 ciphertexts' worth (384 MB at |n| = 2048)
+size_t matvec_budget(uint32_t n_bits);
+// bucket_ok: the key runs a block28 engine.  PB200_MATVEC_METHOD=chain|bucket forces the method, PB200_MATVEC_PASS_ENTRIES caps the
+// sort entries of one pass.  Host only.
+MatvecPlan matvec_plan(uint32_t n_bits, int sms, size_t rows, size_t count, uint32_t k_bits, bool has_neg, bool bucket_ok);
+// bucket method on the block28 engine: out (rows * words_out) canonical; arena: P.bytes of device memory; d_nm1: plan.rb copies of
+// n - 1 (PB200_WORDS(n_bits) words each) when P.nsign == 2
+cudaError_t block28_matvec(Block28Key*, const MatvecPlan& P, const u64* d_c, size_t count, const u64* d_w, uint32_t k_bits, const uint8_t* d_neg,
+                           size_t rows, u64* d_out, void* arena, const u64* d_nm1, cudaStream_t st);
+// plain helpers of the chain method: out <- the magnitudes of sign sgn (others 0); n values of wo words <- 1
+cudaError_t matvec_mask(const u64* d_w, const uint8_t* d_neg, size_t n, int kw, int sgn, u64* d_out, cudaStream_t st);
+cudaError_t matvec_ones(u64* d_out, size_t n, int wo, cudaStream_t st);
 // multi-GPU tally: one launch per GPU, partials exchanged through peer-mapped mailboxes inside the kernel (collective call)
 cudaError_t block28_tally_peer(Block28Key*, const u64* d_c, size_t count, u64* d_out, cudaStream_t st);
 cudaError_t block28_mailbox(Block28Key*, u64** d_mail, cudaStream_t st);

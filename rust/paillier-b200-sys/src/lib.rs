@@ -111,6 +111,11 @@ extern "C" {
     pub fn pb200_scalar_mul_batch_dev(key: *mut pb200_key, d_c_le: *const u64, d_k_le: *const u64, k_bits: u32, count: usize, d_out_le: *mut u64) -> c_int;
     pub fn pb200_tally_weighted(key: *mut pb200_key, c_le: *const u64, k_le: *const u64, k_bits: u32, count: usize, out_le: *mut u64) -> c_int;
     pub fn pb200_tally_weighted_dev(key: *mut pb200_key, d_c_le: *const u64, d_k_le: *const u64, k_bits: u32, count: usize, d_out_le: *mut u64) -> c_int;
+    pub fn pb200_matvec(key: *mut pb200_key, c_le: *const u64, count: usize, w_mag_le: *const u64, w_neg: *const u8, k_bits: u32, rows: usize,
+                        out_le: *mut u64) -> c_int;
+    pub fn pb200_matvec_dev(key: *mut pb200_key, d_c_le: *const u64, count: usize, d_w_mag_le: *const u64, d_w_neg: *const u8, k_bits: u32,
+                            rows: usize, d_out_le: *mut u64) -> c_int;
+    pub fn pb200_matvec_plan(n_bits: u32, sms: c_int, rows: usize, count: usize, k_bits: u32, has_neg: c_int, out11: *mut u64) -> c_int;
 
     pub fn pb200_encrypt_witness_batch(key: *mut pb200_key, m_le: *const u64, r_le: *const u64, count: usize, c_out_le: *mut u64,
                                        max_chunk_units: usize, sink: pb200_witness_sink_fn, user: *mut c_void) -> c_int;
@@ -220,6 +225,24 @@ impl Key {
         }
         let mut out = vec![0u64; wo];
         let rc = unsafe { pb200_tally_weighted(self.raw, c.as_ptr(), k.as_ptr(), k_bits, c.len() / wo, out.as_mut_ptr()) };
+        if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// encrypted matrix-vector product: `c` holds `count * words_out` words, `w_mag` the magnitudes of a `rows x count` weight matrix
+    /// row-major (`ceil(k_bits / 64)` words each, below 2^k_bits), `w_neg` (empty, or `rows * count` bytes) marks the negative ones;
+    /// returns `rows * words_out` words, row r the ciphertext of sum_i w_ri * m_i mod n
+    pub fn matvec(&mut self, c: &[u64], w_mag: &[u64], w_neg: &[u8], k_bits: u32, rows: usize) -> Result<Vec<u64>, i32> {
+        let (wo, kw) = (self.words_out(), ((k_bits as usize) + 63) / 64);
+        if wo == 0 || kw == 0 || c.len() % wo != 0 {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let count = c.len() / wo;
+        if w_mag.len() != rows * count * kw || (!w_neg.is_empty() && w_neg.len() != rows * count) {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let mut out = vec![0u64; rows * wo];
+        let neg = if w_neg.is_empty() { std::ptr::null() } else { w_neg.as_ptr() };
+        let rc = unsafe { pb200_matvec(self.raw, c.as_ptr(), count, w_mag.as_ptr(), neg, k_bits, rows, out.as_mut_ptr()) };
         if rc == PB200_OK { Ok(out) } else { Err(rc) }
     }
 }
