@@ -152,14 +152,17 @@ __device__ __forceinline__ void load_consts(int4* smem_base, const B28Dev& K) {
 
 
 // ---- engine selection: 0 = block28 (all phases on IMAD), 1 = block28t (mma.sync for phases B, C), 2 = block28u (tcgen05) ----------
+// SUPPORTED: the configuration compiles this engine (the host instantiates and launches only those)
 template <class C, int ENG> struct View {
     typedef Smem<C> type;
+    static constexpr bool SUPPORTED = true;
     static constexpr size_t BYTES = C::SMEM_BYTES;
     static constexpr int PER_SM = C::CTAS_PER_SM;
     static constexpr int LG = 1, THREADS = C::THREADS;
 };
 template <class C> struct View<C, 2> {            // block28u, one lane group per CTA
     typedef SmemU<C, 1> type;
+    static constexpr bool SUPPORTED = UL<C, 1>::SUPPORTED;
     static constexpr size_t BYTES = UL<C, 1>::SMEM_BYTES;
     static constexpr int PER_SM = UL<C, 1>::CTAS_PER_SM;
     static constexpr int LG = 1, THREADS = C::THREADS;
@@ -167,6 +170,7 @@ template <class C> struct View<C, 2> {            // block28u, one lane group pe
 template <class C> struct View<C, 4> : View<C, 2> {};      // block28u as the tally runs it: MMAs issued by thread 0 (see phases_bc_umma)
 template <class C> struct View<C, 3> {            // block28u, two lane groups (64 ciphertexts) per CTA
     typedef SmemU<C, 2> type;
+    static constexpr bool SUPPORTED = UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED;
     static constexpr size_t BYTES = UL<C, 2>::SMEM_BYTES;
     static constexpr int PER_SM = UL<C, 2>::CTAS_PER_SM;
     static constexpr int LG = 2, THREADS = 2 * C::THREADS;
@@ -1002,13 +1006,15 @@ __device__ __forceinline__ void load_value_shl(int4* buf, const u64* src, int nw
 // ---- witness engine selection: 0 = block28t arithmetic (mma.sync phases), 1 = block28u arithmetic (tcgen05 phases) ---------------
 template <class C, int WENG> struct WView {
     typedef Smem<C> type;
+    static constexpr bool SUPPORTED = true;
     static constexpr size_t BYTES = C::SMEM_W_BYTES;
-    static constexpr int PER_SM = C::CTAS_PER_SM;
+    static constexpr int PER_SM = C::CTAS_PER_SM, THREADS = C::THREADS;
 };
 template <class C> struct WView<C, 1> {
     typedef SmemU<C, 1, true> type;
+    static constexpr bool SUPPORTED = UL<C, 1, true>::SUPPORTED;
     static constexpr size_t BYTES = UL<C, 1, true>::SMEM_BYTES;
-    static constexpr int PER_SM = UL<C, 1, true>::CTAS_PER_SM;
+    static constexpr int PER_SM = UL<C, 1, true>::CTAS_PER_SM, THREADS = C::THREADS;
 };
 template <class C, int WENG, class SV>
 __device__ __forceinline__ void w_begin(SV& S, int4* smem_base, const B28Dev& K) {
@@ -1295,7 +1301,39 @@ static int window_schedule(const BigInt& e, std::vector<int2>& ops) {
     return first_idx;
 }
 
+#define CUW(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return e_; } while (0)
 #define CUK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { *cuda_err = e_; block28_destroy(key); return nullptr; } } while (0)
+
+static size_t cdiv(size_t a, size_t b) { return (a + b - 1) / b; }
+
+// The engine kernels need more dynamic shared memory than the default limit; the attribute is per device, so it is set on the
+// device of every launch (and before an occupancy query, which counts against the current limit).
+template <class V, class... P>
+static cudaError_t allow_smem(void (*kern)(P...)) {
+    return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V::BYTES);
+}
+// launch of an engine kernel: block and dynamic shared memory from its view V (View<C, ENG> or WView<C, WENG>)
+template <class V, class... P, class... A>
+static cudaError_t launch(void (*kern)(P...), size_t grid, cudaStream_t st, A... args) {
+    CUW(allow_smem<V>(kern));
+    kern<<<(unsigned)grid, V::THREADS, V::BYTES, st>>>(args...);
+    count_launch();
+    return cudaGetLastError();
+}
+
+// f(std::integral_constant<int, ENG>()) for the ENG of E, ENGS... that equals eng and that the configuration compiles
+// (V<C, ENG>::SUPPORTED); cudaErrorInvalidValue when there is none.  The list names the instantiations of one kernel family.
+template <template <class, int> class V, class C, int E, int... ENGS, class F>
+static cudaError_t with_eng(int eng, F&& f) {
+    if constexpr (V<C, E>::SUPPORTED) if (eng == E) return f(std::integral_constant<int, E>());
+    if constexpr (sizeof...(ENGS) > 0) return with_eng<V, C, ENGS...>(eng, f);
+    else return cudaErrorInvalidValue;
+}
+// The key's engine per kernel family (block28_set_engine has already fallen back to an engine the configuration compiles):
+// k_encrypt, k_pow, k_scalar run key->eng itself (0..3); the tally and the bucket kernels run tcgen05 as 4 and have no 3;
+// the witness kernels run tcgen05 (WENG 1) where the key has that variant.
+static int tally_eng(const Block28Key* key) { return key->eng >= 2 ? 4 : key->eng; }
+static int wit_eng(const Block28Key* key) { return key->has_wu && key->eng >= 2 ? 1 : 0; }
 
 template <class C>
 static Block28Key* create_cfg(const BigInt& n, const BigInt& g, uint32_t n_bits, int device, cudaStream_t st, cudaError_t* cuda_err) {
@@ -1343,17 +1381,10 @@ static Block28Key* create_cfg(const BigInt& n, const BigInt& g, uint32_t n_bits,
     if constexpr (UL<C, 1>::SUPPORTED) {
         CUK(u_image(std::integral_constant<int, 1>{}, &key->d_uconsts));
         key->has_u = true;
-        CUK((cudaFuncSetAttribute(k_encrypt<C, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));
-        CUK((cudaFuncSetAttribute(k_tally<C, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));
-        CUK((cudaFuncSetAttribute(k_pow<C, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));
-        CUK((cudaFuncSetAttribute(k_scalar<C, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));
     }
     if constexpr (UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED) {
         CUK(u_image(std::integral_constant<int, 2>{}, &key->d_uconsts2));
         key->has_u2 = true;
-        CUK((cudaFuncSetAttribute(k_encrypt<C, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 2>::SMEM_BYTES)));
-        CUK((cudaFuncSetAttribute(k_pow<C, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 2>::SMEM_BYTES)));
-        CUK((cudaFuncSetAttribute(k_scalar<C, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 2>::SMEM_BYTES)));
     }
     block28_set_engine(key, -1);
     // sliding-window schedule for the exponent n
@@ -1388,26 +1419,19 @@ static Block28Key* create_cfg(const BigInt& n, const BigInt& g, uint32_t n_bits,
     K.sms = (unsigned)key->sms;
     K.nt_top = (unsigned)BigInt::shr(Nt, (size_t)W * (C::L - 2)).bits_at(0, 32);
     // comb table
-    CUK(cudaFuncSetAttribute(k_gtable_bases<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES));
-    CUK(cudaFuncSetAttribute(k_gtable_fill<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES));
-    CUK((cudaFuncSetAttribute(k_encrypt<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
-    CUK((cudaFuncSetAttribute(k_encrypt<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
-    CUK((cudaFuncSetAttribute(k_tally<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
-    CUK((cudaFuncSetAttribute(k_tally<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
     int4* d_bases = nullptr;
+    cudaError_t e = cudaSuccess;
     if (!g_std) {      // the comb table is only needed for a general g
         CUK(cudaMalloc(&d_bases, (size_t)n_windows * C::ENTRY4 * sizeof(int4)));
-        k_gtable_bases<C><<<1, C::THREADS, C::SMEM_BYTES, st>>>(K, key->d_gwords, d_bases); count_launch();
-        k_gtable_fill<C><<<(n_windows + 31) / 32, C::THREADS, C::SMEM_BYTES, st>>>(K, d_bases, key->d_tg); count_launch();
+        e = launch<View<C, 0>>(k_gtable_bases<C>, 1, st, K, key->d_gwords, d_bases);
+        if (e == cudaSuccess) e = launch<View<C, 0>>(k_gtable_fill<C>, cdiv(n_windows, 32), st, K, d_bases, key->d_tg);
     }
-    cudaError_t e = cudaStreamSynchronize(st);
+    const cudaError_t es = cudaStreamSynchronize(st);
     if (d_bases) cudaFree(d_bases);
-    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e == cudaSuccess) e = es;
     if (e != cudaSuccess) { *cuda_err = e; block28_destroy(key); return nullptr; }
     return key;
 }
-
-#define CUW(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return e_; } while (0)
 
 template <class C>
 static cudaError_t ensure_slots(Block28Key* key, cudaStream_t st) {
@@ -1420,9 +1444,11 @@ static cudaError_t ensure_slots(Block28Key* key, cudaStream_t st) {
         CUW(cudaStreamSynchronize(st));
         cudaFree(d_n);
         int per_sm = 0;
+        CUW((allow_smem<View<C, 1>>(k_encrypt<C, 1>)));
         CUW((cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_encrypt<C, 1>, C::THREADS, C::SMEM_BYTES)));
         if constexpr (UL<C, 1>::SUPPORTED) {
             int per_u = 0;
+            CUW((allow_smem<View<C, 2>>(k_encrypt<C, 2>)));
             CUW((cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_u, k_encrypt<C, 2>, C::THREADS, UL<C, 1>::SMEM_BYTES)));
             if (per_u > per_sm) per_sm = per_u;
             if (per_sm < 2) per_sm = 2;       // a CTA of two lane groups takes two slots
@@ -1442,44 +1468,19 @@ template <class C>
 static cudaError_t encrypt_cfg(Block28Key* key, const u64* d_m, const u64* d_r, size_t count, u64* d_c, cudaStream_t st) {
     CUW(ensure_slots<C>(key, st));
     const SlotPool pool{key->d_slot_masks, key->enc_per_sm};
-    const size_t ctas = (count + 31) / 32;
-    bool done = false;
-    if constexpr (UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED) if (key->eng == 3 && key->has_u2) {
-        k_encrypt<C, 3><<<(unsigned)((count + 63) / 64), 2 * C::THREADS, UL<C, 2>::SMEM_BYTES, st>>>(key->dev, d_m, d_r, count, d_c, key->d_scratch, pool);
-        done = true;
-    }
-    if constexpr (UL<C, 1>::SUPPORTED) if (!done && key->eng >= 2 && key->has_u) {
-        k_encrypt<C, 2><<<(unsigned)ctas, C::THREADS, UL<C, 1>::SMEM_BYTES, st>>>(key->dev, d_m, d_r, count, d_c, key->d_scratch, pool);
-        done = true;
-    }
-    if (done) {}
-    else if (key->eng >= 1) k_encrypt<C, 1><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, d_m, d_r, count, d_c, key->d_scratch, pool);
-    else k_encrypt<C, 0><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, d_m, d_r, count, d_c, key->d_scratch, pool);
-    count_launch();
-    return cudaGetLastError();
+    return with_eng<View, C, 0, 1, 2, 3>(key->eng, [&](auto e) {
+        return launch<View<C, e>>(k_encrypt<C, e>, cdiv(count, 32 * View<C, e>::LG), st, key->dev, d_m, d_r, count, d_c, key->d_scratch, pool);
+    });
 }
 
 template <class C>
 static cudaError_t pow_cfg(Block28Key* key, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st) {
     CUW(ensure_slots<C>(key, st));
-    CUW((cudaFuncSetAttribute(k_pow<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
-    CUW((cudaFuncSetAttribute(k_pow<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
     const SlotPool pool{key->d_slot_masks, key->enc_per_sm};
-    const size_t ctas = (count + 31) / 32;
-    bool done = false;
-    if constexpr (UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED) if (key->eng == 3 && key->has_u2) {
-        k_pow<C, 3><<<(unsigned)((count + 63) / 64), 2 * C::THREADS, UL<C, 2>::SMEM_BYTES, st>>>(key->dev, key->pow, d_base, base_words, count, d_out, key->d_scratch, pool);
-        done = true;
-    }
-    if constexpr (UL<C, 1>::SUPPORTED) if (!done && key->eng >= 2 && key->has_u) {
-        k_pow<C, 2><<<(unsigned)ctas, C::THREADS, UL<C, 1>::SMEM_BYTES, st>>>(key->dev, key->pow, d_base, base_words, count, d_out, key->d_scratch, pool);
-        done = true;
-    }
-    if (done) {}
-    else if (key->eng >= 1) k_pow<C, 1><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, key->pow, d_base, base_words, count, d_out, key->d_scratch, pool);
-    else k_pow<C, 0><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, key->pow, d_base, base_words, count, d_out, key->d_scratch, pool);
-    count_launch();
-    return cudaGetLastError();
+    return with_eng<View, C, 0, 1, 2, 3>(key->eng, [&](auto e) {
+        return launch<View<C, e>>(k_pow<C, e>, cdiv(count, 32 * View<C, e>::LG), st, key->dev, key->pow, d_base, base_words, count, d_out,
+                                  key->d_scratch, pool);
+    });
 }
 
 // window width of the scalar chain for k_bits-bit scalars: the w <= SCALAR_MAXW with the fewest multiplications,
@@ -1496,25 +1497,11 @@ static int scalar_window(uint32_t k_bits) {
 template <class C>
 static cudaError_t scalar_cfg(Block28Key* key, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out, cudaStream_t st) {
     CUW(ensure_slots<C>(key, st));
-    CUW((cudaFuncSetAttribute(k_scalar<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
-    CUW((cudaFuncSetAttribute(k_scalar<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));
     const SlotPool pool{key->d_slot_masks, key->enc_per_sm};
     const int kw = (int)((k_bits + 63) / 64), w = scalar_window(k_bits);
-    const size_t ctas = (count + 31) / 32;
-    bool done = false;
-    if constexpr (UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED) if (key->eng == 3 && key->has_u2) {
-        k_scalar<C, 3><<<(unsigned)((count + 63) / 64), 2 * C::THREADS, UL<C, 2>::SMEM_BYTES, st>>>(key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
-        done = true;
-    }
-    if constexpr (UL<C, 1>::SUPPORTED) if (!done && key->eng >= 2 && key->has_u) {
-        k_scalar<C, 2><<<(unsigned)ctas, C::THREADS, UL<C, 1>::SMEM_BYTES, st>>>(key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
-        done = true;
-    }
-    if (done) {}
-    else if (key->eng >= 1) k_scalar<C, 1><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
-    else k_scalar<C, 0><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
-    count_launch();
-    return cudaGetLastError();
+    return with_eng<View, C, 0, 1, 2, 3>(key->eng, [&](auto e) {
+        return launch<View<C, e>>(k_scalar<C, e>, cdiv(count, 32 * View<C, e>::LG), st, key->dev, d_c, d_k, kw, w, count, d_out, key->d_scratch, pool);
+    });
 }
 
 // nodes of the CTA tree over `n` leaves: sum of ceil(n / 2^l) for l >= 1
@@ -1536,16 +1523,9 @@ static cudaError_t tally_cfg(Block28Key* key, const u64* d_c, size_t count, u64*
     TallyPeer P = key->peer;
     if (!collective || P.world <= 1) { P.world = 1; P.rank = 0; }
     else { key->peer.epoch += 1; P.epoch = key->peer.epoch; }
-    bool done = false;
-    if constexpr (UL<C, 1>::SUPPORTED) if (key->eng >= 2 && key->has_u) {
-        k_tally<C, 4><<<(unsigned)ctas, C::THREADS, UL<C, 1>::SMEM_BYTES, st>>>(key->dev, d_c, count, d_out, key->d_nodes, key->d_node_cnt, P);
-        done = true;
-    }
-    if (done) {}
-    else if (key->eng >= 1) k_tally<C, 1><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, d_c, count, d_out, key->d_nodes, key->d_node_cnt, P);
-    else k_tally<C, 0><<<(unsigned)ctas, C::THREADS, C::SMEM_BYTES, st>>>(key->dev, d_c, count, d_out, key->d_nodes, key->d_node_cnt, P);
-    count_launch();
-    return cudaGetLastError();
+    return with_eng<View, C, 0, 1, 4>(tally_eng(key), [&](auto e) {
+        return launch<View<C, e>>(k_tally<C, e>, ctas, st, key->dev, d_c, count, d_out, key->d_nodes, key->d_node_cnt, P);
+    });
 }
 
 
@@ -1590,9 +1570,6 @@ static cudaError_t witness_prepare_cfg(Block28Key* key, u64* d_gchain, bool gcha
     WitDev& Wd = key->wit;
     Wd.gtab = key->d_gtab; Wd.one_s = key->d_one_s; Wd.cpow = key->d_cpow; Wd.n_words = key->d_nwords;
     Wd.exp_bits = (int)n.bits(); Wd.sh = sh; Wd.inv = 1048576.0 / topd;
-    CUW((cudaFuncSetAttribute(k_witness<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_W_BYTES)));
-    CUW((cudaFuncSetAttribute(k_gchain_w<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_W_BYTES)));
-    CUW((cudaFuncSetAttribute(k_add_w<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_W_BYTES)));
     if constexpr (UL<C, 1, true>::SUPPORTED) {
         // the same step on the tcgen05 phases: constants of the witness modulus + their Toeplitz core-matrix tables
         typedef UL<C, 1, true> U;
@@ -1608,22 +1585,16 @@ static cudaError_t witness_prepare_cfg(Block28Key* key, u64* d_gchain, bool gcha
         CUW(cudaStreamSynchronize(st));
         key->wdev.uconsts = key->d_wuconsts;
         key->has_wu = !getenv("PB200_NO_UMMA_WITNESS");
-        CUW((cudaFuncSetAttribute(k_witness<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)U::SMEM_BYTES)));
-        CUW((cudaFuncSetAttribute(k_gchain_w<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)U::SMEM_BYTES)));
-        CUW((cudaFuncSetAttribute(k_add_w<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)U::SMEM_BYTES)));
     }
     if (gchain_ready) {        // g-chain records already produced (simple64): only convert them into table entries
         k_wtab<C><<<(key->n_bits + 63) / 64, 64, 0, st>>>(key->d_gwords, wi, d_gchain, wo, (int)key->n_bits, sh / 2, key->d_gtab);
+        count_launch();
+        CUW(cudaGetLastError());
     } else {                   // produce records and table entries with the witness engine itself
-        bool done = false;
-        if constexpr (UL<C, 1, true>::SUPPORTED) if (key->has_wu && key->eng >= 2) {
-            k_gchain_w<C, 1><<<1, C::THREADS, UL<C, 1, true>::SMEM_BYTES, st>>>(key->wdev, key->wit, key->d_gwords, (int)key->n_bits, d_gchain, key->d_gtab);
-            done = true;
-        }
-        if (!done) k_gchain_w<C, 0><<<1, C::THREADS, C::SMEM_W_BYTES, st>>>(key->wdev, key->wit, key->d_gwords, (int)key->n_bits, d_gchain, key->d_gtab);
+        CUW((with_eng<WView, C, 0, 1>(wit_eng(key), [&](auto e) {
+            return launch<WView<C, e>>(k_gchain_w<C, e>, 1, st, key->wdev, key->wit, key->d_gwords, (int)key->n_bits, d_gchain, key->d_gtab);
+        })));
     }
-    count_launch();
-    CUW(cudaGetLastError());
     CUW(cudaStreamSynchronize(st));                        // the staging vectors above go out of scope
     key->wit_ready = true;
     return cudaSuccess;
@@ -1642,14 +1613,7 @@ static cudaError_t witness_cfg(Block28Key* key, const u64* d_m, const u64* d_r, 
     WitIO A;
     A.m = d_m; A.r = d_r; A.count = count; A.c_out = d_c; A.records = d_records; A.offsets = d_offsets; A.digest = d_digest;
     A.scratch = key->d_wscratch;
-    bool done = false;
-    if constexpr (UL<C, 1, true>::SUPPORTED) if (key->has_wu && key->eng >= 2) {
-        k_witness<C, 1><<<(unsigned)ctas, C::THREADS, UL<C, 1, true>::SMEM_BYTES, st>>>(key->wdev, key->wit, A);
-        done = true;
-    }
-    if (!done) k_witness<C, 0><<<(unsigned)ctas, C::THREADS, C::SMEM_W_BYTES, st>>>(key->wdev, key->wit, A);
-    count_launch();
-    return cudaGetLastError();
+    return with_eng<WView, C, 0, 1>(wit_eng(key), [&](auto e) { return launch<WView<C, e>>(k_witness<C, e>, ctas, st, key->wdev, key->wit, A); });
 }
 
 // Compiled configurations <G warps, BL digits per block>: L = G*BL digits of 28 bits; n^2 must fit KN - 2 bits.
@@ -1660,6 +1624,20 @@ typedef Cfg<16, 19> Cfg4096;   // L = 304: n^2 up to 8486 bits (|n| <= 4096)
 
 template <class C>
 static bool covers(uint32_t n_bits) { return 2 * (size_t)n_bits <= (size_t)C::KN - 2 && n_bits % 8 == 0; }
+
+template <class... Cs> struct CfgList {
+    // (G, BL) of the first configuration that covers a key of n_bits; false when none does
+    static bool shape(uint32_t n_bits, int* G, int* BL) { return ((covers<Cs>(n_bits) ? (*G = Cs::G, *BL = Cs::BL, true) : false) || ...); }
+    // f(C()) for the configuration C of shape (G, BL) (a value of the configuration type as its tag): f's result, `none` when no
+    // configuration has that shape
+    template <class R, class F> static R with(int G, int BL, R none, F&& f) {
+        (void)((G == Cs::G && BL == Cs::BL ? (none = f(Cs()), true) : false) || ...);
+        return none;
+    }
+};
+typedef CfgList<Cfg1024, Cfg2048, Cfg3072, Cfg4096> Configs;      // in the order a key size picks them
+// f(C()) for the key's configuration C
+template <class F> static cudaError_t with_cfg(const Block28Key* key, F&& f) { return Configs::with(key->G, key->BL, cudaErrorInvalidValue, f); }
 
 // layout constants of a block28u variant (host only, no device needed): the CPU model of the tcgen05 data path in
 // tests/test_umma_layout.py checks its own derivation against these
@@ -1679,22 +1657,18 @@ static bool ul_cfg(int lg, int wit, int* out) {
     return true;
 }
 bool block28_umma_layout(int G, int BL, int lg, int wit, int* out) {
-    if (G == 4 && BL == 19) return ul_cfg<Cfg1024>(lg, wit, out);
-    if (G == 8 && BL == 19) return ul_cfg<Cfg2048>(lg, wit, out);
-    if (G == 16 && BL == 14) return ul_cfg<Cfg3072>(lg, wit, out);
-    if (G == 16 && BL == 19) return ul_cfg<Cfg4096>(lg, wit, out);
-    return false;
+    return Configs::with(G, BL, false, [&](auto c) { return ul_cfg<decltype(c)>(lg, wit, out); });
 }
 
 Block28Key* block28_create(const BigInt& n, const BigInt& g, uint32_t n_bits, int device, cudaStream_t st,
                            std::string* why, cudaError_t* cuda_err) {
     *cuda_err = cudaSuccess;
-    if (covers<Cfg1024>(n_bits)) return create_cfg<Cfg1024>(n, g, n_bits, device, st, cuda_err);
-    if (covers<Cfg2048>(n_bits)) return create_cfg<Cfg2048>(n, g, n_bits, device, st, cuda_err);
-    if (covers<Cfg3072>(n_bits)) return create_cfg<Cfg3072>(n, g, n_bits, device, st, cuda_err);
-    if (covers<Cfg4096>(n_bits)) return create_cfg<Cfg4096>(n, g, n_bits, device, st, cuda_err);
-    if (why) *why = "block28: no compiled configuration covers this key size";
-    return nullptr;
+    int G = 0, BL = 0;
+    if (!Configs::shape(n_bits, &G, &BL)) {
+        if (why) *why = "block28: no compiled configuration covers this key size";
+        return nullptr;
+    }
+    return Configs::with(G, BL, (Block28Key*)nullptr, [&](auto c) { return create_cfg<decltype(c)>(n, g, n_bits, device, st, cuda_err); });
 }
 void block28_destroy(Block28Key* key) {
     if (!key) return;
@@ -1733,14 +1707,10 @@ int block28_set_engine(Block28Key* key, int eng) {
                 std::to_string(key->BL) + ">";
     return eng;
 }
-bool block28_has_umma(const Block28Key* key) { return key->has_u; }
-bool block28_has_umma2(const Block28Key* key) { return key->has_u2; }
+bool block28_has_engine(const Block28Key* key, int eng) { return eng == 0 || eng == 1 || (eng == 2 && key->has_u) || (eng == 3 && key->has_u2); }
 void block28_chain_counts(const Block28Key* key, uint64_t* n_sqr, uint64_t* n_mul) { *n_sqr = key->n_sqr; *n_mul = key->n_mul; }
 cudaError_t block28_encrypt(Block28Key* key, const u64* d_m, const u64* d_r, size_t count, u64* d_c, cudaStream_t st) {
-    if (key->G == 4) return encrypt_cfg<Cfg1024>(key, d_m, d_r, count, d_c, st);
-    if (key->G == 8) return encrypt_cfg<Cfg2048>(key, d_m, d_r, count, d_c, st);
-    if (key->BL == 14) return encrypt_cfg<Cfg3072>(key, d_m, d_r, count, d_c, st);
-    return encrypt_cfg<Cfg4096>(key, d_m, d_r, count, d_c, st);
+    return with_cfg(key, [&](auto c) { return encrypt_cfg<decltype(c)>(key, d_m, d_r, count, d_c, st); });
 }
 cudaError_t block28_pow_prepare(Block28Key* key, const BigInt& e, cudaStream_t st) {
     std::vector<int2> ops;
@@ -1756,32 +1726,20 @@ cudaError_t block28_pow_prepare(Block28Key* key, const BigInt& e, cudaStream_t s
 cudaError_t block28_pow(Block28Key* key, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st) {
     if (!count) return cudaSuccess;
     if (!key->pow_ready) return cudaErrorInvalidValue;
-    if (key->G == 4) return pow_cfg<Cfg1024>(key, d_base, base_words, count, d_out, st);
-    if (key->G == 8) return pow_cfg<Cfg2048>(key, d_base, base_words, count, d_out, st);
-    if (key->BL == 14) return pow_cfg<Cfg3072>(key, d_base, base_words, count, d_out, st);
-    return pow_cfg<Cfg4096>(key, d_base, base_words, count, d_out, st);
+    return with_cfg(key, [&](auto c) { return pow_cfg<decltype(c)>(key, d_base, base_words, count, d_out, st); });
 }
 cudaError_t block28_scalar(Block28Key* key, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out, cudaStream_t st) {
     if (!count) return cudaSuccess;
     if (k_bits == 0) return cudaErrorInvalidValue;
-    if (key->G == 4) return scalar_cfg<Cfg1024>(key, d_c, d_k, k_bits, count, d_out, st);
-    if (key->G == 8) return scalar_cfg<Cfg2048>(key, d_c, d_k, k_bits, count, d_out, st);
-    if (key->BL == 14) return scalar_cfg<Cfg3072>(key, d_c, d_k, k_bits, count, d_out, st);
-    return scalar_cfg<Cfg4096>(key, d_c, d_k, k_bits, count, d_out, st);
+    return with_cfg(key, [&](auto c) { return scalar_cfg<decltype(c)>(key, d_c, d_k, k_bits, count, d_out, st); });
 }
 
-static cudaError_t tally_dispatch(Block28Key* key, const u64* d_c, size_t count, u64* d_out, bool collective, cudaStream_t st) {
-    if (key->G == 4) return tally_cfg<Cfg1024>(key, d_c, count, d_out, collective, st);
-    if (key->G == 8) return tally_cfg<Cfg2048>(key, d_c, count, d_out, collective, st);
-    if (key->BL == 14) return tally_cfg<Cfg3072>(key, d_c, count, d_out, collective, st);
-    return tally_cfg<Cfg4096>(key, d_c, count, d_out, collective, st);
-}
 cudaError_t block28_tally(Block28Key* key, const u64* d_c, size_t count, u64* d_out, cudaStream_t st) {
-    return tally_dispatch(key, d_c, count, d_out, false, st);
+    return with_cfg(key, [&](auto c) { return tally_cfg<decltype(c)>(key, d_c, count, d_out, false, st); });
 }
 // collective over the connected peer group: every rank calls it once per tally, in the same order
 cudaError_t block28_tally_peer(Block28Key* key, const u64* d_c, size_t count, u64* d_out, cudaStream_t st) {
-    return tally_dispatch(key, d_c, count, d_out, true, st);
+    return with_cfg(key, [&](auto c) { return tally_cfg<decltype(c)>(key, d_c, count, d_out, true, st); });
 }
 int block28_peer_world(const Block28Key* key) { return key->peer.world; }
 
@@ -1813,13 +1771,6 @@ cudaError_t block28_tally_peer_connect(Block28Key* key, int rank, int world, u64
 }
 
 
-template <class C, int ENG>
-static cudaError_t debug_launch(Block28Key* key, const int4* d_v, const int4* d_y, int reps, int4* d_vout, int4* d_t, unsigned* d_rows, cudaStream_t st) {
-    CUW((cudaFuncSetAttribute(k_mulmod_dbg<C, ENG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)View<C, ENG>::BYTES)));
-    k_mulmod_dbg<C, ENG><<<1, View<C, ENG>::THREADS, View<C, ENG>::BYTES, st>>>(key->dev, d_v, d_y, reps, d_vout, d_t, d_rows);
-    count_launch();
-    return cudaGetLastError();
-}
 template <class C>
 static cudaError_t debug_cfg(Block28Key* key, int eng, const int* h_v, const int* h_y, int reps, int* h_vout, int* h_t, unsigned* h_rows, cudaStream_t st) {
     const size_t vb = (size_t)C::VAL4 * 16;
@@ -1831,12 +1782,9 @@ static cudaError_t debug_cfg(Block28Key* key, int eng, const int* h_v, const int
         CUW(cudaMemset(d_rows, 0, (size_t)32 * C::L * 4));
         CUW(cudaMemcpy(d_v, h_v, vb, cudaMemcpyHostToDevice));
         if (h_y) CUW(cudaMemcpy(d_y, h_y, vb, cudaMemcpyHostToDevice));
-        cudaError_t r = cudaErrorInvalidValue;
-        if (eng == 3) { if constexpr (UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED) { if (key->has_u2) r = debug_launch<C, 3>(key, d_v, h_y ? d_y : nullptr, reps, d_vout, h_t ? d_t : nullptr, d_rows, st); } }
-        else if (eng == 2) { if constexpr (UL<C, 1>::SUPPORTED) { if (key->has_u) r = debug_launch<C, 2>(key, d_v, h_y ? d_y : nullptr, reps, d_vout, h_t ? d_t : nullptr, d_rows, st); } }
-        else if (eng == 1) r = debug_launch<C, 1>(key, d_v, h_y ? d_y : nullptr, reps, d_vout, h_t ? d_t : nullptr, d_rows, st);
-        else if (eng == 0) r = debug_launch<C, 0>(key, d_v, h_y ? d_y : nullptr, reps, d_vout, h_t ? d_t : nullptr, d_rows, st);
-        CUW(r);
+        CUW((with_eng<View, C, 0, 1, 2, 3>(eng, [&](auto e) {
+            return launch<View<C, e>>(k_mulmod_dbg<C, e>, 1, st, key->dev, d_v, h_y ? d_y : nullptr, reps, d_vout, h_t ? d_t : nullptr, d_rows);
+        })));
         CUW(cudaStreamSynchronize(st));
         if (h_t) CUW(cudaMemcpy(h_t, d_t, 2 * vb, cudaMemcpyDeviceToHost));
         else {
@@ -1852,36 +1800,24 @@ static cudaError_t debug_cfg(Block28Key* key, int eng, const int* h_v, const int
 // eng: 0 block28, 1 block28t, 2 block28u.  h_t non-null: phase A only, the 2L-digit product; else `reps` multiplications, V and q-hat rows
 cudaError_t block28_debug_mulmod(Block28Key* key, int eng, const int* h_v, const int* h_y, int reps, int* h_vout, int* h_t, unsigned* h_rows,
                                  cudaStream_t st) {
-    if (key->G == 4) return debug_cfg<Cfg1024>(key, eng, h_v, h_y, reps, h_vout, h_t, h_rows, st);
-    if (key->G == 8) return debug_cfg<Cfg2048>(key, eng, h_v, h_y, reps, h_vout, h_t, h_rows, st);
-    if (key->BL == 14) return debug_cfg<Cfg3072>(key, eng, h_v, h_y, reps, h_vout, h_t, h_rows, st);
-    return debug_cfg<Cfg4096>(key, eng, h_v, h_y, reps, h_vout, h_t, h_rows, st);
+    return with_cfg(key, [&](auto c) { return debug_cfg<decltype(c)>(key, eng, h_v, h_y, reps, h_vout, h_t, h_rows, st); });
 }
 void block28_shape(const Block28Key* key, int* G, int* BL) { *G = key->G; *BL = key->BL; }
 
 
-template <class C, int ENG>
-static cudaError_t time_launch(Block28Key* key, const int4* d_v, int ctas, int reps, int stagger, long long* d_cyc, unsigned* d_cnt, cudaStream_t st) {
-    CUW((cudaFuncSetAttribute(k_mulmod_time<C, ENG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)View<C, ENG>::BYTES)));
-    k_mulmod_time<C, ENG><<<ctas, View<C, ENG>::THREADS, View<C, ENG>::BYTES, st>>>(key->dev, d_v, reps, stagger, d_cyc, d_cnt);
-    count_launch();
-    return cudaGetLastError();
-}
-// eng 1 / 2; h_cyc: 3 * ctas values
+// eng 1 / 2 / 3; h_cyc: 3 * ctas values
 cudaError_t block28_debug_time(Block28Key* key, int eng, const int* h_v, int ctas, int reps, int stagger, long long* h_cyc, cudaStream_t st) {
-    if (key->G != 8) return cudaErrorInvalidValue;
     typedef Cfg2048 C;
+    if (key->G != C::G || key->BL != C::BL) return cudaErrorInvalidValue;
     const size_t vb = (size_t)C::VAL4 * 16;
     int4* d_v = nullptr; long long* d_cyc = nullptr; unsigned* d_cnt = nullptr;
     auto run = [&]() -> cudaError_t {
         CUW(cudaMalloc(&d_v, vb)); CUW(cudaMalloc(&d_cyc, (size_t)ctas * 3 * sizeof(long long)));
         CUW(cudaMalloc(&d_cnt, 1024 * sizeof(unsigned))); CUW(cudaMemset(d_cnt, 0, 1024 * sizeof(unsigned)));
         CUW(cudaMemcpy(d_v, h_v, vb, cudaMemcpyHostToDevice));
-        cudaError_t r = cudaErrorInvalidValue;
-        if (eng == 3) { if (key->has_u2) r = time_launch<C, 3>(key, d_v, ctas, reps, stagger, d_cyc, d_cnt, st); }
-        else if (eng == 2) { if (key->has_u) r = time_launch<C, 2>(key, d_v, ctas, reps, stagger, d_cyc, d_cnt, st); }
-        else if (eng == 1) r = time_launch<C, 1>(key, d_v, ctas, reps, stagger, d_cyc, d_cnt, st);
-        CUW(r);
+        CUW((with_eng<View, C, 1, 2, 3>(eng, [&](auto e) {
+            return launch<View<C, e>>(k_mulmod_time<C, e>, ctas, st, key->dev, d_v, reps, stagger, d_cyc, d_cnt);
+        })));
         CUW(cudaStreamSynchronize(st));
         CUW(cudaMemcpy(h_cyc, d_cyc, (size_t)ctas * 3 * sizeof(long long), cudaMemcpyDeviceToHost));
         return cudaSuccess;
@@ -1896,14 +1832,9 @@ static cudaError_t add_cfg(Block28Key* key, const u64* d_c1, const u64* d_c2, in
                            int* d_flags, cudaStream_t st) {
     size_t ctas = (count + 31) / 32, cap = (size_t)C::CTAS_PER_SM * key->sms;
     if (ctas > cap) ctas = cap;
-    bool done = false;
-    if constexpr (UL<C, 1, true>::SUPPORTED) if (key->has_wu && key->eng >= 2) {
-        k_add_w<C, 1><<<(unsigned)ctas, C::THREADS, UL<C, 1, true>::SMEM_BYTES, st>>>(key->wdev, key->wit, d_c1, d_c2, c_words, count, d_out, d_q, d_flags);
-        done = true;
-    }
-    if (!done) k_add_w<C, 0><<<(unsigned)ctas, C::THREADS, C::SMEM_W_BYTES, st>>>(key->wdev, key->wit, d_c1, d_c2, c_words, count, d_out, d_q, d_flags);
-    count_launch();
-    return cudaGetLastError();
+    return with_eng<WView, C, 0, 1>(wit_eng(key), [&](auto e) {
+        return launch<WView<C, e>>(k_add_w<C, e>, ctas, st, key->wdev, key->wit, d_c1, d_c2, c_words, count, d_out, d_q, d_flags);
+    });
 }
 
 // The witness engine needs canonical chain values below n^2 from the first step on: n must fill its declared width
@@ -1912,32 +1843,22 @@ bool block28_witness_supported(const Block28Key* key) { return key->eng >= 1 && 
 cudaError_t block28_witness_prepare(Block28Key* key, u64* d_gchain, bool gchain_ready, cudaStream_t st) {
     if (key->wit_ready) return cudaSuccess;
     try {
-        if (key->G == 4) return witness_prepare_cfg<Cfg1024>(key, d_gchain, gchain_ready, st);
-        if (key->G == 8) return witness_prepare_cfg<Cfg2048>(key, d_gchain, gchain_ready, st);
-        if (key->BL == 14) return witness_prepare_cfg<Cfg3072>(key, d_gchain, gchain_ready, st);
-        return witness_prepare_cfg<Cfg4096>(key, d_gchain, gchain_ready, st);
+        return with_cfg(key, [&](auto c) { return witness_prepare_cfg<decltype(c)>(key, d_gchain, gchain_ready, st); });
     } catch (const std::exception&) { return cudaErrorInvalidValue; }
 }
 cudaError_t block28_witness(Block28Key* key, const u64* d_m, const u64* d_r, size_t count, u64* d_c, u64* d_records,
                             const u64* d_offsets, u64* d_digest, cudaStream_t st) {
     if (!count) return cudaSuccess;
-    if (key->G == 4) return witness_cfg<Cfg1024>(key, d_m, d_r, count, d_c, d_records, d_offsets, d_digest, st);
-    if (key->G == 8) return witness_cfg<Cfg2048>(key, d_m, d_r, count, d_c, d_records, d_offsets, d_digest, st);
-    if (key->BL == 14) return witness_cfg<Cfg3072>(key, d_m, d_r, count, d_c, d_records, d_offsets, d_digest, st);
-    return witness_cfg<Cfg4096>(key, d_m, d_r, count, d_c, d_records, d_offsets, d_digest, st);
+    return with_cfg(key, [&](auto c) { return witness_cfg<decltype(c)>(key, d_m, d_r, count, d_c, d_records, d_offsets, d_digest, st); });
 }
 
 cudaError_t block28_add(Block28Key* key, const u64* d_c1, const u64* d_c2, int c_words, size_t count, u64* d_out, u64* d_q,
                         int* d_flags, cudaStream_t st) {
     if (!count) return cudaSuccess;
-    if (key->G == 4) return add_cfg<Cfg1024>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st);
-    if (key->G == 8) return add_cfg<Cfg2048>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st);
-    if (key->BL == 14) return add_cfg<Cfg3072>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st);
-    return add_cfg<Cfg4096>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st);
+    return with_cfg(key, [&](auto c) { return add_cfg<decltype(c)>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st); });
 }
 
 // ---- matvec: planner and driver (DESIGN.md §9b) ---------------------------------------------------------------------------------
-static size_t cdiv(size_t a, size_t b) { return (a + b - 1) / b; }
 // multiplications of k_scalar's chain for k_bits-bit scalars (table, windows, finalize)
 static uint64_t scalar_chain(uint32_t k_bits) {
     const int w = scalar_window(k_bits);
@@ -1964,11 +1885,9 @@ static MvShape mv_shape_cfg(uint32_t n_bits, int sms) {
     return s;
 }
 static MvShape mv_shape(uint32_t n_bits, int sms) {
-    if (covers<Cfg1024>(n_bits)) return mv_shape_cfg<Cfg1024>(n_bits, sms);
-    if (covers<Cfg2048>(n_bits)) return mv_shape_cfg<Cfg2048>(n_bits, sms);
-    if (covers<Cfg3072>(n_bits)) return mv_shape_cfg<Cfg3072>(n_bits, sms);
-    if (covers<Cfg4096>(n_bits)) return mv_shape_cfg<Cfg4096>(n_bits, sms);
-    return MvShape();
+    int G = 0, BL = 0;
+    Configs::shape(n_bits, &G, &BL);
+    return Configs::with(G, BL, MvShape(), [&](auto c) { return mv_shape_cfg<decltype(c)>(n_bits, sms); });
 }
 
 // the bucket method's arena, carved in this order (every piece 256-byte aligned)
@@ -2065,46 +1984,37 @@ MatvecPlan matvec_plan(uint32_t n_bits, int sms, size_t rows, size_t count, uint
     return best_slots < slots_chain ? best : ch;
 }
 
-#define MV_LAUNCH(KERN, grid, ...) do {                                                                                             \
-    if (eng == 4) { if constexpr (UL<C, 1>::SUPPORTED) {                                                                            \
-        CUW((cudaFuncSetAttribute(KERN<C, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UL<C, 1>::SMEM_BYTES)));           \
-        KERN<C, 4><<<(unsigned)(grid), C::THREADS, UL<C, 1>::SMEM_BYTES, st>>>(__VA_ARGS__); } }                                     \
-    else if (eng == 1) {                                                                                                             \
-        CUW((cudaFuncSetAttribute(KERN<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));                  \
-        KERN<C, 1><<<(unsigned)(grid), C::THREADS, C::SMEM_BYTES, st>>>(__VA_ARGS__); }                                              \
-    else {                                                                                                                           \
-        CUW((cudaFuncSetAttribute(KERN<C, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES)));                  \
-        KERN<C, 0><<<(unsigned)(grid), C::THREADS, C::SMEM_BYTES, st>>>(__VA_ARGS__); }                                              \
-    count_launch(); CUW(cudaGetLastError()); } while (0)
-
 // k_bucket_fold over an entry list, level after level until the carry list is empty.  n_dev: the entry count is *cnt (device);
 // else n_ub exactly.  Level l reads its count from cnt[l] and writes the next one to cnt[l + 1].
-template <class C>
-static cudaError_t mv_fold(Block28Key* key, int eng, const unsigned* keys, const unsigned* idx, const u64* src, bool n_dev, size_t n_ub,
+template <class C, int ENG>
+static cudaError_t mv_fold(Block28Key* key, const unsigned* keys, const unsigned* idx, const u64* src, bool n_dev, size_t n_ub,
                            int4* out, const MvLayout& L, unsigned char* A, size_t lanes, cudaStream_t st) {
+    typedef View<C, ENG> V;
     unsigned* cnt = (unsigned*)(A + L.cnt);
     int lv = 0, ls = fold_ls(n_ub, lanes);
     size_t ln = cdiv(n_ub, (size_t)ls);
-    MV_LAUNCH(k_bucket_fold, cdiv(ln, 32), key->dev, keys, idx, src, key->dev.words_out, (const int4*)nullptr, n_dev ? cnt : nullptr, n_ub, ls,
-              out, (unsigned*)(A + L.ckeys[0]), (int4*)(A + L.cvals[0]), cnt + 1);
+    CUW(launch<V>(k_bucket_fold<C, ENG>, cdiv(ln, 32), st, key->dev, keys, idx, src, key->dev.words_out, (const int4*)nullptr,
+                      n_dev ? cnt : nullptr, n_ub, ls, out, (unsigned*)(A + L.ckeys[0]), (int4*)(A + L.cvals[0]), cnt + 1));
     while (ln > 1) {
         const size_t n = 2 * ln;
         ls = fold_ls(n, lanes); ln = cdiv(n, (size_t)ls); lv++;
         const int i = (lv - 1) & 1;
-        MV_LAUNCH(k_bucket_fold, cdiv(ln, 32), key->dev, (const unsigned*)(A + L.ckeys[i]), (const unsigned*)nullptr, (const u64*)nullptr, 0,
-                  (const int4*)(A + L.cvals[i]), cnt + lv, n, ls, out, (unsigned*)(A + L.ckeys[i ^ 1]), (int4*)(A + L.cvals[i ^ 1]), cnt + lv + 1);
+        CUW(launch<V>(k_bucket_fold<C, ENG>, cdiv(ln, 32), st, key->dev, (const unsigned*)(A + L.ckeys[i]), (const unsigned*)nullptr,
+                      (const u64*)nullptr, 0, (const int4*)(A + L.cvals[i]), cnt + lv, n, ls, out, (unsigned*)(A + L.ckeys[i ^ 1]),
+                      (int4*)(A + L.cvals[i ^ 1]), cnt + lv + 1));
         if (lv >= 62) return cudaErrorInvalidValue;
     }
     return cudaSuccess;
 }
 
-template <class C>
+// ENG: the key's engine as the bucket kernels run it (tally_eng); k_scalar runs the key's own engine
+template <class C, int ENG>
 static cudaError_t matvec_cfg(Block28Key* key, const MatvecPlan& P, const u64* d_c, size_t count, const u64* d_w, uint32_t k_bits,
                               const uint8_t* d_neg, size_t rows, u64* d_out, unsigned char* A, const u64* d_nm1, cudaStream_t st) {
+    typedef View<C, ENG> V;
     CUW(ensure_slots<C>(key, st));
     const MvShape S = mv_shape_cfg<C>(key->n_bits, key->sms);
     const MvLayout L = mv_layout(P, S);
-    const int eng = key->eng >= 2 && key->has_u ? 4 : key->eng;
     const int c = P.c, kw = (int)((k_bits + 63) / 64), wo = key->dev.words_out;
     const size_t vb = (size_t)wo;                                   // u64 per canonical value
     u64* vals = (u64*)(A + L.vals); u64* x = (u64*)(A + L.x);
@@ -2127,19 +2037,19 @@ static cudaError_t matvec_cfg(Block28Key* key, const MatvecPlan& P, const u64* d
                 k_mv_one_lazy<<<(unsigned)cdiv(nkeys * C::ENTRY4, 256), 256, 0, st>>>((int4*)(A + L.buckets), nkeys, C::ENTRY4);
                 count_launch(4);
                 CUW(cudaGetLastError());
-                CUW(mv_fold<C>(key, eng, (const unsigned*)(A + L.keys), (const unsigned*)(A + L.idx), d_c + i0 * wo, true, rb * jg * nc,
-                               (int4*)(A + L.buckets), L, A, S.lanes, st));
-                MV_LAUNCH(k_bucket_reduce, cdiv(units, 32), key->dev, (const int4*)(A + L.buckets), c, P.nseg, P.lseg, units, vals,
-                          (u64*)(A + L.aseg), (u64*)(A + L.scal), (int4*)(A + L.rscr));
+                CUW((mv_fold<C, ENG>(key, (const unsigned*)(A + L.keys), (const unsigned*)(A + L.idx), d_c + i0 * wo, true, rb * jg * nc,
+                                     (int4*)(A + L.buckets), L, A, S.lanes, st)));
+                CUW(launch<V>(k_bucket_reduce<C, ENG>, cdiv(units, 32), st, key->dev, (const int4*)(A + L.buckets), c, P.nseg, P.lseg, units, vals,
+                              (u64*)(A + L.aseg), (u64*)(A + L.scal), (int4*)(A + L.rscr)));
                 CUW(scalar_cfg<C>(key, (const u64*)(A + L.aseg), (const u64*)(A + L.scal), (uint32_t)c, units, vals + units * vb, st));
                 const int per = 2 * P.nseg + 1;
                 k_mv_block_entries<<<(unsigned)cdiv(sp * per, 256), 256, 0, st>>>((unsigned*)(A + L.skeys), (unsigned*)(A + L.sidx), sp, P.nseg, per);
                 count_launch(); CUW(cudaGetLastError());
-                CUW(mv_fold<C>(key, eng, (const unsigned*)(A + L.skeys), (const unsigned*)(A + L.sidx), vals, false, sp * per,
-                               (int4*)(A + L.wlazy), L, A, S.lanes, st));
-                MV_LAUNCH(k_lazy_canon, cdiv(sp, 32), key->dev, (const int4*)(A + L.wlazy), sp, w_acc);
+                CUW((mv_fold<C, ENG>(key, (const unsigned*)(A + L.skeys), (const unsigned*)(A + L.sidx), vals, false, sp * per,
+                                     (int4*)(A + L.wlazy), L, A, S.lanes, st)));
+                CUW(launch<V>(k_lazy_canon<C, ENG>, cdiv(sp, 32), st, key->dev, (const int4*)(A + L.wlazy), sp, w_acc));
             }
-            MV_LAUNCH(k_horner, cdiv(xs, 32), key->dev, x, (const u64*)w_acc, xs, jg, c);
+            CUW(launch<V>(k_horner<C, ENG>, cdiv(xs, 32), st, key->dev, x, (const u64*)w_acc, xs, jg, c));
         }
         u64* out = d_out + r0 * vb;
         if (P.nsign == 1) { CUW(cudaMemcpyAsync(out, x, rb * vb * 8, cudaMemcpyDeviceToDevice, st)); continue; }
@@ -2149,22 +2059,23 @@ static cudaError_t matvec_cfg(Block28Key* key, const MatvecPlan& P, const u64* d
         CUW(cudaMemcpyAsync(x + rb * vb, np, rb * vb * 8, cudaMemcpyDeviceToDevice, st));
         k_mv_block_entries<<<(unsigned)cdiv(2 * rb, 256), 256, 0, st>>>((unsigned*)(A + L.skeys), (unsigned*)(A + L.sidx), rb, 1, 2);
         count_launch(); CUW(cudaGetLastError());
-        CUW(mv_fold<C>(key, eng, (const unsigned*)(A + L.skeys), (const unsigned*)(A + L.sidx), x, false, 2 * rb, (int4*)(A + L.wlazy), L, A,
-                       S.lanes, st));
-        MV_LAUNCH(k_lazy_canon, cdiv(rb, 32), key->dev, (const int4*)(A + L.wlazy), rb, out);
+        CUW((mv_fold<C, ENG>(key, (const unsigned*)(A + L.skeys), (const unsigned*)(A + L.sidx), x, false, 2 * rb, (int4*)(A + L.wlazy), L, A,
+                             S.lanes, st)));
+        CUW(launch<V>(k_lazy_canon<C, ENG>, cdiv(rb, 32), st, key->dev, (const int4*)(A + L.wlazy), rb, out));
     }
     return cudaSuccess;
 }
-#undef MV_LAUNCH
 
 cudaError_t block28_matvec(Block28Key* key, const MatvecPlan& P, const u64* d_c, size_t count, const u64* d_w, uint32_t k_bits, const uint8_t* d_neg,
                            size_t rows, u64* d_out, void* arena, const u64* d_nm1, cudaStream_t st) {
     if (!rows || !count || P.method != 1) return cudaErrorInvalidValue;
     unsigned char* A = (unsigned char*)arena;
-    if (key->G == 4) return matvec_cfg<Cfg1024>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
-    if (key->G == 8) return matvec_cfg<Cfg2048>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
-    if (key->BL == 14) return matvec_cfg<Cfg3072>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
-    return matvec_cfg<Cfg4096>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
+    return with_cfg(key, [&](auto c) {
+        typedef decltype(c) C;
+        return with_eng<View, C, 0, 1, 4>(tally_eng(key), [&](auto e) {
+            return matvec_cfg<C, e>(key, P, d_c, count, d_w, k_bits, d_neg, rows, d_out, A, d_nm1, st);
+        });
+    });
 }
 cudaError_t matvec_mask(const u64* d_w, const uint8_t* d_neg, size_t n, int kw, int sgn, u64* d_out, cudaStream_t st) {
     if (!n) return cudaSuccess;

@@ -217,14 +217,18 @@ const char* pb200_key_engine(const pb200_key* k) {
     if (!k) return "";
     return use_fast(k) ? k->engine_name.c_str() : "simple64";
 }
+// internal numbering of the block28 family: 0 block28, 1 block28t, 2 block28u (32 ciphertexts per CTA), 3 block28u2 (64).
+// *eng <- the internal number of public engine 2..5; false when the key has no block28 engine or its configuration lacks that one.
+static bool fast_engine(const pb200_key* k, int engine, int* eng) {
+    *eng = engine - 2;
+    return k->fast && block28_has_engine(k->fast, *eng);
+}
 int pb200_key_set_engine(pb200_key* k, int engine) try {
     if (!k || engine < 0 || engine > 5) return PB200_ERR_INVALID_ARG;
-    if (engine >= 2 && !k->fast) return PB200_ERR_UNSUPPORTED;
-    if (engine == 4 && !block28_has_umma(k->fast)) return PB200_ERR_UNSUPPORTED;
-    if (engine == 5 && !block28_has_umma2(k->fast)) return PB200_ERR_UNSUPPORTED;
+    int eng = -1;                   // 0 (automatic) and 1 (simple64) leave the fastest block28 engine selected on the key
+    if (engine >= 2 && !fast_engine(k, engine, &eng)) return PB200_ERR_UNSUPPORTED;
     k->engine = engine;
-    // internal numbering of the block28 family: 0 block28, 1 block28t, 2 block28u (32 ciphertexts per CTA), 3 block28u2 (64)
-    if (k->fast) { block28_set_engine(k->fast, engine <= 1 ? -1 : engine - 2); k->engine_name = block28_name(k->fast); }
+    if (k->fast) { block28_set_engine(k->fast, eng); k->engine_name = block28_name(k->fast); }
     return PB200_OK;
 } PB200_CATCH
 void* pb200_key_stream(const pb200_key* k) { return k ? (void*)k->stream : nullptr; }
@@ -278,21 +282,19 @@ int pb200_key_take_flags(pb200_key* k, uint32_t* flags_out) try {
 int pb200_debug_mulmod(pb200_key* k, int engine, const int32_t* v_in, const int32_t* y_in, int reps, int32_t* v_out, int32_t* t_out,
                        uint32_t* qhat_rows) try {
     if (!k || !v_in || engine < 2 || engine > 5 || (!v_out && !t_out) || reps < 1) return PB200_ERR_INVALID_ARG;
-    if (!k->fast) return PB200_ERR_UNSUPPORTED;
-    if (engine == 4 && !block28_has_umma(k->fast)) return PB200_ERR_UNSUPPORTED;
-    if (engine == 5 && !block28_has_umma2(k->fast)) return PB200_ERR_UNSUPPORTED;
+    int eng;
+    if (!fast_engine(k, engine, &eng)) return PB200_ERR_UNSUPPORTED;
     USE_DEVICE(k);
-    CU(block28_debug_mulmod(k->fast, engine - 2, v_in, y_in, reps, v_out, t_out, qhat_rows, k->stream));
+    CU(block28_debug_mulmod(k->fast, eng, v_in, y_in, reps, v_out, t_out, qhat_rows, k->stream));
     return PB200_OK;
 } PB200_CATCH
 int pb200_debug_mulmod_cycles(pb200_key* k, int engine, const int32_t* v_in, int ctas, int reps, int stagger_cycles, int64_t* cycles_out) try {
     if (!k || !v_in || !cycles_out || engine < 3 || engine > 5 || ctas < 1 || reps < 1) return PB200_ERR_INVALID_ARG;
-    if (!k->fast) return PB200_ERR_UNSUPPORTED;
-    if (engine == 4 && !block28_has_umma(k->fast)) return PB200_ERR_UNSUPPORTED;
-    if (engine == 5 && !block28_has_umma2(k->fast)) return PB200_ERR_UNSUPPORTED;
+    int eng;
+    if (!fast_engine(k, engine, &eng)) return PB200_ERR_UNSUPPORTED;
     { int g = 0, bl = 0; block28_shape(k->fast, &g, &bl); if (g != 8) return PB200_ERR_UNSUPPORTED; }      // the |n| = 2048 configuration only
     USE_DEVICE(k);
-    CU(block28_debug_time(k->fast, engine - 2, v_in, ctas, reps, stagger_cycles, (long long*)cycles_out, k->stream));
+    CU(block28_debug_time(k->fast, eng, v_in, ctas, reps, stagger_cycles, (long long*)cycles_out, k->stream));
     return PB200_OK;
 } PB200_CATCH
 int pb200_umma_layout(int g, int bl, int lane_groups, int witness, int32_t* out20) try {

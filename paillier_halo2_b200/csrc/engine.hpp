@@ -46,8 +46,8 @@ const char* block28_name(const Block28Key*);
 // CTA (block28u), 3: with 64 per CTA (block28u2); each falls back to the next lower one the key size has; -1: fastest available.
 // Returns the engine in effect.
 int block28_set_engine(Block28Key*, int eng);
-bool block28_has_umma(const Block28Key*);
-bool block28_has_umma2(const Block28Key*);
+// whether the key's configuration compiles engine eng (0..3 as above; no fallback)
+bool block28_has_engine(const Block28Key*, int eng);
 void block28_chain_counts(const Block28Key*, uint64_t* n_sqr, uint64_t* n_mul);
 cudaError_t block28_encrypt(Block28Key*, const u64* d_m, const u64* d_r, size_t count, u64* d_c, cudaStream_t st);
 cudaError_t block28_tally(Block28Key*, const u64* d_c, size_t count, u64* d_out, cudaStream_t st);
