@@ -155,6 +155,35 @@ int pb200_tally_dev(pb200_key* key, const uint64_t* d_c_le, size_t count, uint64
  * key's device: the same fold on the key's own engine */
 int pb200_tally_combine(pb200_key* key, const uint64_t* partials_le, size_t n_partials, uint64_t* out_le);
 
+/* ---- running-tally trace ------------------------------------------------------------------------
+ * The witness of a circuit that proves a running tally: PaillierChip::add(acc, c_i) once per ballot, each step taking the previous
+ * step's rem.  For every chain j < chains and step i < count:
+ *   a = (i == 0 ? init_j : acc_(i-1, j)),  b = c_(i, j),  q_(i, j) = floor(a b / n^2),  acc_(i, j) = a b mod n^2
+ * exactly the values pb200_add_batch(a, b, c_words = words_out, .., q_out) returns for that pair.  A K-option ballot is K chains.
+ * Layout: step-major, one ballot per row: entry (i, j) of c, acc and q at (i * chains + j) * words_out words; init: chains *
+ * words_out words.  Inputs are any words_out-word values (reduced or not, as for pb200_add_batch): step 0 uses init exactly as given,
+ * every later a is canonical, so a q that does not fit words_out words (PB200_ERR_RANGE, host variant; PB200_FLAG_RANGE, _dev) can
+ * only come from step 0 with an unreduced init.  q_out == NULL skips the quotients (the prefix products alone).  count == 0 or
+ * chains == 0 does nothing; PB200_ERR_INVALID_ARG for null pointers where data is needed.
+ *
+ * Work: the chains are cut into chunks of about count * chains / lanes steps (lanes = 32 x resident CTAs per SM x SMs, one wave).
+ * Phase 1 multiplies each chunk into a total on the tally's engine, level after level over the totals; phase 2 turns them into every
+ * chunk's carry-in, init_j * the totals before it; phase 3 runs each chunk's exact chain on the witness engine.  About one fast and
+ * one exact multiplication per step; no host synchronise.  Temporary device memory does not depend on count: one buffer per level
+ * below the top, sum over l of ceil(n_l / s_l) * chains values, at most 3 * (lanes + chains) lazy values of the block28
+ * configuration (slightly more than words_out words each; canonical values on simple64), plus lanes + chains canonical carries
+ * (derivation in DESIGN.md §9c); the host variant's staged init, c, acc and q come on top.  PB200_TRACE_LANES=<n> replaces the
+ * wave size (a test and diagnostic switch: small waves reach every chunk and level boundary with few steps; output is the same).
+ *
+ * Contiguous operands for the advice cells: allocate (count + 1) * chains values, put init in row 0 and pass acc_out one row in
+ * (buf + chains * words_out).  Then (buf, c, q, buf + chains * words_out) are the (a, b, q, rem) arrays of pb200_mulmod_cells_batch
+ * for the count * chains steps, and the cells of the whole trace come from that one call.
+ * _dev: device pointers on the key's device, enqueued on the key's stream, no final synchronise. */
+int pb200_tally_trace(pb200_key* key, const uint64_t* init_le, const uint64_t* c_le, size_t count, size_t chains,
+                      uint64_t* acc_out_le, uint64_t* q_out_le /* nullable */);
+int pb200_tally_trace_dev(pb200_key* key, const uint64_t* d_init_le, const uint64_t* d_c_le, size_t count, size_t chains,
+                          uint64_t* d_acc_out_le, uint64_t* d_q_out_le /* nullable */);
+
 /* ---- multi-GPU tally (BASELINE.json configs[2]; SURVEY.md 8b pb200_tally(keys[], n_gpus, ..)) --------------------------------
  * Replaces: the fold of paillier_add_native (src/paillier.rs:94-97) over ciphertexts that are sharded across the GPUs of one
  * NVLink/NVSwitch domain.  ONE kernel launch per GPU: every GPU folds its shard, stores its 2|n|/8-byte partial into every

@@ -73,6 +73,8 @@ SYMBOLS = {
     "pb200_tally": (C.c_int, [C.c_void_p, u64p, C.c_size_t, u64p]),
     "pb200_tally_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "pb200_tally_combine": (C.c_int, [C.c_void_p, u64p, C.c_size_t, u64p]),
+    "pb200_tally_trace": (C.c_int, [C.c_void_p, u64p, u64p, C.c_size_t, C.c_size_t, u64p, u64p]),
+    "pb200_tally_trace_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p]),
     "pb200_tally_multi": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), u64p]),
     "pb200_tally_peer_export": (C.c_int, [C.c_void_p, C.c_void_p]),
     "pb200_tally_peer_connect": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),

@@ -14,6 +14,7 @@ Every call goes to CUDA through libpaillier_b200.so; nothing here computes a cip
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 from typing import Callable, Iterable, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -325,6 +326,44 @@ class PaillierKey(CellMixin):
     def tally(self, cs: Sequence[int]) -> int:
         c_w = ints_to_words(cs, self.words_out) if len(cs) else np.empty((0, self.words_out), dtype="<u8")
         return words_to_ints(self.tally_words(c_w))[0]
+
+    # -- running-tally trace: (q_i, acc_i) = divmod(acc_(i-1) * c_i, n^2) for every step of every chain --------------------------
+    def tally_trace_words(self, init_w: np.ndarray, c_w: np.ndarray, want_q: bool = True):
+        """init_w: (chains, words_out); c_w: (count, chains, words_out), any values -> acc (and q when want_q), each of shape
+        (count, chains, words_out): step i of chain j multiplies acc_(i-1, j) (init_j for i = 0) by c_(i, j) (pb200_tally_trace)."""
+        init_w = np.ascontiguousarray(init_w, dtype="<u8").reshape(-1, self.words_out)
+        chains = init_w.shape[0]
+        c_w = np.ascontiguousarray(c_w, dtype="<u8").reshape(-1, chains, self.words_out)
+        count = c_w.shape[0]
+        acc = np.empty((count, chains, self.words_out), dtype="<u8")
+        q = np.empty((count, chains, self.words_out), dtype="<u8") if want_q else None
+        if count and chains:
+            check(self._lib.pb200_tally_trace(self._h, _p(init_w), _p(c_w), count, chains, _p(acc), _p(q) if want_q else None),
+                  "pb200_tally_trace")
+        return (acc, q) if want_q else acc
+
+    def tally_trace_dev(self, d_init: int, d_c: int, count: int, chains: int, d_acc: int, d_q: Optional[int] = None) -> None:
+        """Device-pointer variant (pb200_tally_trace_dev): enqueues on the key's stream, no synchronise; a quotient that does not fit
+        raises PB200_FLAG_RANGE in the flag word (take_flags)."""
+        check(self._lib.pb200_tally_trace_dev(self._h, d_init, d_c, count, chains, d_acc, d_q or None), "pb200_tally_trace_dev")
+
+    def tally_trace(self, init, cs: Sequence, want_q: bool = True):
+        """Running tally on Python ints.  init: an int (one chain) or a sequence of one int per chain; cs: one element per step,
+        an int (one chain) or a sequence of one int per chain.  Returns acc (and q when want_q) as lists shaped like cs."""
+        single = isinstance(init, numbers.Integral)
+        inits = [int(init)] if single else [int(x) for x in init]
+        rows = [[int(c)] if single else [int(x) for x in c] for c in cs]
+        assert all(len(r) == len(inits) for r in rows), "every step needs one ciphertext per chain"
+        init_w = self._ciphertexts(inits, "tally_trace")
+        c_w = self._ciphertexts([c for r in rows for c in r], "tally_trace") if rows else np.empty((0, self.words_out), dtype="<u8")
+        res = self.tally_trace_words(init_w, c_w.reshape(len(rows), len(inits), self.words_out), want_q)
+        arrs = res if want_q else (res,)
+        outs = []
+        for a in arrs:
+            flat = words_to_ints(a.reshape(-1, self.words_out)) if rows else []
+            outs.append([flat[i] for i in range(len(rows))] if single else
+                        [flat[i * len(inits):(i + 1) * len(inits)] for i in range(len(rows))])
+        return (outs[0], outs[1]) if want_q else outs[0]
 
     # -- decryption (SURVEY.md 8f-4) -----------------------------------------------------------------------------------
     def set_private(self, lam: int, mu: int) -> None:

@@ -1214,6 +1214,131 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_add_w(B2
     w_end<C, WENG>(S);
 }
 
+// ---- running-tally trace (pb200_tally_trace, DESIGN.md §9c) --------------------------------------------------------------------
+// `chains` chains of n entries each, entry (i, j) of chain j at i * chains + j.  A level cuts every chain into chunks of s
+// consecutive entries; lane u = b * chains + j owns chunk b of chain j.  Phase 1 (k_trace_reduce, fast engine) multiplies each chunk
+// into a lazy total, level after level; phase 2 (k_trace_apply) turns the totals into exclusive prefixes from the top level down;
+// phase 3 (k_trace_w, witness engine) runs the exact chain of every leaf chunk from its carry-in.
+
+// smem per-lane value <- one lazy entry, or 1 where !real (the entry is then not read)
+template <class C>
+__device__ __forceinline__ void gather_or_one(int4* buf, const int4* entry, bool real, int role, int lane) {
+#pragma unroll
+    for (int c = 0; c < C::CH; c++)
+        buf[(role * C::CH + c) * 32 + lane] = real ? entry[role * C::CH + c] : make_int4(role == 0 && c == 0 ? 1 : 0, 0, 0, 0);
+    __syncthreads();
+}
+
+// totals[u] = product of chunk b of chain j (lazy).  Level 0 reads words (in_words, words_out each, any value), later levels the lazy
+// totals of the level below.  The first entry is loaded, the others multiplied in; entries past the end of the chain multiply by 1.
+template <class C, int ENG>
+__global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_trace_reduce(B28Dev K, const u64* __restrict__ in_words,
+                                                                             const int4* __restrict__ in_lazy, size_t n, size_t chains,
+                                                                             size_t s, int4* __restrict__ totals) {
+    extern __shared__ int4 smem[];
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
+    cta_begin<C, ENG>(S, smem, K);
+    const size_t units = (n + s - 1) / s * chains;
+    size_t u = (size_t)blockIdx.x * 32 + lane;
+    const bool active = u < units;
+    if (!active) u = units - 1;
+    const size_t b = u / chains, j = u - b * chains;
+    for (size_t t = 0; t < s; t++) {
+        const size_t i = b * s + t;
+        const bool real = i < n;                                                         // always true for t = 0
+        const size_t e = (real ? i : n - 1) * chains + j;
+        int4* dst = t ? S.B : S.V;
+        if (in_words) load_value<C>(dst, in_words + e * K.words_out, K.words_out, role, lane);
+        else gather_entry<C>(dst, in_lazy + e * C::ENTRY4, role, lane);
+        if (t) {
+            set_one_where<C>(S.B, !real, role, lane);
+            mm<C, false, ENG>(S, S.B, role, lane);
+        }
+    }
+    if (active) scatter_entry<C>(totals + u * C::ENTRY4, S.V, role, lane);
+    cta_end<C, ENG>(S);
+}
+
+// Exclusive prefix products of one level, in place: entry (b s + t, j) <- carry(b, j) * the entries before it in its chunk.  The carry
+// of chunk b is the lazy prefix the level above wrote for it, or init_j at the top level (carry == null: one chunk per chain).
+template <class C, int ENG>
+__global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_trace_apply(B28Dev K, const u64* __restrict__ init,
+                                                                            const int4* __restrict__ carry, int4* items, size_t n,
+                                                                            size_t chains, size_t s) {
+    extern __shared__ int4 smem[];
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
+    cta_begin<C, ENG>(S, smem, K);
+    const size_t units = (n + s - 1) / s * chains;
+    size_t u = (size_t)blockIdx.x * 32 + lane;
+    const bool active = u < units;
+    if (!active) u = units - 1;
+    const size_t b = u / chains, j = u - b * chains;
+    if (carry) gather_entry<C>(S.V, carry + u * C::ENTRY4, role, lane);
+    else load_value<C>(S.V, init + j * K.words_out, K.words_out, role, lane);
+    for (size_t t = 0; t < s; t++) {
+        const size_t i = b * s + t;
+        const bool real = active && i < n;
+        int4* e = items + (real ? i * chains + j : 0) * C::ENTRY4;
+        gather_or_one<C>(S.B, e, real, role, lane);                                      // the total, read before its slot is overwritten
+        if (real) scatter_entry<C>(e, S.V, role, lane);
+        if (t + 1 < s) mm<C, false, ENG>(S, S.B, role, lane);                            // the chunk's own product is not needed
+    }
+    cta_end<C, ENG>(S);
+}
+
+// The exact chain of every leaf chunk on the witness engine: a <- carry-in (init_j for chunk 0, as given; else carry[u], canonical),
+// then per step (q, rem) = divmod(a c_(i, j), n^2), rem to acc (and q to q_out), a <- rem.  Steps past the end multiply by 1 and store
+// nothing.  A quotient that does not fit words_out words raises the range flag, as in k_add_w.
+template <class C, int WENG>
+__global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_trace_w(B28Dev K, WitDev Wd, const u64* __restrict__ init,
+                                                                        const u64* __restrict__ c, const u64* __restrict__ carry,
+                                                                        size_t count, size_t chains, size_t s, u64* __restrict__ acc,
+                                                                        u64* __restrict__ q_out, int* flags) {
+    extern __shared__ int4 smem[];
+    typename WView<C, WENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
+    w_begin<C, WENG>(S, smem, K);
+    const int wo = K.words_out;
+    const size_t units = (count + s - 1) / s * chains;
+    size_t u = (size_t)blockIdx.x * 32 + lane;
+    const bool active = u < units;
+    if (!active) u = units - 1;
+    const size_t b = u / chains, j = u - b * chains;
+    load_value_shl<C>(S.V, b ? carry + u * wo : init + j * wo, wo, Wd.sh >> 1, role, lane);
+    for (size_t t = 0; t < s; t++) {
+        const size_t i = b * s + t;
+        const bool real = active && i < count;
+        const size_t e = (i < count ? i : count - 1) * chains + j;
+        load_value_shl<C>(S.B, c + e * wo, wo, Wd.sh >> 1, role, lane);
+        if (!real) {
+#pragma unroll
+            for (int ch = 0; ch < C::CH; ch++) S.B[(role * C::CH + ch) * 32 + lane] = __ldg(Wd.one_s + role * C::CH + ch);
+        }
+        __syncthreads();
+        WStep o; o.rec = nullptr; o.rem_out = real ? acc + e * wo : nullptr;
+        o.q_out = (real && q_out) ? q_out + e * wo : nullptr;
+        wmm<C, WENG>(smem, S, S.B, 0, S.V, o, Wd.sh, wo, Wd.inv, Wd.cpow);
+        {   // q must fit words_out words (the check of k_add_w)
+            const int* Qf = (const int*)S.T + C::L * 32;
+            const int qbits = 64 * wo;
+            int bad = 0;
+#pragma unroll
+            for (int k = 0; k < C::BL; k++) {
+                const int p = role * C::BL + k;
+                const unsigned d = (unsigned)Qf[p * 32 + lane];
+                const int lo = W * p;
+                if (lo >= qbits) bad |= d != 0;
+                else if (lo + W > qbits) bad |= (d >> (qbits - lo)) != 0;
+            }
+            if (bad && real) atomicOr(flags, 1);
+        }
+        __syncthreads();
+    }
+    w_end<C, WENG>(S);
+}
+
 // ---- host side ---------------------------------------------------------------------------------
 struct Block28Key {
     int G = 0, BL = 0;
@@ -1856,6 +1981,60 @@ cudaError_t block28_add(Block28Key* key, const u64* d_c1, const u64* d_c2, int c
                         int* d_flags, cudaStream_t st) {
     if (!count) return cudaSuccess;
     return with_cfg(key, [&](auto c) { return add_cfg<decltype(c)>(key, d_c1, d_c2, c_words, count, d_out, d_q, d_flags, st); });
+}
+
+// ---- running-tally trace: driver (DESIGN.md §9c) ----------------------------------------------------------------------------------
+// one wave of the trace's scan kernels: 32 lanes x the CTAs per SM of the key's tally engine (View<C, 4> on tcgen05) x SMs
+size_t block28_lanes(const Block28Key* key) {
+    return Configs::with(key->G, key->BL, (size_t)0, [&](auto c) {
+        typedef decltype(c) C;
+        return (size_t)(tally_eng(key) == 4 ? View<C, 4>::PER_SM : View<C, 0>::PER_SM) * key->sms * 32;
+    });
+}
+// one buffer of lazy values per level below the top (the totals of its chunks, then in place their carries)
+template <class C>
+static size_t trace_scan_bytes_cfg(const TracePlan& P, size_t chains) {
+    size_t b = 0;
+    for (size_t l = 0; l + 1 < P.n.size(); l++) b += P.n[l + 1] * chains * C::ENTRY4 * sizeof(int4);
+    return b;
+}
+size_t block28_trace_scan_bytes(const Block28Key* key, const TracePlan& P, size_t chains) {
+    return Configs::with(key->G, key->BL, (size_t)0, [&](auto c) { return trace_scan_bytes_cfg<decltype(c)>(P, chains); });
+}
+template <class C, int ENG>
+static cudaError_t trace_scan_cfg(Block28Key* key, const TracePlan& P, const u64* d_init, const u64* d_c, size_t chains,
+                                  unsigned char* tmp, u64* d_carry, cudaStream_t st) {
+    typedef View<C, ENG> V;
+    const size_t L = P.n.size() - 1;                                 // levels below the top
+    std::vector<int4*> buf(L);
+    for (size_t l = 0, o = 0; l < L; l++) { buf[l] = (int4*)(tmp + o); o += P.n[l + 1] * chains * C::ENTRY4 * sizeof(int4); }
+    for (size_t l = 0; l < L; l++)                                   // phase 1: the totals of every chunk, level after level
+        CUW(launch<V>(k_trace_reduce<C, ENG>, cdiv(P.n[l + 1] * chains, 32), st, key->dev, l ? (const u64*)nullptr : d_c,
+                      l ? (const int4*)buf[l - 1] : (const int4*)nullptr, P.n[l], chains, P.s[l], buf[l]));
+    for (size_t l = L; l >= 1; l--)                                  // phase 2: the carries of level l - 1 from the top down
+        CUW(launch<V>(k_trace_apply<C, ENG>, cdiv(cdiv(P.n[l], P.s[l]) * chains, 32), st, key->dev, d_init,
+                      l == L ? (const int4*)nullptr : (const int4*)buf[l], buf[l - 1], P.n[l], chains, P.s[l]));
+    return launch<V>(k_lazy_canon<C, ENG>, cdiv(P.n[1] * chains, 32), st, key->dev, (const int4*)buf[0], P.n[1] * chains, d_carry);
+}
+cudaError_t block28_trace_scan(Block28Key* key, const TracePlan& P, const u64* d_init, const u64* d_c, size_t chains, void* tmp, u64* d_carry,
+                               cudaStream_t st) {
+    if (P.n.size() < 2) return cudaSuccess;
+    return with_cfg(key, [&](auto c) {
+        typedef decltype(c) C;
+        return with_eng<View, C, 0, 1, 4>(tally_eng(key), [&](auto e) {
+            return trace_scan_cfg<C, e>(key, P, d_init, d_c, chains, (unsigned char*)tmp, d_carry, st);
+        });
+    });
+}
+cudaError_t block28_trace_chain(Block28Key* key, const u64* d_init, const u64* d_c, const u64* d_carry, size_t count, size_t chains, size_t s,
+                                u64* d_acc, u64* d_q, int* d_flags, cudaStream_t st) {
+    return with_cfg(key, [&](auto c) {
+        typedef decltype(c) C;
+        return with_eng<WView, C, 0, 1>(wit_eng(key), [&](auto e) {
+            return launch<WView<C, e>>(k_trace_w<C, e>, cdiv(cdiv(count, s) * chains, 32), st, key->wdev, key->wit, d_init, d_c, d_carry,
+                                       count, chains, s, d_acc, d_q, d_flags);
+        });
+    });
 }
 
 // ---- matvec: planner and driver (DESIGN.md §9b) ---------------------------------------------------------------------------------

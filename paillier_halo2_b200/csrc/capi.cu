@@ -72,6 +72,7 @@ struct pb200_key {
     DevBuf wt_chunk, wt_part;               // weighted tally: one chunk's scalar products, the per-chunk partial products
     DevBuf mv_arena, mv_neg, mv_nm1;        // matvec: temporary memory of the plan, staged signs, copies of n - 1 for the sign step
     size_t mv_nm1_units = 0;
+    DevBuf tr_tmp;                          // running-tally trace: per-level chunk totals and the leaf chunks' carries
     std::string engine_name;
     // K4 cell expansion: per lookup_bits layout + device constants (n^2 limbs, word_max, q_acc, mod_acc), refresh spill vector
     struct CellCtx { CellLayout Y; u64* d_consts = nullptr; int* d_inc = nullptr; u64* d_mtab = nullptr; int n_out = 0; int n2_cells = 0; };
@@ -187,6 +188,7 @@ void pb200_key_destroy(pb200_key* k) {
     k->in_a.release(); k->in_b.release(); k->out_a.release(); k->out_b.release(); k->scratch.release(); k->offs.release();
     k->wt_chunk.release(); k->wt_part.release();
     k->mv_arena.release(); k->mv_neg.release(); k->mv_nm1.release();
+    k->tr_tmp.release();
     k->cin_a.release(); k->cin_b.release(); k->cin_q.release(); k->cin_r.release();
     if (k->pipe.ready) {
         if (k->pipe.copy) { cudaStreamSynchronize(k->pipe.copy); cudaStreamDestroy(k->pipe.copy); }
@@ -435,6 +437,81 @@ int pb200_tally(pb200_key* k, const uint64_t* c, size_t count, uint64_t* out) tr
 int pb200_tally_combine(pb200_key* k, const uint64_t* partials, size_t n_partials, uint64_t* out) try {
     // the combine of per-shard partials is the same fold, on the key's own engine
     return pb200_tally(k, partials, n_partials, out);
+} PB200_CATCH
+
+// ---- running-tally trace: every step (q_i, acc_i) = divmod(acc_(i-1) * c_i, n^2) of `chains` chains ---------------------------------
+// Level 0 cuts every chain into chunks of s_0 steps, about one wave of lanes over all the chains; every level above cuts the chunk
+// totals of the one below the same way, with at least TRACE_MIN_S per chunk, until one chunk covers a chain.  Every level's size
+// follows from (count, chains, lanes), so the whole trace is enqueued without a host synchronise.  PB200_TRACE_LANES replaces the
+// wave (a development switch: a small wave gives many levels on few steps).
+static const size_t TRACE_MIN_S = 4;
+static TracePlan trace_plan(size_t count, size_t chains, size_t lanes) {
+    TracePlan P;
+    size_t n = count, s = (count * chains + lanes - 1) / lanes;
+    if (s < 1) s = 1;
+    for (;;) {
+        P.n.push_back(n); P.s.push_back(s);
+        n = (n + s - 1) / s;
+        if (n <= 1) return P;
+        s = (n * chains + lanes - 1) / lanes;
+        if (s < TRACE_MIN_S) s = TRACE_MIN_S;
+    }
+}
+static int trace_dev_impl(pb200_key* k, const u64* d_init, const u64* d_c, size_t count, size_t chains, u64* d_acc, u64* d_q) {
+    const size_t wo = k->words_out;
+    // phases 1 and 2 on the tally's engine, phase 3 on the witness engine (both simple64 when the key runs no block28 engine)
+    const bool fast_scan = use_fast(k), fast_chain = fast_scan && block28_witness_supported(k->fast);
+    if (fast_chain) { bool f = false; int rc = witness_engine(k, &f); if (rc) return rc; }
+    size_t lanes = fast_scan ? block28_lanes(k->fast) : (size_t)k->sms * 64;
+    if (const char* e = getenv("PB200_TRACE_LANES")) { const long long v = atoll(e); if (v >= 1) lanes = (size_t)v; }
+    const TracePlan P = trace_plan(count, chains, lanes);
+    u64* d_carry = nullptr;                                           // carry-in of level-0 chunk b >= 1; none with one chunk per chain
+    if (P.n.size() > 1) {
+        if (fast_scan) {
+            const size_t scan = block28_trace_scan_bytes(k->fast, P, chains);
+            CU(k->tr_tmp.reserve(scan + P.n[1] * chains * wo * sizeof(u64)));
+            d_carry = (u64*)((unsigned char*)k->tr_tmp.p + scan);
+            CU(block28_trace_scan(k->fast, P, d_init, d_c, chains, k->tr_tmp.p, d_carry, k->stream));
+        } else {
+            CU(k->tr_tmp.reserve(simple_trace_scan_words(P, chains, (int)wo) * sizeof(u64)));
+            d_carry = (u64*)k->tr_tmp.p;
+            CU(simple_trace_scan(k->d_simple, (int)wo, P, d_init, d_c, chains, d_carry, k->stream));
+        }
+    }
+    if (fast_chain) CU(block28_trace_chain(k->fast, d_init, d_c, d_carry, count, chains, P.s[0], d_acc, d_q, k->d_flags, k->stream));
+    else CU(simple_trace_chain(k->d_simple, d_init, d_c, d_carry, count, chains, P.s[0], d_acc, d_q, k->d_flags, k->stream));
+    return PB200_OK;
+}
+// count * chains * words_out words must be addressable
+static bool trace_size_ok(const pb200_key* k, size_t count, size_t chains) {
+    return chains <= SIZE_MAX / count / (k->words_out * sizeof(u64)) / 2;
+}
+int pb200_tally_trace_dev(pb200_key* k, const uint64_t* d_init, const uint64_t* d_c, size_t count, size_t chains, uint64_t* d_acc,
+                          uint64_t* d_q) try {
+    if (!k || (count && chains && (!d_init || !d_c || !d_acc))) return PB200_ERR_INVALID_ARG;
+    if (!count || !chains) return PB200_OK;
+    if (!trace_size_ok(k, count, chains)) return PB200_ERR_INVALID_ARG;
+    USE_DEVICE(k);
+    return trace_dev_impl(k, (const u64*)d_init, (const u64*)d_c, count, chains, (u64*)d_acc, (u64*)d_q);
+} PB200_CATCH
+int pb200_tally_trace(pb200_key* k, const uint64_t* init, const uint64_t* c, size_t count, size_t chains, uint64_t* acc_out,
+                      uint64_t* q_out) try {
+    if (!k || (count && chains && (!init || !c || !acc_out))) return PB200_ERR_INVALID_ARG;
+    if (!count || !chains) return PB200_OK;
+    if (!trace_size_ok(k, count, chains)) return PB200_ERR_INVALID_ARG;
+    USE_DEVICE(k);
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bi = chains * k->words_out * sizeof(u64), bc = count * bi;
+    CU(k->in_a.reserve(bi)); CU(k->in_b.reserve(bc)); CU(k->out_a.reserve(bc));
+    if (q_out) CU(k->out_b.reserve(bc));
+    CU(cudaMemcpyAsync(k->in_a.p, init, bi, cudaMemcpyHostToDevice, k->stream));
+    CU(cudaMemcpyAsync(k->in_b.p, c, bc, cudaMemcpyHostToDevice, k->stream));
+    int rc = trace_dev_impl(k, (const u64*)k->in_a.p, (const u64*)k->in_b.p, count, chains, (u64*)k->out_a.p, q_out ? (u64*)k->out_b.p : nullptr);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(acc_out, k->out_a.p, bc, cudaMemcpyDeviceToHost, k->stream));
+    if (q_out) CU(cudaMemcpyAsync(q_out, k->out_b.p, bc, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
 } PB200_CATCH
 
 // ---- multi-GPU tally ------------------------------------------------------------------------------------

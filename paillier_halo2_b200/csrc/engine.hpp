@@ -35,6 +35,17 @@ cudaError_t simple_pow(const SimpleConsts* dK, const u64* d_base, int base_words
                        u64* d_out, int* d_flags, cudaStream_t st);
 cudaError_t simple_lfunc(const SimpleConsts* dKn, const u64* d_x, size_t count, u64* d_m, int* d_flags, cudaStream_t st);
 
+// running-tally trace (pb200_tally_trace): level l holds n[l] entries per chain in chunks of s[l]; n[l + 1] = ceil(n[l] / s[l]) and the
+// last level has one chunk per chain.  Level 0 is the steps themselves.
+struct TracePlan { std::vector<size_t> n, s; };
+// phases 1 and 2 on simple64: d_tmp (simple_trace_scan_words) ends with the canonical carry-in of every level-0 chunk at its start
+size_t simple_trace_scan_words(const TracePlan& P, size_t chains, int k);
+cudaError_t simple_trace_scan(const SimpleConsts* dK, int k, const TracePlan& P, const u64* d_init, const u64* d_c, size_t chains,
+                              u64* d_tmp, cudaStream_t st);
+// phase 3 on simple64: one thread per level-0 chunk (d_carry: carry-in of chunk b >= 1 at (b * chains + j) * k; null with one chunk)
+cudaError_t simple_trace_chain(const SimpleConsts* dK, const u64* d_init, const u64* d_c, const u64* d_carry, size_t count, size_t chains,
+                               size_t s, u64* d_acc, u64* d_q /*nullable*/, int* d_flags, cudaStream_t st);
+
 // ---- block28 engine (block28_kernels.cu) ----------------------------------------------------
 struct Block28Key;  // opaque per-key state of the fast engine
 // returns nullptr (and leaves *why) when no compiled configuration covers the key size
@@ -94,6 +105,17 @@ cudaError_t block28_witness(Block28Key*, const u64* d_m, const u64* d_r, size_t 
 // one exact mul_mod per pair on the witness engine (requires block28_witness_prepare); range flag bit 0 when q does not fit
 cudaError_t block28_add(Block28Key*, const u64* d_c1, const u64* d_c2, int c_words, size_t count, u64* d_out, u64* d_q /*nullable*/,
                         int* d_flags, cudaStream_t st);
+
+// running-tally trace.  Lanes of one wave of the tally's CTA shape (32 x resident CTAs per SM x SMs).
+size_t block28_lanes(const Block28Key*);
+// phases 1 and 2 on the key's tally engine: d_carry (P.n[1] * chains * words_out words) <- the canonical carry-in of every level-0
+// chunk; tmp: block28_trace_scan_bytes of device memory.  Nothing to do when P has a single level.
+size_t block28_trace_scan_bytes(const Block28Key*, const TracePlan& P, size_t chains);
+cudaError_t block28_trace_scan(Block28Key*, const TracePlan& P, const u64* d_init, const u64* d_c, size_t chains, void* tmp, u64* d_carry,
+                               cudaStream_t st);
+// phase 3 on the witness engine (requires block28_witness_prepare); d_carry as simple_trace_chain
+cudaError_t block28_trace_chain(Block28Key*, const u64* d_init, const u64* d_c, const u64* d_carry, size_t count, size_t chains, size_t s,
+                                u64* d_acc, u64* d_q /*nullable*/, int* d_flags, cudaStream_t st);
 
 // diagnostic: one CTA's modular multiplication on raw lazy digits (shared-memory image layout), see k_mulmod_dbg
 cudaError_t block28_debug_mulmod(Block28Key*, int eng, const int* h_v, const int* h_y, int reps, int* h_vout, int* h_t, unsigned* h_rows,

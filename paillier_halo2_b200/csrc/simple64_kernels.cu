@@ -174,6 +174,61 @@ __global__ void __launch_bounds__(32) k_simple_lfunc(const SimpleConsts* __restr
     if (bad) atomicOr(flags, 8);
 }
 
+// ---- running-tally trace (pb200_tally_trace): the three phases of block28_kernels.cu, one thread per chunk, canonical values -------
+// totals[u] = product of chunk b of chain j, u = b * chains + j (entries (i, j) at (i * chains + j) * k, any k-word value)
+__global__ void __launch_bounds__(32) k_simple_trace_reduce(const SimpleConsts* __restrict__ K, const u64* __restrict__ in, size_t n,
+                                                            size_t chains, size_t s, u64* __restrict__ totals) {
+    const size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= (n + s - 1) / s * chains) return;
+    const size_t b = u / chains, j = u - b * chains;
+    const int k = K->k;
+    u64 acc[PB200_SIMPLE_MAXK], x[PB200_SIMPLE_MAXK], q[PB200_SIMPLE_MAXK];
+    set_one(acc, k);
+    for (size_t i = b * s; i < n && i < (b + 1) * s; i++) {
+        for (int w = 0; w < k; w++) x[w] = in[(i * chains + j) * k + w];
+        mulmod_simple(K, q, acc, acc, x);                  // acc is canonical: q always fits
+    }
+    for (int w = 0; w < k; w++) totals[u * k + w] = acc[w];
+}
+// exclusive prefix products of one level, in place; the carry of chunk b is carry[u], or init_j reduced mod n^2 (carry == null)
+__global__ void __launch_bounds__(32) k_simple_trace_apply(const SimpleConsts* __restrict__ K, const u64* __restrict__ init,
+                                                           const u64* __restrict__ carry, u64* items, size_t n, size_t chains, size_t s) {
+    const size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= (n + s - 1) / s * chains) return;
+    const size_t b = u / chains, j = u - b * chains;
+    const int k = K->k;
+    u64 acc[PB200_SIMPLE_MAXK], x[PB200_SIMPLE_MAXK], q[PB200_SIMPLE_MAXK];
+    if (carry) for (int w = 0; w < k; w++) acc[w] = carry[u * k + w];
+    else { set_one(x, k); mulmod_simple(K, q, acc, init + j * k, x); }
+    for (size_t i = b * s; i < n && i < (b + 1) * s; i++) {
+        u64* e = items + (i * chains + j) * k;
+        for (int w = 0; w < k; w++) { x[w] = e[w]; e[w] = acc[w]; }
+        mulmod_simple(K, q, acc, acc, x);
+    }
+}
+// the exact chain of every level-0 chunk: a <- init_j (chunk 0, as given) or carry[u]; (q, rem) = divmod(a c_(i, j), n^2), a <- rem
+__global__ void __launch_bounds__(32) k_simple_trace_chain(const SimpleConsts* __restrict__ K, const u64* __restrict__ init,
+                                                           const u64* __restrict__ c, const u64* __restrict__ carry, size_t count,
+                                                           size_t chains, size_t s, u64* __restrict__ acc_out, u64* __restrict__ q_out,
+                                                           int* flags) {
+    const size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= (count + s - 1) / s * chains) return;
+    const size_t b = u / chains, j = u - b * chains;
+    const int k = K->k;
+    u64 a[PB200_SIMPLE_MAXK], x[PB200_SIMPLE_MAXK], q[PB200_SIMPLE_MAXK];
+    const u64* a0 = b ? carry + u * k : init + j * k;
+    for (int w = 0; w < k; w++) a[w] = a0[w];
+    int bad = 0;
+    for (size_t i = b * s; i < count && i < (b + 1) * s; i++) {
+        const size_t e = (i * chains + j) * k;
+        for (int w = 0; w < k; w++) x[w] = c[e + w];
+        bad |= mulmod_simple(K, q, a, a, x);
+        for (int w = 0; w < k; w++) acc_out[e + w] = a[w];
+        if (q_out) for (int w = 0; w < k; w++) q_out[e + w] = q[w];
+    }
+    if (bad) atomicOr(flags, 1);
+}
+
 // K5: value (words_per_value u64 words) -> value_bits/limb_bits limbs, 2 words per limb (lo, hi)
 __global__ void k_repack(const u64* __restrict__ vals, size_t count, int wpv, int nl, int limb_bits, u64* __restrict__ out) {
     size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -237,6 +292,34 @@ cudaError_t simple_pow(const SimpleConsts* dK, const u64* d_base, int base_words
 cudaError_t simple_lfunc(const SimpleConsts* dKn, const u64* d_x, size_t count, u64* d_m, int* d_flags, cudaStream_t st) {
     if (!count) return cudaSuccess;
     k_simple_lfunc<<<(unsigned)((count + 31) / 32), 32, 0, st>>>(dKn, d_x, count, d_m, d_flags); count_launch();
+    return cudaGetLastError();
+}
+size_t simple_trace_scan_words(const TracePlan& P, size_t chains, int k) {
+    size_t w = 0;
+    for (size_t l = 0; l + 1 < P.n.size(); l++) w += P.n[l + 1] * chains * k;
+    return w;
+}
+cudaError_t simple_trace_scan(const SimpleConsts* dK, int k, const TracePlan& P, const u64* d_init, const u64* d_c, size_t chains, u64* d_tmp,
+                              cudaStream_t st) {
+    const size_t L = P.n.size() - 1;
+    std::vector<u64*> buf(L);
+    for (size_t l = 0, o = 0; l < L; l++) { buf[l] = d_tmp + o; o += P.n[l + 1] * chains * k; }
+    for (size_t l = 0; l < L; l++) {
+        k_simple_trace_reduce<<<(unsigned)((P.n[l + 1] * chains + 31) / 32), 32, 0, st>>>(dK, l ? buf[l - 1] : d_c, P.n[l], chains, P.s[l], buf[l]);
+        count_launch();
+    }
+    for (size_t l = L; l >= 1; l--) {
+        const size_t units = (P.n[l] + P.s[l] - 1) / P.s[l] * chains;
+        k_simple_trace_apply<<<(unsigned)((units + 31) / 32), 32, 0, st>>>(dK, d_init, l == L ? nullptr : buf[l], buf[l - 1], P.n[l], chains, P.s[l]);
+        count_launch();
+    }
+    return cudaGetLastError();
+}
+cudaError_t simple_trace_chain(const SimpleConsts* dK, const u64* d_init, const u64* d_c, const u64* d_carry, size_t count, size_t chains,
+                               size_t s, u64* d_acc, u64* d_q, int* d_flags, cudaStream_t st) {
+    const size_t units = (count + s - 1) / s * chains;
+    k_simple_trace_chain<<<(unsigned)((units + 31) / 32), 32, 0, st>>>(dK, d_init, d_c, d_carry, count, chains, s, d_acc, d_q, d_flags);
+    count_launch();
     return cudaGetLastError();
 }
 cudaError_t repack_limbs(const u64* d_vals, size_t count, int wpv, int value_bits, int limb_bits, u64* d_out, cudaStream_t st) {

@@ -98,6 +98,10 @@ extern "C" {
     pub fn pb200_tally(key: *mut pb200_key, c_le: *const u64, count: usize, out_le: *mut u64) -> c_int;
     pub fn pb200_tally_dev(key: *mut pb200_key, d_c_le: *const u64, count: usize, d_partial_out_le: *mut u64) -> c_int;
     pub fn pb200_tally_combine(key: *mut pb200_key, partials_le: *const u64, n_partials: usize, out_le: *mut u64) -> c_int;
+    pub fn pb200_tally_trace(key: *mut pb200_key, init_le: *const u64, c_le: *const u64, count: usize, chains: usize, acc_out_le: *mut u64,
+                             q_out_le: *mut u64) -> c_int;
+    pub fn pb200_tally_trace_dev(key: *mut pb200_key, d_init_le: *const u64, d_c_le: *const u64, count: usize, chains: usize,
+                                 d_acc_out_le: *mut u64, d_q_out_le: *mut u64) -> c_int;
     pub fn pb200_tally_multi(keys: *const *mut pb200_key, n_gpus: c_int, d_c: *const *const u64, counts: *const usize, out_le: *mut u64) -> c_int;
     pub fn pb200_tally_peer_export(key: *mut pb200_key, out: *mut pb200_ipc_handle) -> c_int;
     pub fn pb200_tally_peer_connect(key: *mut pb200_key, rank: c_int, world: c_int, handles: *const pb200_ipc_handle) -> c_int;
@@ -244,6 +248,20 @@ impl Key {
         let neg = if w_neg.is_empty() { std::ptr::null() } else { w_neg.as_ptr() };
         let rc = unsafe { pb200_matvec(self.raw, c.as_ptr(), count, w_mag.as_ptr(), neg, k_bits, rows, out.as_mut_ptr()) };
         if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// running-tally trace: `init` holds `chains * words_out` words, `c` the steps row by row (`count * chains * words_out` words, entry
+    /// (i, j) at `(i * chains + j) * words_out`); returns (acc, q), each laid out like `c`, with
+    /// (q_ij, acc_ij) = divmod(acc_(i-1)j * c_ij, n^2) and acc_(-1)j = init_j: the (q, rem) of every `PaillierChip::add` of the chains
+    pub fn tally_trace(&mut self, init: &[u64], c: &[u64]) -> Result<(Vec<u64>, Vec<u64>), i32> {
+        let wo = self.words_out();
+        if wo == 0 || init.is_empty() || init.len() % wo != 0 || c.len() % init.len() != 0 {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let (chains, count) = (init.len() / wo, c.len() / init.len());
+        let (mut acc, mut q) = (vec![0u64; c.len()], vec![0u64; c.len()]);
+        let rc = unsafe { pb200_tally_trace(self.raw, init.as_ptr(), c.as_ptr(), count, chains, acc.as_mut_ptr(), q.as_mut_ptr()) };
+        if rc == PB200_OK { Ok((acc, q)) } else { Err(rc) }
     }
 }
 
