@@ -24,13 +24,15 @@ constexpr int WIN = 6;                 // sliding window of the r-chain (6: 293 
 constexpr int TABN = 1 << (WIN - 1);   // odd powers r^1, r^3, ..., r^(2*TABN-1)
 constexpr int SCRATCH_ENTRIES = TABN + 2;   // + r^2 (table build) + rn (kept while g^m is computed)
 
+// left-to-right sliding-window schedule of a fixed exponent (window_schedule): the chain starts from odd-power table entry first_idx
+// (-1: the exponent is 0), then runs n_ops steps (number of squarings, table index to multiply by or -1)
+struct PowSched { const int2* ops; int n_ops; int first_idx; };
+
 struct B28Dev {            // per-key device-side descriptor (same for every configuration)
     const int4* consts;    // mu, Nt, two_sh : 3 * ENTRY4 int4
     const int4* uconsts2;  // the same for the two-lane-group variant
     const int4* uconsts;   // block28u: constants + CM tables (UL<C>::KEY_BYTES), null when the configuration has no tcgen05 variant
-    const int2* ops;       // r-chain schedule: (number of squarings, table index or -1)
-    int n_ops;
-    int first_idx;         // table index the chain starts from
+    PowSched rn;           // r-chain schedule (the exponent n)
     const int4* tg;        // comb table: [window][2^comb_bits][ENTRY4]
     int n_windows;
     int comb_bits;         // window width of the fixed-base comb for g^m
@@ -49,28 +51,43 @@ __device__ __forceinline__ int& digit_ref(int4* buf, int p, int lane) {
     return ((int*)(buf + blk * C::BLK4 + (k >> 2) * 32 + lane))[k & 3];
 }
 
-// per-lane buffer <- strict digits of the unsigned integer in src[0..nwords) (u64 little-endian)
-template <class C>
-__device__ __forceinline__ void load_value(int4* buf, const u64* src, int nwords, int role, int lane) {
+// The digit loader: the strict digit of (value << shl) at bit position bit = 28 p - shl of the value, from the 28-bit field there
+// plus the carry out of the digit below (updated).  The value is the unsigned integer word(0 .. nwords), u64 little-endian, read
+// through the accessor `word`, so every caller keeps its own load flavour and layout.
+template <class F>
+__device__ __forceinline__ int strict_digit(const F& word, int nwords, int bit, int& carry) {
+    u64 v = 0;
+    if (bit >= 0) {
+        const int wi = bit >> 6, sh = bit & 63;
+        const u64 lo = wi < nwords ? word(wi) : 0, hi = wi + 1 < nwords ? word(wi + 1) : 0;
+        v = sh ? (lo >> sh) | (hi << (64 - sh)) : lo;
+    } else if (bit > -W) {
+        v = word(0) << (-bit);
+    }
+    const int t = (int)(v & ((1u << W) - 1)) + carry;
+    const int d = sgxt28(t);
+    carry = (t - d) >> W;
+    return d;
+}
+// per-lane buffer <- strict digits of (value << shl), value = word(0 .. nwords) (see strict_digit); the carry out of a block is added
+// to the first digit of the next one
+template <class C, class F>
+__device__ __forceinline__ void load_words(int4* buf, const F& word, int nwords, int shl, int role, int lane) {
     int a[C::CH * 4];
     int carry = 0;
 #pragma unroll
-    for (int k = 0; k < C::BL; k++) {
-        int bit = W * (role * C::BL + k);
-        int wi = bit >> 6, sh = bit & 63;
-        u64 lo = wi < nwords ? src[wi] : 0, hi = wi + 1 < nwords ? src[wi + 1] : 0;
-        u64 v = sh ? (lo >> sh) | (hi << (64 - sh)) : lo;
-        int t = (int)(v & ((1u << W) - 1)) + carry;
-        int d = sgxt28(t);
-        carry = (t - d) >> W;
-        a[k] = d;
-    }
+    for (int k = 0; k < C::BL; k++) a[k] = strict_digit(word, nwords, W * (role * C::BL + k) - shl, carry);
 #pragma unroll
     for (int k = C::BL; k < C::CH * 4; k++) a[k] = 0;
     store_block<C>(blk_ptr<C>(buf, role, lane), a);
     __syncthreads();
     if (role + 1 < C::G) *(int*)blk_ptr<C>(buf, role + 1, lane) += carry;
     __syncthreads();
+}
+// per-lane buffer <- strict digits of (src[0..nwords) << shl) (u64 little-endian)
+template <class C>
+__device__ __forceinline__ void load_value(int4* buf, const u64* src, int nwords, int role, int lane, int shl = 0) {
+    load_words<C>(buf, [src](int i) { return src[i]; }, nwords, shl, role, lane);
 }
 
 // The 32 inputs of a CTA step are contiguous in global memory: copy them with coalesced loads into a word-major staging area
@@ -87,34 +104,19 @@ __device__ __forceinline__ void stage_words(u64* stage, const u64* src, int unit
 }
 template <class C>
 __device__ __forceinline__ void load_value_staged(int4* buf, const u64* stage, int nwords, int role, int lane) {
-    int a[C::CH * 4];
-    int carry = 0;
-#pragma unroll
-    for (int k = 0; k < C::BL; k++) {
-        int bit = W * (role * C::BL + k);
-        int wi = bit >> 6, sh = bit & 63;
-        u64 lo = wi < nwords ? stage[wi * 33 + lane] : 0, hi = wi + 1 < nwords ? stage[(wi + 1) * 33 + lane] : 0;
-        u64 v = sh ? (lo >> sh) | (hi << (64 - sh)) : lo;
-        int t = (int)(v & ((1u << W) - 1)) + carry;
-        int d = sgxt28(t);
-        carry = (t - d) >> W;
-        a[k] = d;
-    }
-#pragma unroll
-    for (int k = C::BL; k < C::CH * 4; k++) a[k] = 0;
-    store_block<C>(blk_ptr<C>(buf, role, lane), a);
-    __syncthreads();
-    if (role + 1 < C::G) *(int*)blk_ptr<C>(buf, role + 1, lane) += carry;
-    __syncthreads();
+    load_words<C>(buf, [stage, lane](int i) { return stage[i * 33 + lane]; }, nwords, 0, role, lane);
 }
 
+// per-lane buffer <- 1 where cond (the others keep their value); barrier
 template <class C>
-__device__ __forceinline__ void set_one(int4* buf, int role, int lane) {
-    int a[C::CH * 4];
+__device__ __forceinline__ void set_one_where(int4* buf, bool cond, int role, int lane) {
+    if (cond) {
+        int a[C::CH * 4];
 #pragma unroll
-    for (int k = 0; k < C::CH * 4; k++) a[k] = 0;
-    if (role == 0) a[0] = 1;
-    store_block<C>(blk_ptr<C>(buf, role, lane), a);
+        for (int k = 0; k < C::CH * 4; k++) a[k] = 0;
+        if (role == 0) a[0] = 1;
+        store_block<C>(blk_ptr<C>(buf, role, lane), a);
+    }
     __syncthreads();
 }
 
@@ -180,20 +182,31 @@ __device__ __forceinline__ void mm(SV& S, const int4* Y, int role, int lane) {
     if constexpr (ENG >= 2) mulmod_u<C, View<C, ENG>::LG, SQR, ENG != 4>(S, Y);
     else mulmod<C, SQR, ENG == 1>(S, Y, role, lane);
 }
-// per-key constants into shared memory (+ TMEM and mbarriers for block28u)
-template <class C, int ENG, class SV>
-__device__ __forceinline__ void cta_begin(SV& S, int4* smem_base, const B28Dev& K) {
-    if constexpr (ENG >= 2) {
-        typedef UL<C, View<C, ENG>::LG> U;
-        int4* dst = (int4*)((unsigned char*)smem_base + U::OFF_CONST);
-        const int4* src = ENG == 3 ? K.uconsts2 : K.uconsts;
-        for (int i = threadIdx.x; i < U::KEY_BYTES / 16; i += U::THREADS) dst[i] = src[i];
-        umma_setup<C, View<C, ENG>::LG>(S);
-    } else load_consts<C>(smem_base, K);
+// Per-key constants into shared memory (+ TMEM and mbarriers for block28u), by the kernel's shared-memory view: Smem<C> (IMAD and
+// mma.sync phases) takes the constant block, SmemU<C, LG, WIT> (tcgen05 phases) its layout's image, the two-lane-group one for LG 2
+// (K.uconsts of the witness engine's descriptor is the witness modulus's image)
+template <class C>
+__device__ __forceinline__ void cta_begin(Smem<C>&, int4* smem_base, const B28Dev& K) { load_consts<C>(smem_base, K); }
+template <class C, int LG, bool WIT>
+__device__ __forceinline__ void cta_begin(SmemU<C, LG, WIT>& S, int4* smem_base, const B28Dev& K) {
+    typedef UL<C, LG, WIT> U;
+    int4* dst = (int4*)((unsigned char*)smem_base + U::OFF_CONST);
+    const int4* src = LG == 2 ? K.uconsts2 : K.uconsts;
+    for (int i = threadIdx.x; i < U::KEY_BYTES / 16; i += U::THREADS) dst[i] = src[i];
+    umma_setup(S);
 }
-template <class C, int ENG, class SV>
-__device__ __forceinline__ void cta_end(SV& S) {
-    if constexpr (ENG >= 2) umma_teardown<C, View<C, ENG>::LG>(S);
+template <class C>
+__device__ __forceinline__ void cta_end(Smem<C>&) {}
+template <class C, int LG, bool WIT>
+__device__ __forceinline__ void cta_end(SmemU<C, LG, WIT>& S) { umma_teardown(S); }
+
+// The unit of a lane: the 32 lanes of lane group grp take consecutive units from first + 32 grp (first: the CTA's first unit, LG
+// groups of 32 per CTA).  A lane past `count` works on unit count - 1 and is not active: it multiplies like the others, stores nothing.
+struct LaneUnit { size_t unit; bool active; };
+template <int LG = 1>
+__device__ __forceinline__ LaneUnit lane_unit(size_t count, int lane, int grp = 0, size_t first = (size_t)blockIdx.x * (32 * LG)) {
+    const size_t u = first + grp * 32 + lane;
+    return {u < count ? u : count - 1, u < count};
 }
 
 // V <- V * (constant in shared memory, ENTRY4 int4, broadcast)
@@ -295,7 +308,7 @@ __global__ void __launch_bounds__(C::THREADS, 1) k_gtable_fill(B28Dev K, const i
     if (!active) win = K.n_windows - 1;
     const int nd = 1 << K.comb_bits;
     int4* row = tg + (size_t)win * nd * C::ENTRY4;
-    set_one<C>(S.V, role, lane);
+    set_one_where<C>(S.V, true, role, lane);
     if (active) scatter_entry<C>(row, S.V, role, lane);
     gather_entry<C>(S.V, bases + (size_t)win * C::ENTRY4, role, lane);
     gather_entry<C>(S.B, bases + (size_t)win * C::ENTRY4, role, lane);
@@ -326,94 +339,21 @@ __device__ __forceinline__ void slot_release(const SlotPool& P, int slot) {
 }
 __global__ void k_nsmid(unsigned* out) { unsigned v; asm volatile("mov.u32 %0, %%nsmid;" : "=r"(v)); *out = v; }
 
-template <class C, int ENG>
-__global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k_encrypt(B28Dev K, const u64* __restrict__ m, const u64* __restrict__ r,
-                                                            size_t count, u64* __restrict__ c_out, int4* scratch, SlotPool pool) {
-    extern __shared__ int4 smem[];
-    __shared__ int s_slot[2];
-    constexpr int LG = View<C, ENG>::LG;
-    typename View<C, ENG>::type S(smem);
-    const int lane = threadIdx.x & 31, role = (threadIdx.x >> 5) % C::G, grp = (threadIdx.x >> 5) / C::G;      // grp: lane group (LG per CTA)
-    if (threadIdx.x == 0) for (int g = 0; g < LG; g++) s_slot[g] = slot_acquire(pool);
-    cta_begin<C, ENG>(S, smem, K);
-    const int slot = s_slot[grp];
-    size_t unit = (size_t)blockIdx.x * (32 * LG) + grp * 32 + lane;
-    const bool active = unit < count;
-    if (!active) unit = count - 1;
-    int4* tab = scratch + (size_t)slot * SCRATCH_ENTRIES * C::VAL4;
-    // ---- r^n: odd powers table, then the per-key window schedule
-    load_value<C>(S.V, r + unit * K.words_in, K.words_in, role, lane);
-    copy_to_global<C>(tab, S.V, role, lane);                                   // tab[0] = r
-    mm<C, true, ENG>(S, nullptr, role, lane);                                   // r^2
-    copy_to_global<C>(tab + (size_t)TABN * C::VAL4, S.V, role, lane);
-    __syncthreads();
-    copy_from_global<C>(S.V, tab, role, lane);
-    for (int j = 1; j < TABN; j++) {
-        copy_from_global<C>(S.B, tab + (size_t)TABN * C::VAL4, role, lane);
-        mm<C, false, ENG>(S, S.B, role, lane);                                  // r^(2j+1)
-        copy_to_global<C>(tab + (size_t)j * C::VAL4, S.V, role, lane);
-    }
-    __syncthreads();
-    copy_from_global<C>(S.V, tab + (size_t)K.first_idx * C::VAL4, role, lane);
-    for (int o = 0; o < K.n_ops; o++) {
-        int2 op = K.ops[o];
-        for (int s = 0; s < op.x; s++) mm<C, true, ENG>(S, nullptr, role, lane);
-        if (op.y >= 0) {
-            copy_from_global<C>(S.B, tab + (size_t)op.y * C::VAL4, role, lane);
-            mm<C, false, ENG>(S, S.B, role, lane);
-        }
-    }
-    copy_to_global<C>(tab + (size_t)(TABN + 1) * C::VAL4, S.V, role, lane);    // rn
-    __syncthreads();
-    // ---- g^m: comb over the bytes of m
-    const u64* mw = m + unit * K.words_in;
-    const int cb = K.comb_bits;
-    auto comb_digit = [&](int i) -> int {
-        const int bit = i * cb, w = bit >> 6, sft = bit & 63;
-        u64 v = mw[w] >> sft;
-        if (sft + cb > 64 && w + 1 < K.words_in) v |= mw[w + 1] << (64 - sft);
-        return (int)(v & ((1u << cb) - 1));
-    };
-    if (K.n_entry) {
-        // g = n + 1: (1 + n)^m = 1 + m n (mod n^2) — one multiplication by the per-key constant n instead of the comb
-        load_value<C>(S.V, mw, K.words_in, role, lane);
-        mulmod_const<C, ENG>(S, K.n_entry, role, lane);
-        if (role == 0) ((int*)blk_ptr<C>(S.V, 0, lane))[0] += 1;
-        __syncthreads();
-    } else {
-        gather_entry<C>(S.V, K.tg + (size_t)comb_digit(0) * C::ENTRY4, role, lane);
-        for (int i = 1; i < K.n_windows; i++) {
-            gather_entry<C>(S.B, K.tg + (((size_t)i << cb) + comb_digit(i)) * C::ENTRY4, role, lane);
-            mm<C, false, ENG>(S, S.B, role, lane);
-        }
-    }
-    // ---- c = gm * rn, canonical
-    copy_from_global<C>(S.B, tab + (size_t)(TABN + 1) * C::VAL4, role, lane);
-    mm<C, false, ENG>(S, S.B, role, lane);
-    finalize<C, ENG>(S, K, c_out + unit * K.words_out, active, role, lane);
-    if (threadIdx.x == 0) for (int g = 0; g < LG; g++) slot_release(pool, s_slot[g]);
-    cta_end<C, ENG>(S);
+// the slots of a CTA's LG lane groups, s_slot[g] in shared memory: thread 0 takes them before cta_begin (whose barrier publishes
+// them) and gives them back when the CTA ends
+template <int LG>
+__device__ __forceinline__ void slots_acquire(const SlotPool& P, int* s_slot) {
+    if (threadIdx.x == 0) for (int g = 0; g < LG; g++) s_slot[g] = slot_acquire(P);
+}
+template <int LG>
+__device__ __forceinline__ void slots_release(const SlotPool& P, const int* s_slot) {
+    if (threadIdx.x == 0) for (int g = 0; g < LG; g++) slot_release(P, s_slot[g]);
 }
 
-// out = base^e mod n^2 for a per-key exponent e: the r-chain of k_encrypt (odd-power table in the CTA's scratch slot, sliding-window
-// schedule computed once per key) with its own schedule.  Decryption's c^lambda mod n^2 (SURVEY.md 8f-4).
-struct PowSched { const int2* ops; int n_ops; int first_idx; };
-template <class C, int ENG>
-__global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k_pow(B28Dev K, PowSched E, const u64* __restrict__ base, int base_words,
-                                                                    size_t count, u64* __restrict__ out, int4* scratch, SlotPool pool) {
-    extern __shared__ int4 smem[];
-    __shared__ int s_slot[2];
-    constexpr int LG = View<C, ENG>::LG;
-    typename View<C, ENG>::type S(smem);
-    const int lane = threadIdx.x & 31, role = (threadIdx.x >> 5) % C::G, grp = (threadIdx.x >> 5) / C::G;      // grp: lane group (LG per CTA)
-    if (threadIdx.x == 0) for (int g = 0; g < LG; g++) s_slot[g] = slot_acquire(pool);
-    cta_begin<C, ENG>(S, smem, K);
-    const int slot = s_slot[grp];
-    size_t unit = (size_t)blockIdx.x * (32 * LG) + grp * 32 + lane;
-    const bool active = unit < count;
-    if (!active) unit = count - 1;
-    int4* tab = scratch + (size_t)slot * SCRATCH_ENTRIES * C::VAL4;
-    load_value<C>(S.V, base + unit * base_words, base_words, role, lane);
+// V <- x^e for the x in V (each lane its own), e given by its sliding-window schedule E; e == 0 gives 1.  The odd powers x, x^3, ..,
+// x^(2 TABN - 1) go to tab[0 .. TABN) of the CTA's scratch slot, x^2 to tab[TABN].
+template <class C, int ENG, class SV>
+__device__ __forceinline__ void window_pow(SV& S, const PowSched& E, int4* tab, int role, int lane) {
     copy_to_global<C>(tab, S.V, role, lane);                                        // tab[0] = x
     mm<C, true, ENG>(S, nullptr, role, lane);                                   // x^2
     copy_to_global<C>(tab + (size_t)TABN * C::VAL4, S.V, role, lane);
@@ -425,7 +365,7 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
         copy_to_global<C>(tab + (size_t)j * C::VAL4, S.V, role, lane);
     }
     __syncthreads();
-    if (E.first_idx < 0) set_one<C>(S.V, role, lane);                               // e == 0
+    if (E.first_idx < 0) set_one_where<C>(S.V, true, role, lane);                   // e == 0
     else copy_from_global<C>(S.V, tab + (size_t)E.first_idx * C::VAL4, role, lane);
     for (int o = 0; o < E.n_ops; o++) {
         const int2 op = E.ops[o];
@@ -435,9 +375,76 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
             mm<C, false, ENG>(S, S.B, role, lane);
         }
     }
+}
+
+// c-bit window i (c <= 16) of the unsigned integer w[0 .. nwords) (u64 little-endian): bits [i c, i c + c)
+__device__ __forceinline__ int window_digit(const u64* w, int nwords, int i, int c) {
+    const int bit = i * c, wi = bit >> 6, sft = bit & 63;
+    u64 v = w[wi] >> sft;
+    if (sft + c > 64 && wi + 1 < nwords) v |= w[wi + 1] << (64 - sft);
+    return (int)(v & ((1u << c) - 1));
+}
+
+template <class C, int ENG>
+__global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k_encrypt(B28Dev K, const u64* __restrict__ m, const u64* __restrict__ r,
+                                                            size_t count, u64* __restrict__ c_out, int4* scratch, SlotPool pool) {
+    extern __shared__ int4 smem[];
+    __shared__ int s_slot[2];
+    constexpr int LG = View<C, ENG>::LG;
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = (threadIdx.x >> 5) % C::G, grp = (threadIdx.x >> 5) / C::G;      // grp: lane group (LG per CTA)
+    slots_acquire<LG>(pool, s_slot);
+    cta_begin(S, smem, K);
+    const auto [unit, active] = lane_unit<LG>(count, lane, grp);
+    int4* tab = scratch + (size_t)s_slot[grp] * SCRATCH_ENTRIES * C::VAL4;
+    // ---- r^n: odd powers table, then the per-key window schedule
+    load_value<C>(S.V, r + unit * K.words_in, K.words_in, role, lane);
+    window_pow<C, ENG>(S, K.rn, tab, role, lane);
+    copy_to_global<C>(tab + (size_t)(TABN + 1) * C::VAL4, S.V, role, lane);    // rn
+    __syncthreads();
+    // ---- g^m: comb over the bytes of m
+    const u64* mw = m + unit * K.words_in;
+    const int cb = K.comb_bits;
+    if (K.n_entry) {
+        // g = n + 1: (1 + n)^m = 1 + m n (mod n^2) — one multiplication by the per-key constant n instead of the comb
+        load_value<C>(S.V, mw, K.words_in, role, lane);
+        mulmod_const<C, ENG>(S, K.n_entry, role, lane);
+        if (role == 0) ((int*)blk_ptr<C>(S.V, 0, lane))[0] += 1;
+        __syncthreads();
+    } else {
+        gather_entry<C>(S.V, K.tg + (size_t)window_digit(mw, K.words_in, 0, cb) * C::ENTRY4, role, lane);
+        for (int i = 1; i < K.n_windows; i++) {
+            gather_entry<C>(S.B, K.tg + (((size_t)i << cb) + window_digit(mw, K.words_in, i, cb)) * C::ENTRY4, role, lane);
+            mm<C, false, ENG>(S, S.B, role, lane);
+        }
+    }
+    // ---- c = gm * rn, canonical
+    copy_from_global<C>(S.B, tab + (size_t)(TABN + 1) * C::VAL4, role, lane);
+    mm<C, false, ENG>(S, S.B, role, lane);
+    finalize<C, ENG>(S, K, c_out + unit * K.words_out, active, role, lane);
+    slots_release<LG>(pool, s_slot);
+    cta_end(S);
+}
+
+// out = base^e mod n^2 for a per-key exponent e: the r-chain of k_encrypt (window_pow) with its own schedule.  Decryption's
+// c^lambda mod n^2 (SURVEY.md 8f-4).
+template <class C, int ENG>
+__global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k_pow(B28Dev K, PowSched E, const u64* __restrict__ base, int base_words,
+                                                                    size_t count, u64* __restrict__ out, int4* scratch, SlotPool pool) {
+    extern __shared__ int4 smem[];
+    __shared__ int s_slot[2];
+    constexpr int LG = View<C, ENG>::LG;
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = (threadIdx.x >> 5) % C::G, grp = (threadIdx.x >> 5) / C::G;      // grp: lane group (LG per CTA)
+    slots_acquire<LG>(pool, s_slot);
+    cta_begin(S, smem, K);
+    const auto [unit, active] = lane_unit<LG>(count, lane, grp);
+    int4* tab = scratch + (size_t)s_slot[grp] * SCRATCH_ENTRIES * C::VAL4;
+    load_value<C>(S.V, base + unit * base_words, base_words, role, lane);
+    window_pow<C, ENG>(S, E, tab, role, lane);
     finalize<C, ENG>(S, K, out + unit * K.words_out, active, role, lane);
-    if (threadIdx.x == 0) for (int g = 0; g < LG; g++) slot_release(pool, s_slot[g]);
-    cta_end<C, ENG>(S);
+    slots_release<LG>(pool, s_slot);
+    cta_end(S);
 }
 
 // out = c^k mod n^2 with its own scalar k per lane: homomorphic scalar multiplication, Dec(c^k) = k Dec(c) mod n.  Fixed window of
@@ -446,15 +453,6 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
 // never depends on the lane and the lanes of a CTA share every mulmod.  The chain is as long as the CTA's longest scalar.
 constexpr int SCALAR_MAXW = 5;
 static_assert((1 << SCALAR_MAXW) <= SCRATCH_ENTRIES, "the scalar window's table must fit the CTA's scratch slot");
-
-// smem per-lane value <- entry d (this lane's own) of a per-lane table in the [entry][blk][chunk][lane] layout
-template <class C>
-__device__ __forceinline__ void copy_from_global_lane(int4* buf, const int4* tab, int d, int role, int lane) {
-    const int4* e = tab + (size_t)d * C::VAL4;
-#pragma unroll
-    for (int c = 0; c < C::CH; c++) buf[(role * C::CH + c) * 32 + lane] = e[(role * C::CH + c) * 32 + lane];
-    __syncthreads();
-}
 
 template <class C, int ENG>
 __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k_scalar(B28Dev K, const u64* __restrict__ c, const u64* __restrict__ k,
@@ -466,13 +464,11 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
     constexpr int LG = View<C, ENG>::LG;
     typename View<C, ENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = (threadIdx.x >> 5) % C::G, grp = (threadIdx.x >> 5) / C::G;      // grp: lane group (LG per CTA)
-    if (threadIdx.x == 0) { for (int g = 0; g < LG; g++) s_slot[g] = slot_acquire(pool); s_bits = 0; }
-    cta_begin<C, ENG>(S, smem, K);
-    const int slot = s_slot[grp];
-    size_t unit = (size_t)blockIdx.x * (32 * LG) + grp * 32 + lane;
-    const bool active = unit < count;
-    if (!active) unit = count - 1;
-    int4* tab = scratch + (size_t)slot * SCRATCH_ENTRIES * C::VAL4;
+    slots_acquire<LG>(pool, s_slot);
+    if (threadIdx.x == 0) s_bits = 0;
+    cta_begin(S, smem, K);
+    const auto [unit, active] = lane_unit<LG>(count, lane, grp);
+    int4* tab = scratch + (size_t)s_slot[grp] * SCRATCH_ENTRIES * C::VAL4;
     const u64* kw = k + unit * k_words;
     // chain length: bits of the CTA's longest scalar (over both lane groups)
     if (role == 0 && active) {
@@ -483,7 +479,7 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
     // table: tab[0] = 1, tab[1] = x, tab[e] = x^e (even e by squaring x^(e/2), odd e as x^(e-1) * x)
     load_value<C>(S.V, c + unit * K.words_out, K.words_out, role, lane);
     copy_to_global<C>(tab + C::VAL4, S.V, role, lane);
-    set_one<C>(S.B, role, lane);
+    set_one_where<C>(S.B, true, role, lane);
     copy_to_global<C>(tab, S.B, role, lane);
     for (int e = 2; e < (1 << w); e++) {
         if (e & 1) {
@@ -496,23 +492,18 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
         copy_to_global<C>(tab + (size_t)e * C::VAL4, S.V, role, lane);
     }
     __syncthreads();
+    // the chain: window digits straight from the scalar, table entries from this lane's own column
     const int nwin = (s_bits + w - 1) / w;
-    auto digit = [&](int i) -> int {
-        const int bit = i * w, wi = bit >> 6, sft = bit & 63;
-        u64 v = kw[wi] >> sft;
-        if (sft + w > 64 && wi + 1 < k_words) v |= kw[wi + 1] << (64 - sft);
-        return (int)(v & ((1u << w) - 1));
-    };
-    if (nwin == 0) set_one<C>(S.V, role, lane);                                        // every scalar of the CTA is 0
-    else copy_from_global_lane<C>(S.V, tab, digit(nwin - 1), role, lane);
+    if (nwin == 0) set_one_where<C>(S.V, true, role, lane);                            // every scalar of the CTA is 0
+    else copy_from_global<C>(S.V, tab + (size_t)window_digit(kw, k_words, nwin - 1, w) * C::VAL4, role, lane);
     for (int i = nwin - 2; i >= 0; i--) {
         for (int s_ = 0; s_ < w; s_++) mm<C, true, ENG>(S, nullptr, role, lane);
-        copy_from_global_lane<C>(S.B, tab, digit(i), role, lane);
+        copy_from_global<C>(S.B, tab + (size_t)window_digit(kw, k_words, i, w) * C::VAL4, role, lane);
         mm<C, false, ENG>(S, S.B, role, lane);
     }
     finalize<C, ENG>(S, K, out + unit * K.words_out, active, role, lane);
-    if (threadIdx.x == 0) for (int g = 0; g < LG; g++) slot_release(pool, s_slot[g]);
-    cta_end<C, ENG>(S);
+    slots_release<LG>(pool, s_slot);
+    cta_end(S);
 }
 
 // ---- tally: the N-ary fold of paillier_add_native (/root/reference/src/paillier.rs:94-97) in ONE launch per GPU -------------------
@@ -541,17 +532,6 @@ __device__ __forceinline__ void copy_from_global_cg(int4* buf, const int4* g, in
     for (int c = 0; c < C::CH; c++) buf[(role * C::CH + c) * 32 + lane] = __ldcg(g + (role * C::CH + c) * 32 + lane);
     __syncthreads();
 }
-template <class C>
-__device__ __forceinline__ void set_one_where(int4* buf, bool cond, int role, int lane) {
-    if (cond) {
-        int a[C::CH * 4];
-#pragma unroll
-        for (int k = 0; k < C::CH * 4; k++) a[k] = 0;
-        if (role == 0) a[0] = 1;
-        store_block<C>(blk_ptr<C>(buf, role, lane), a);
-    }
-    __syncthreads();
-}
 // V[lane] <- product over the lanes of its aligned group of `width` lanes (width a power of two <= 32)
 template <class C, int ENG, class SV>
 __device__ __forceinline__ void fold_lanes(SV& S, int width, int role, int lane) {
@@ -570,12 +550,12 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_tally(B28D
     __shared__ int s_first;
     typename View<C, ENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    cta_begin<C, ENG>(S, smem, K);
+    cta_begin(S, smem, K);
     // ---- 1. main loop
     const size_t stride = (size_t)gridDim.x * 32;
     const size_t first = (size_t)blockIdx.x * 32 + lane;
     const size_t max_iters = (count + stride - 1) / stride;
-    set_one<C>(S.V, role, lane);
+    set_one_where<C>(S.V, true, role, lane);
     for (size_t it = 0; it < max_iters; it++) {
         const size_t u = first + it * stride;
         const size_t base = (size_t)blockIdx.x * 32 + it * stride;                  // first unit of this CTA step
@@ -597,7 +577,7 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_tally(B28D
                 __syncthreads();
                 if (threadIdx.x == 0) s_first = atomicAdd(node_cnt + node_base + j, 1u) == 0u;
                 __syncthreads();
-                if (s_first) { cta_end<C, ENG>(S); return; }                                              // the sibling will pick this value up
+                if (s_first) { cta_end(S); return; }                                              // the sibling will pick this value up
                 if (threadIdx.x == 0) node_cnt[node_base + j] = 0;                   // both arrived: ready for the next launch
                 __threadfence();
                 copy_from_global_cg<C>(S.B, slot + (size_t)((idx & 1) ^ 1) * C::VAL4, role, lane);
@@ -609,7 +589,7 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_tally(B28D
     }
     // ---- 3. the surviving CTA: fold its lanes, canonical partial
     fold_lanes<C, ENG>(S, 32, role, lane);
-    if (P.world <= 1) { finalize<C, ENG>(S, K, out, lane == 0, role, lane); cta_end<C, ENG>(S); return; }
+    if (P.world <= 1) { finalize<C, ENG>(S, K, out, lane == 0, role, lane); cta_end(S); return; }
     // ---- 4. exchange over peer memory and combine.  What crosses NVLink is lane 0's LAZY value (strict digits, ENTRY4 int4): the
     // receivers multiply digit arrays directly, so neither a canonicalisation before the exchange nor a digit conversion after it
     const int par = (int)(P.epoch & 1);
@@ -649,7 +629,7 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_tally(B28D
     int width = 1; while (width < P.world) width <<= 1;
     fold_lanes<C, ENG>(S, width, role, lane);
     finalize<C, ENG>(S, K, out, lane == 0, role, lane);
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 // ---- matvec: bucket (Pippenger) multi-exponentiation, DESIGN.md §9b ------------------------------------------------------------
@@ -681,12 +661,12 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_bucket_fol
     const bool last = lanes <= 1;
     if (blockIdx.x == 0 && threadIdx.x == 0) *d_n_next = last ? 0u : (unsigned)(2 * lanes);
     if ((size_t)blockIdx.x * 32 >= lanes) return;                                   // the whole CTA is past the list
-    cta_begin<C, ENG>(S, smem, K);
+    cta_begin(S, smem, K);
     const size_t l = (size_t)blockIdx.x * 32 + lane, a = l * ls;
     const bool active = l < lanes;
     unsigned cur = active ? keys[a] : 0u;
     bool head = true;
-    set_one<C>(S.V, role, lane);
+    set_one_where<C>(S.V, true, role, lane);
     for (int it = 0; it < ls; it++) {
         const size_t t = a + it;
         const bool real = active && t < n;
@@ -712,7 +692,7 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_bucket_fol
             if (role == 0) { keys_next[2 * l + 1] = cur; if (head) keys_next[2 * l] = cur; }
         }
     }
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 // Buckets B_1 .. B_(2^c - 1) of a set -> per segment [a, a + lseg): T = prod B_d^(d - a + 1) and A = prod B_d, as running products from
@@ -726,16 +706,14 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_bucket_red
     extern __shared__ int4 smem[];
     typename View<C, ENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    cta_begin<C, ENG>(S, smem, K);
-    size_t unit = (size_t)blockIdx.x * 32 + lane;
-    const bool active = unit < units;
-    if (!active) unit = units - 1;
+    cta_begin(S, smem, K);
+    const auto [unit, active] = lane_unit(units, lane);
     const size_t set = unit / nseg;
     const int a = 1 + (int)(unit % nseg) * lseg, dmax = (1 << c) - 1;
     const int4* bk = buckets + (set << c) * C::ENTRY4;
     int4* sa = scratch + (size_t)blockIdx.x * 2 * C::VAL4;
     int4* stt = sa + C::VAL4;
-    set_one<C>(S.V, role, lane);
+    set_one_where<C>(S.V, true, role, lane);
     copy_to_global<C>(sa, S.V, role, lane);                                             // A = 1, T = 1 (in V)
     for (int it = lseg - 1; it >= 0; it--) {
         const int d = a + it;
@@ -755,7 +733,7 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_bucket_red
     copy_from_global<C>(S.V, sa, role, lane);
     finalize<C, ENG>(S, K, a_out + unit * K.words_out, active, role, lane);
     if (active && threadIdx.x < 32) a_exp[unit] = (u64)(a - 1);
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 // x_u <- x_u^(2^(c * jg)) * prod_jl W_(u, jl)^(2^(c * jl)) (Horner over a group of windows, most significant first), one lane per
@@ -765,10 +743,8 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_horner(B28
     extern __shared__ int4 smem[];
     typename View<C, ENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    cta_begin<C, ENG>(S, smem, K);
-    size_t unit = (size_t)blockIdx.x * 32 + lane;
-    const bool active = unit < units;
-    if (!active) unit = units - 1;
+    cta_begin(S, smem, K);
+    const auto [unit, active] = lane_unit(units, lane);
     load_value<C>(S.V, x + unit * K.words_out, K.words_out, role, lane);
     for (int jl = jg - 1; jl >= 0; jl--) {
         for (int s_ = 0; s_ < c; s_++) mm<C, true, ENG>(S, nullptr, role, lane);
@@ -776,7 +752,7 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_horner(B28
         mm<C, false, ENG>(S, S.B, role, lane);
     }
     finalize<C, ENG>(S, K, x + unit * K.words_out, active, role, lane);
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 // lazy digits -> canonical words, one lane per value
@@ -785,13 +761,11 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_lazy_canon
     extern __shared__ int4 smem[];
     typename View<C, ENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    cta_begin<C, ENG>(S, smem, K);
-    size_t unit = (size_t)blockIdx.x * 32 + lane;
-    const bool active = unit < count;
-    if (!active) unit = count - 1;
+    cta_begin(S, smem, K);
+    const auto [unit, active] = lane_unit(count, lane);
     gather_entry<C>(S.V, in + unit * C::ENTRY4, role, lane);
     finalize<C, ENG>(S, K, out + unit * K.words_out, active, role, lane);
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 // Digits of one pass (rows [r0, r0 + rb), ciphertexts [i0, i0 + nc), windows [j0, j0 + jg)), one thread per (row, ciphertext): every
@@ -805,10 +779,7 @@ __global__ void k_mv_digits(const u64* __restrict__ w, const uint8_t* __restrict
     const u64* m = w + e * kw;
     const unsigned sgn = neg && neg[e] ? 1u : 0u;
     for (int jl = 0; jl < jg; jl++) {
-        const int bit = (j0 + jl) * c, wi = bit >> 6, sft = bit & 63;
-        u64 v = m[wi] >> sft;
-        if (sft + c > 64 && wi + 1 < kw) v |= m[wi + 1] << (64 - sft);
-        const unsigned d = (unsigned)(v & ((1ull << c) - 1));
+        const unsigned d = (unsigned)window_digit(m, kw, j0 + jl, c);
         if (!d) continue;
         const unsigned key = (((sgn * (unsigned)rb + (unsigned)r) * (unsigned)jg + (unsigned)jl) << c) + d;
         const unsigned p = atomicAdd(cursor + key, 1u);
@@ -876,7 +847,7 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
     typename View<C, ENG>::type S(smem);
     constexpr int LG = View<C, ENG>::LG;
     const int lane = threadIdx.x & 31, role = (threadIdx.x >> 5) % C::G, grp = (threadIdx.x >> 5) / C::G;      // every lane group works on the same input
-    cta_begin<C, ENG>(S, smem, K);
+    cta_begin(S, smem, K);
     copy_from_global<C>(S.V, v_in, role, lane);
     if (t_out) {            // phase A alone
         if (y_in) copy_from_global<C>(S.B, y_in, role, lane);
@@ -905,7 +876,7 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
         }
         __syncthreads();
     }
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 
@@ -917,7 +888,7 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
     typename View<C, ENG>::type S(smem);
     constexpr int LG = View<C, ENG>::LG;
     const int lane = threadIdx.x & 31, role = (threadIdx.x >> 5) % C::G;
-    cta_begin<C, ENG>(S, smem, K);
+    cta_begin(S, smem, K);
     copy_from_global<C>(S.V, v_in, role, lane);
     __shared__ unsigned s_order;
     if (threadIdx.x == 0) s_order = atomicAdd(sm_count + smid(), 1u);
@@ -953,7 +924,7 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
         ta += t1 - t0; tb += t2 - t1;
     }
     if (threadIdx.x == 0) { cyc[3 * blockIdx.x] = ta; cyc[3 * blockIdx.x + 1] = tb; cyc[3 * blockIdx.x + 2] = clock64() - t_begin; }
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 // ---- witness kernels (reference chain with exact (q, rem) per mul_mod) ---------------------------------
@@ -974,35 +945,6 @@ struct WitIO {
     int4* scratch;             // 2 values per CTA: acc of the r-chain, gm
 };
 
-// per-lane buffer <- strict digits of (src << shl)
-template <class C>
-__device__ __forceinline__ void load_value_shl(int4* buf, const u64* src, int nwords, int shl, int role, int lane) {
-    int a[C::CH * 4];
-    int carry = 0;
-#pragma unroll
-    for (int k = 0; k < C::BL; k++) {
-        const int bit = W * (role * C::BL + k) - shl;
-        u64 v = 0;
-        if (bit >= 0) {
-            const int wi = bit >> 6, sh = bit & 63;
-            const u64 lo = wi < nwords ? src[wi] : 0, hi = wi + 1 < nwords ? src[wi + 1] : 0;
-            v = sh ? (lo >> sh) | (hi << (64 - sh)) : lo;
-        } else if (bit > -W) {
-            v = src[0] << (-bit);
-        }
-        const int t = (int)(v & ((1u << W) - 1)) + carry;
-        const int d = sgxt28(t);
-        carry = (t - d) >> W;
-        a[k] = d;
-    }
-#pragma unroll
-    for (int k = C::BL; k < C::CH * 4; k++) a[k] = 0;
-    store_block<C>(blk_ptr<C>(buf, role, lane), a);
-    __syncthreads();
-    if (role + 1 < C::G) *(int*)blk_ptr<C>(buf, role + 1, lane) += carry;
-    __syncthreads();
-}
-
 // ---- witness engine selection: 0 = block28t arithmetic (mma.sync phases), 1 = block28u arithmetic (tcgen05 phases) ---------------
 template <class C, int WENG> struct WView {
     typedef Smem<C> type;
@@ -1016,18 +958,22 @@ template <class C> struct WView<C, 1> {
     static constexpr size_t BYTES = UL<C, 1, true>::SMEM_BYTES;
     static constexpr int PER_SM = UL<C, 1, true>::CTAS_PER_SM, THREADS = C::THREADS;
 };
-template <class C, int WENG, class SV>
-__device__ __forceinline__ void w_begin(SV& S, int4* smem_base, const B28Dev& K) {
-    if constexpr (WENG == 1) {
-        typedef UL<C, 1, true> U;
-        int4* dst = (int4*)((unsigned char*)smem_base + U::OFF_CONST);
-        for (int i = threadIdx.x; i < U::KEY_BYTES / 16; i += C::THREADS) dst[i] = K.uconsts[i];
-        umma_setup<C, 1, true>(S);
-    } else load_consts<C>(smem_base, K);
-}
-template <class C, int WENG, class SV>
-__device__ __forceinline__ void w_end(SV& S) {
-    if constexpr (WENG == 1) umma_teardown<C, 1, true>(S);
+// q of the last witnessed mul_mod must fit words_out words (range check of assign_integer(q, 2*enc_bits), SURVEY.md A.4): true
+// when this thread's block of the canonical q digits, which the step leaves in T, has a bit at or above 64 words_out
+template <class C, class SV>
+__device__ __forceinline__ bool q_too_wide(const SV& S, int words_out, int role, int lane) {
+    const int* Qf = (const int*)S.T + C::L * 32;
+    const int qbits = 64 * words_out;
+    int bad = 0;
+#pragma unroll
+    for (int k = 0; k < C::BL; k++) {
+        const int p = role * C::BL + k;
+        const unsigned d = (unsigned)Qf[p * 32 + lane];
+        const int lo = W * p;
+        if (lo >= qbits) bad |= d != 0;
+        else if (lo + W > qbits) bad |= (d >> (qbits - lo)) != 0;
+    }
+    return bad;
 }
 // one witnessed mul_mod (contract of mulmod_w, block28.cuh)
 template <class C, int WENG, class SV>
@@ -1049,21 +995,8 @@ __global__ void k_wtab(const u64* __restrict__ g_words, int words_in, const u64*
     int* dst = (int*)(gtab + (size_t)i * C::ENTRY4);
     for (int k = 0; k < C::ENTRY4 * 4; k++) dst[k] = 0;
     int carry = 0;
-    for (int p = 0; p < C::L; p++) {
-        const int bit = W * p - shl;
-        u64 v = 0;
-        if (bit >= 0) {
-            const int wi = bit >> 6, sh = bit & 63;
-            const u64 lo = wi < nwords ? src[wi] : 0, hi = wi + 1 < nwords ? src[wi + 1] : 0;
-            v = sh ? (lo >> sh) | (hi << (64 - sh)) : lo;
-        } else if (bit > -W) {
-            v = src[0] << (-bit);
-        }
-        const int t = (int)(v & ((1u << W) - 1)) + carry;
-        const int d = sgxt28(t);
-        carry = (t - d) >> W;
-        dst[(p / C::BL) * C::CH * 4 + (p % C::BL)] = d;
-    }
+    for (int p = 0; p < C::L; p++)
+        dst[(p / C::BL) * C::CH * 4 + (p % C::BL)] = strict_digit([src](int wi) { return src[wi]; }, nwords, W * p - shl, carry);
 }
 
 // per-key g-chain on the witness engine: record i = (q, rem) of (g^(2^i))^2, i < n_bits, and the table entries
@@ -1074,21 +1007,14 @@ __global__ void __launch_bounds__(C::THREADS, 1) k_gchain_w(B28Dev K, WitDev Wd,
     extern __shared__ int4 smem[];
     typename WView<C, WENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    w_begin<C, WENG>(S, smem, K);
-    load_value_shl<C>(S.V, g_words, K.words_in, Wd.sh >> 1, role, lane);
+    cta_begin(S, smem, K);
+    load_value<C>(S.V, g_words, K.words_in, role, lane, Wd.sh >> 1);
     for (int i = 0; i < n_bits; i++) {
         if (lane == 0) scatter_entry<C>(gtab + (size_t)i * C::ENTRY4, S.V, role, lane);
         WStep o; o.rec = lane == 0 ? gchain + (size_t)i * 2 * K.words_out : nullptr; o.rem_out = nullptr;
         wmm<C, WENG>(smem, S, nullptr, 1, S.V, o, Wd.sh, K.words_out, Wd.inv, Wd.cpow);
     }
-    w_end<C, WENG>(S);
-}
-
-template <class C>
-__device__ __forceinline__ void bcast_entry(int4* buf, const int4* entry, int role, int lane) {
-#pragma unroll
-    for (int c = 0; c < C::CH; c++) buf[(role * C::CH + c) * 32 + lane] = __ldg(entry + role * C::CH + c);
-    __syncthreads();
+    cta_end(S);
 }
 
 // One unit per lane, the reference's chain (src/paillier.rs:51,55,57 -> pow_mod_fixed_exp, SURVEY.md A.5):
@@ -1102,10 +1028,8 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_witness(
     extern __shared__ int4 smem[];
     typename WView<C, WENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    w_begin<C, WENG>(S, smem, K);
-    size_t unit = (size_t)blockIdx.x * 32 + lane;
-    const bool active = unit < A.count;
-    if (!active) unit = A.count - 1;
+    cta_begin(S, smem, K);
+    const auto [unit, active] = lane_unit(A.count, lane);
     const int wo = K.words_out;
     const size_t recw = 2 * (size_t)wo;
     const u64* mw = A.m + unit * K.words_in;
@@ -1119,7 +1043,7 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_witness(
     int4* sc_acc = A.scratch + (size_t)blockIdx.x * 2 * C::VAL4;
     int4* sc_gm = sc_acc + C::VAL4;
     // ---- g-chain
-    bcast_entry<C>(S.V, Wd.one_s, role, lane);
+    gather_entry<C>(S.V, Wd.one_s, role, lane);
     {
         int wi = 0; u64 cur = mw[0];
         for (int t = 0; t < maxpc; t++) {
@@ -1131,7 +1055,7 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_witness(
                 cur &= cur - 1;
                 e = Wd.gtab + (size_t)(64 * wi + b) * C::ENTRY4;
             }
-            bcast_entry<C>(S.B, e, role, lane);
+            gather_entry<C>(S.B, e, role, lane);
             WStep o; o.rec = (act && rec) ? rec + (size_t)t * recw : nullptr; o.rem_out = nullptr;
             const u64 H = wmm<C, WENG>(smem, S, S.B, 0, S.V, o, Wd.sh, wo, Wd.inv, Wd.cpow);
             if (act) D = (D ^ H) * PB200_DIGEST_PRIME;
@@ -1139,9 +1063,9 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_witness(
     }
     copy_to_global<C>(sc_gm, S.V, role, lane);
     // ---- r-chain
-    bcast_entry<C>(S.B, Wd.one_s, role, lane);
+    gather_entry<C>(S.B, Wd.one_s, role, lane);
     copy_to_global<C>(sc_acc, S.B, role, lane);
-    load_value_shl<C>(S.V, A.r + unit * K.words_in, K.words_in, Wd.sh >> 1, role, lane);
+    load_value<C>(S.V, A.r + unit * K.words_in, K.words_in, role, lane, Wd.sh >> 1);
     size_t idx = (size_t)pc;
     for (int i = 0; i < Wd.exp_bits; i++) {
         const bool bit = (Wd.n_words[i >> 6] >> (i & 63)) & 1;
@@ -1169,7 +1093,7 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_witness(
         D = (D ^ H) * PB200_DIGEST_PRIME;
     }
     if (role == 0 && active && A.digest) A.digest[unit] = D;
-    w_end<C, WENG>(S);
+    cta_end(S);
 }
 
 // paillier_add_native / PaillierChip::add (src/paillier.rs:62-85, :94-97) for `count` pairs on the witness engine:
@@ -1182,36 +1106,20 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_add_w(B2
     extern __shared__ int4 smem[];
     typename WView<C, WENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    w_begin<C, WENG>(S, smem, K);
+    cta_begin(S, smem, K);
     const int wo = K.words_out;
     for (size_t first = (size_t)blockIdx.x * 32; first < count; first += (size_t)gridDim.x * 32) {
-        size_t unit = first + lane;
-        const bool active = unit < count;
-        if (!active) unit = count - 1;
-        load_value_shl<C>(S.V, c1 + unit * c_words, c_words, Wd.sh >> 1, role, lane);
-        load_value_shl<C>(S.B, c2 + unit * c_words, c_words, Wd.sh >> 1, role, lane);
+        const auto [unit, active] = lane_unit(count, lane, 0, first);
+        load_value<C>(S.V, c1 + unit * c_words, c_words, role, lane, Wd.sh >> 1);
+        load_value<C>(S.B, c2 + unit * c_words, c_words, role, lane, Wd.sh >> 1);
         // the record goes through a per-lane staging area only when q is wanted; rem alone is written directly
         WStep o; o.rec = nullptr; o.rem_out = active ? out + unit * wo : nullptr;
         o.q_out = (active && q_out) ? q_out + unit * wo : nullptr;
         wmm<C, WENG>(smem, S, S.B, 0, nullptr, o, Wd.sh, wo, Wd.inv, Wd.cpow);
-        // q must fit words_out words (range check of assign_integer(q, 2*enc_bits), SURVEY.md A.4): canonical q digits are in T
-        {
-            const int* Qf = (const int*)S.T + C::L * 32;
-            const int qbits = 64 * wo;
-            int bad = 0;
-#pragma unroll
-            for (int k = 0; k < C::BL; k++) {
-                const int p = role * C::BL + k;
-                const unsigned d = (unsigned)Qf[p * 32 + lane];
-                const int lo = W * p;
-                if (lo >= qbits) bad |= d != 0;
-                else if (lo + W > qbits) bad |= (d >> (qbits - lo)) != 0;
-            }
-            if (bad && active) atomicOr(flags, 1);
-        }
+        if (q_too_wide<C>(S, wo, role, lane) && active) atomicOr(flags, 1);
         __syncthreads();
     }
-    w_end<C, WENG>(S);
+    cta_end(S);
 }
 
 // ---- running-tally trace (pb200_tally_trace, DESIGN.md §9c) --------------------------------------------------------------------
@@ -1238,11 +1146,9 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_trace_redu
     extern __shared__ int4 smem[];
     typename View<C, ENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    cta_begin<C, ENG>(S, smem, K);
+    cta_begin(S, smem, K);
     const size_t units = (n + s - 1) / s * chains;
-    size_t u = (size_t)blockIdx.x * 32 + lane;
-    const bool active = u < units;
-    if (!active) u = units - 1;
+    const auto [u, active] = lane_unit(units, lane);
     const size_t b = u / chains, j = u - b * chains;
     for (size_t t = 0; t < s; t++) {
         const size_t i = b * s + t;
@@ -1257,7 +1163,7 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_trace_redu
         }
     }
     if (active) scatter_entry<C>(totals + u * C::ENTRY4, S.V, role, lane);
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 // Exclusive prefix products of one level, in place: entry (b s + t, j) <- carry(b, j) * the entries before it in its chunk.  The carry
@@ -1269,11 +1175,9 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_trace_appl
     extern __shared__ int4 smem[];
     typename View<C, ENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    cta_begin<C, ENG>(S, smem, K);
+    cta_begin(S, smem, K);
     const size_t units = (n + s - 1) / s * chains;
-    size_t u = (size_t)blockIdx.x * 32 + lane;
-    const bool active = u < units;
-    if (!active) u = units - 1;
+    const auto [u, active] = lane_unit(units, lane);
     const size_t b = u / chains, j = u - b * chains;
     if (carry) gather_entry<C>(S.V, carry + u * C::ENTRY4, role, lane);
     else load_value<C>(S.V, init + j * K.words_out, K.words_out, role, lane);
@@ -1285,7 +1189,7 @@ __global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_trace_appl
         if (real) scatter_entry<C>(e, S.V, role, lane);
         if (t + 1 < s) mm<C, false, ENG>(S, S.B, role, lane);                            // the chunk's own product is not needed
     }
-    cta_end<C, ENG>(S);
+    cta_end(S);
 }
 
 // The exact chain of every leaf chunk on the witness engine: a <- carry-in (init_j for chunk 0, as given; else carry[u], canonical),
@@ -1299,19 +1203,17 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_trace_w(
     extern __shared__ int4 smem[];
     typename WView<C, WENG>::type S(smem);
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    w_begin<C, WENG>(S, smem, K);
+    cta_begin(S, smem, K);
     const int wo = K.words_out;
     const size_t units = (count + s - 1) / s * chains;
-    size_t u = (size_t)blockIdx.x * 32 + lane;
-    const bool active = u < units;
-    if (!active) u = units - 1;
+    const auto [u, active] = lane_unit(units, lane);
     const size_t b = u / chains, j = u - b * chains;
-    load_value_shl<C>(S.V, b ? carry + u * wo : init + j * wo, wo, Wd.sh >> 1, role, lane);
+    load_value<C>(S.V, b ? carry + u * wo : init + j * wo, wo, role, lane, Wd.sh >> 1);
     for (size_t t = 0; t < s; t++) {
         const size_t i = b * s + t;
         const bool real = active && i < count;
         const size_t e = (i < count ? i : count - 1) * chains + j;
-        load_value_shl<C>(S.B, c + e * wo, wo, Wd.sh >> 1, role, lane);
+        load_value<C>(S.B, c + e * wo, wo, role, lane, Wd.sh >> 1);
         if (!real) {
 #pragma unroll
             for (int ch = 0; ch < C::CH; ch++) S.B[(role * C::CH + ch) * 32 + lane] = __ldg(Wd.one_s + role * C::CH + ch);
@@ -1320,23 +1222,10 @@ __global__ void __launch_bounds__(C::THREADS, WView<C, WENG>::PER_SM) k_trace_w(
         WStep o; o.rec = nullptr; o.rem_out = real ? acc + e * wo : nullptr;
         o.q_out = (real && q_out) ? q_out + e * wo : nullptr;
         wmm<C, WENG>(smem, S, S.B, 0, S.V, o, Wd.sh, wo, Wd.inv, Wd.cpow);
-        {   // q must fit words_out words (the check of k_add_w)
-            const int* Qf = (const int*)S.T + C::L * 32;
-            const int qbits = 64 * wo;
-            int bad = 0;
-#pragma unroll
-            for (int k = 0; k < C::BL; k++) {
-                const int p = role * C::BL + k;
-                const unsigned d = (unsigned)Qf[p * 32 + lane];
-                const int lo = W * p;
-                if (lo >= qbits) bad |= d != 0;
-                else if (lo + W > qbits) bad |= (d >> (qbits - lo)) != 0;
-            }
-            if (bad && real) atomicOr(flags, 1);
-        }
+        if (q_too_wide<C>(S, wo, role, lane) && real) atomicOr(flags, 1);
         __syncthreads();
     }
-    w_end<C, WENG>(S);
+    cta_end(S);
 }
 
 // ---- host side ---------------------------------------------------------------------------------
@@ -1431,6 +1320,53 @@ static int window_schedule(const BigInt& e, std::vector<int2>& ops) {
 
 static size_t cdiv(size_t a, size_t b) { return (a + b - 1) / b; }
 
+// *d <- a device copy of a host array, which must live until st is synchronised; an empty array still gets an address
+template <class T, class E>
+static cudaError_t upload(T** d, const std::vector<E>& h, cudaStream_t st) {
+    const size_t bytes = h.size() * sizeof(E);
+    CUW(cudaMalloc(d, bytes ? bytes : sizeof(E)));
+    return bytes ? cudaMemcpyAsync(*d, h.data(), bytes, cudaMemcpyHostToDevice, st) : cudaSuccess;
+}
+// *E <- the sliding-window schedule of the exponent e, its steps uploaded to *d_ops (ops: the host copy, kept by the caller until st
+// is synchronised)
+static cudaError_t upload_schedule(const BigInt& e, std::vector<int2>& ops, int2** d_ops, PowSched* E, cudaStream_t st) {
+    ops.clear();
+    const int first_idx = window_schedule(e, ops);
+    CUW(upload(d_ops, ops, st));
+    *E = PowSched{*d_ops, (int)ops.size(), first_idx};
+    return cudaSuccess;
+}
+
+// Per-key constants of a modulus Nt: mu = floor(2^(2 BETA) / Nt) and Nt as entries, and the constant block load_consts copies into
+// shared memory: mu, Nt, `third` (an entry: 2^sh for the value engine, the unsigned digits of Nt for the witness engine), then the
+// reversed s8 tables of mu and Nt
+template <class C>
+struct KeyConsts {
+    std::vector<int> mu, nt, block;
+    KeyConsts(const BigInt& Nt, const std::vector<int>& third) {
+        to_entry<C>(BigInt::div(BigInt::pow2(2 * (size_t)C::BETA), Nt), mu);
+        to_entry<C>(Nt, nt);
+        std::vector<int> r_mu, r_nt;
+        to_rtab<C>(mu, r_mu); to_rtab<C>(nt, r_nt);
+        auto put = [&](const std::vector<int>& v) { block.insert(block.end(), v.begin(), v.end()); };
+        put(mu); put(nt); put(third); put(r_mu); put(r_nt);
+    }
+};
+// *d <- block28u's per-key shared-memory image for the layout UL<C, LG, WIT> (from OFF_CONST on): the first three constants of the
+// block, then the Toeplitz core-matrix tables of mu and Nt.  Synchronises st (the image is a local).
+template <class C, int LG, bool WIT = false>
+static cudaError_t upload_u_image(int4** d, const KeyConsts<C>& k, cudaStream_t st) {
+    typedef UL<C, LG, WIT> U;
+    std::vector<signed char> img(U::KEY_BYTES, 0), k7;
+    memcpy(img.data(), k.block.data(), 3 * C::ENTRY4 * 16);
+    to_k7<C>(k.mu, k7);
+    umma_cm_table<C, LG>(k7.data(), true, img.data() + (U::OFF_CMH - U::OFF_CONST));
+    to_k7<C>(k.nt, k7);
+    umma_cm_table<C, LG>(k7.data(), false, img.data() + (U::OFF_CML - U::OFF_CONST));
+    CUW(upload(d, img, st));
+    return cudaStreamSynchronize(st);
+}
+
 // The engine kernels need more dynamic shared memory than the default limit; the attribute is per device, so it is set on the
 // device of every launch (and before an occupancy query, which counts against the current limit).
 template <class V, class... P>
@@ -1472,73 +1408,43 @@ static Block28Key* create_cfg(const BigInt& n, const BigInt& g, uint32_t n_bits,
     BigInt n2 = BigInt::mul(n, n);
     int sh = C::KN - (int)n2.bits();
     BigInt Nt = BigInt::shl(n2, sh);
-    BigInt mu = BigInt::div(BigInt::pow2(2 * (size_t)C::BETA), Nt);
-    BigInt two_sh = BigInt::pow2(sh);
-    std::vector<int> e_mu, e_nt, e_sh, all;
-    to_entry<C>(mu, e_mu); to_entry<C>(Nt, e_nt); to_entry<C>(two_sh, e_sh);
-    all.insert(all.end(), e_mu.begin(), e_mu.end());
-    all.insert(all.end(), e_nt.begin(), e_nt.end());
-    all.insert(all.end(), e_sh.begin(), e_sh.end());
-    std::vector<int> r_mu, r_nt;
-    to_rtab<C>(e_mu, r_mu); to_rtab<C>(e_nt, r_nt);
-    all.insert(all.end(), r_mu.begin(), r_mu.end());
-    all.insert(all.end(), r_nt.begin(), r_nt.end());
-    CUK(cudaMalloc(&key->d_consts, all.size() * sizeof(int)));
-    CUK(cudaMemcpyAsync(key->d_consts, all.data(), all.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-    // block28u: the same constants followed by the two Toeplitz core-matrix tables (image of shared memory from OFF_CONST on), for
-    // one and for two lane groups per CTA
-    auto u_image = [&](auto LGC, int4** d_out) -> cudaError_t {
-        constexpr int LG = decltype(LGC)::value;
-        typedef UL<C, LG> U;
-        std::vector<signed char> img(U::KEY_BYTES, 0);
-        memcpy(img.data(), all.data(), 3 * C::ENTRY4 * 16);
-        std::vector<signed char> k7(C::K7);
-        to_k7<C>(e_mu, k7);
-        umma_cm_table<C, LG>(k7.data(), true, img.data() + (U::OFF_CMH - U::OFF_CONST));
-        to_k7<C>(e_nt, k7);
-        umma_cm_table<C, LG>(k7.data(), false, img.data() + (U::OFF_CML - U::OFF_CONST));
-        cudaError_t e = cudaMalloc(d_out, img.size());
-        if (e != cudaSuccess) return e;
-        e = cudaMemcpyAsync(*d_out, img.data(), img.size(), cudaMemcpyHostToDevice, st);
-        if (e != cudaSuccess) return e;
-        return cudaStreamSynchronize(st);
-    };
+    std::vector<int> e_sh;
+    to_entry<C>(BigInt::pow2(sh), e_sh);
+    const KeyConsts<C> kc(Nt, e_sh);
+    CUK(upload(&key->d_consts, kc.block, st));
+    // block28u: the same constants followed by the two Toeplitz core-matrix tables, for one and for two lane groups per CTA
     if constexpr (UL<C, 1>::SUPPORTED) {
-        CUK(u_image(std::integral_constant<int, 1>{}, &key->d_uconsts));
+        CUK((upload_u_image<C, 1>(&key->d_uconsts, kc, st)));
         key->has_u = true;
     }
     if constexpr (UL<C, 1>::SUPPORTED && UL<C, 2>::SUPPORTED) {
-        CUK(u_image(std::integral_constant<int, 2>{}, &key->d_uconsts2));
+        CUK((upload_u_image<C, 2>(&key->d_uconsts2, kc, st)));
         key->has_u2 = true;
     }
     block28_set_engine(key, -1);
     // sliding-window schedule for the exponent n
     std::vector<int2> ops;
-    int first_idx = window_schedule(n, ops);
+    CUK(upload_schedule(n, ops, &key->d_ops, &key->dev.rn, st));
     int comb_bits = n_bits >= 1024 ? 12 : 8;
     if (const char* e = getenv("PB200_COMB_BITS")) { int v = atoi(e); if (v >= 4 && v <= 16) comb_bits = v; }
     const int n_windows = (int)((n_bits + comb_bits - 1) / comb_bits);
     const bool g_std = g == BigInt::add(n, BigInt(1)) && !getenv("PB200_NO_GSTD");
     key->n_sqr = 1; key->n_mul = (TABN - 1) + (g_std ? 1 : (uint64_t)(n_windows - 1)) + 1;   // r^2; table; comb (or m*n); gm*rn
     for (auto& o : ops) { key->n_sqr += (uint64_t)o.x; if (o.y >= 0) key->n_mul += 1; }
-    CUK(cudaMalloc(&key->d_ops, (ops.size() + 1) * sizeof(int2)));
-    if (!ops.empty()) CUK(cudaMemcpyAsync(key->d_ops, ops.data(), ops.size() * sizeof(int2), cudaMemcpyHostToDevice, st));
     uint32_t win = (n_bits + 63) / 64;
     std::vector<u64> gw(win);
     g.to_u64_le(gw.data(), win);
-    CUK(cudaMalloc(&key->d_gwords, win * sizeof(u64)));
-    CUK(cudaMemcpyAsync(key->d_gwords, gw.data(), win * sizeof(u64), cudaMemcpyHostToDevice, st));
+    CUK(upload(&key->d_gwords, gw, st));
     if (!g_std) CUK(cudaMalloc(&key->d_tg, ((size_t)n_windows << comb_bits) * C::ENTRY4 * sizeof(int4)));
     if (g_std) {
         std::vector<int> e_n;
         to_entry<C>(n, e_n);
-        CUK(cudaMalloc(&key->d_nentry, e_n.size() * sizeof(int)));
-        CUK(cudaMemcpyAsync(key->d_nentry, e_n.data(), e_n.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+        CUK(upload(&key->d_nentry, e_n, st));
         CUK(cudaStreamSynchronize(st));
     }
     B28Dev& K = key->dev;
     K.n_entry = key->d_nentry;
-    K.consts = key->d_consts; K.uconsts = key->d_uconsts; K.uconsts2 = key->d_uconsts2; K.ops = key->d_ops; K.n_ops = (int)ops.size(); K.first_idx = first_idx;
+    K.consts = key->d_consts; K.uconsts = key->d_uconsts; K.uconsts2 = key->d_uconsts2;
     K.tg = key->d_tg; K.n_windows = n_windows; K.comb_bits = comb_bits; K.words_in = (int)win; K.words_out = (int)((2 * n_bits + 63) / 64);
     K.sh = sh;
     K.sms = (unsigned)key->sms;
@@ -1608,14 +1514,13 @@ static cudaError_t pow_cfg(Block28Key* key, const u64* d_base, int base_words, s
     });
 }
 
-// window width of the scalar chain for k_bits-bit scalars: the w <= SCALAR_MAXW with the fewest multiplications,
-// (2^w - 2) for the table + (ceil(k_bits / w) - 1) * (w + 1) for the chain (5 at 2048 bits, 3 at 32)
+// multiplications of k_scalar's table and chain for k_bits-bit scalars with a w-bit window:
+// (2^w - 2) for the table + (ceil(k_bits / w) - 1) * (w + 1) for the chain
+static uint64_t scalar_cost(uint32_t k_bits, int w) { return ((1u << w) - 2) + ((k_bits + w - 1) / w - 1) * (uint64_t)(w + 1); }
+// window width of the scalar chain for k_bits-bit scalars: the w <= SCALAR_MAXW with the fewest multiplications (5 at 2048 bits, 3 at 32)
 static int scalar_window(uint32_t k_bits) {
-    int best = 1; uint64_t best_cost = ~0ull;
-    for (int w = 1; w <= SCALAR_MAXW; w++) {
-        const uint64_t cost = ((1u << w) - 2) + ((k_bits + w - 1) / w - 1) * (uint64_t)(w + 1);
-        if (cost < best_cost) { best = w; best_cost = cost; }
-    }
+    int best = 1;
+    for (int w = 2; w <= SCALAR_MAXW; w++) if (scalar_cost(k_bits, w) < scalar_cost(k_bits, best)) best = w;
     return best;
 }
 
@@ -1663,30 +1568,19 @@ static cudaError_t witness_prepare_cfg(Block28Key* key, u64* d_gchain, bool gcha
     int sh = C::KN - (int)n2.bits();
     if (sh & 1) sh -= 1;                                   // chain values carry 2^(sh/2)
     BigInt Nt = BigInt::shl(n2, sh);
-    BigInt mu = BigInt::div(BigInt::pow2(2 * (size_t)C::BETA), Nt);
-    std::vector<int> e_mu, e_nt, e_ntu(C::ENTRY4 * 4, 0), e_one, all;
-    to_entry<C>(mu, e_mu); to_entry<C>(Nt, e_nt); to_entry<C>(BigInt::pow2(sh / 2), e_one);
+    std::vector<int> e_ntu(C::ENTRY4 * 4, 0), e_one;
+    to_entry<C>(BigInt::pow2(sh / 2), e_one);
     for (int p = 0; p < C::L; p++) e_ntu[(p / C::BL) * C::CH * 4 + (p % C::BL)] = (int)Nt.bits_at((size_t)W * p, W);
-    all.insert(all.end(), e_mu.begin(), e_mu.end());
-    all.insert(all.end(), e_nt.begin(), e_nt.end());
-    all.insert(all.end(), e_ntu.begin(), e_ntu.end());     // in the slot the value engine uses for 2^sh
-    std::vector<int> r_mu, r_nt;
-    to_rtab<C>(e_mu, r_mu); to_rtab<C>(e_nt, r_nt);
-    all.insert(all.end(), r_mu.begin(), r_mu.end());
-    all.insert(all.end(), r_nt.begin(), r_nt.end());
-    CUW(cudaMalloc(&key->d_wconsts, all.size() * sizeof(int)));
-    CUW(cudaMemcpyAsync(key->d_wconsts, all.data(), all.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-    CUW(cudaMalloc(&key->d_one_s, e_one.size() * sizeof(int)));
-    CUW(cudaMemcpyAsync(key->d_one_s, e_one.data(), e_one.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    const KeyConsts<C> kc(Nt, e_ntu);                      // the unsigned digits of Nt in the slot the value engine uses for 2^sh
+    CUW(upload(&key->d_wconsts, kc.block, st));
+    CUW(upload(&key->d_one_s, e_one, st));
     const int wo = key->dev.words_out, wi = key->dev.words_in;
     std::vector<u64> cpow(2 * (size_t)wo);
     { u64 c = PB200_DIGEST_C; for (size_t j = 0; j < cpow.size(); j++) { cpow[j] = c; c *= PB200_DIGEST_C; } }
-    CUW(cudaMalloc(&key->d_cpow, cpow.size() * sizeof(u64)));
-    CUW(cudaMemcpyAsync(key->d_cpow, cpow.data(), cpow.size() * sizeof(u64), cudaMemcpyHostToDevice, st));
+    CUW(upload(&key->d_cpow, cpow, st));
     std::vector<u64> nw(wi);
     n.to_u64_le(nw.data(), wi);
-    CUW(cudaMalloc(&key->d_nwords, nw.size() * sizeof(u64)));
-    CUW(cudaMemcpyAsync(key->d_nwords, nw.data(), nw.size() * sizeof(u64), cudaMemcpyHostToDevice, st));
+    CUW(upload(&key->d_nwords, nw, st));
     CUW(cudaMalloc(&key->d_gtab, (size_t)key->n_bits * C::ENTRY4 * sizeof(int4)));
     // 2^(28(L-2)) / Nt_w from the top 52 bits of Nt_w
     BigInt top = BigInt::shr(Nt, (size_t)W * (C::L - 2) - 20);
@@ -1697,17 +1591,7 @@ static cudaError_t witness_prepare_cfg(Block28Key* key, u64* d_gchain, bool gcha
     Wd.exp_bits = (int)n.bits(); Wd.sh = sh; Wd.inv = 1048576.0 / topd;
     if constexpr (UL<C, 1, true>::SUPPORTED) {
         // the same step on the tcgen05 phases: constants of the witness modulus + their Toeplitz core-matrix tables
-        typedef UL<C, 1, true> U;
-        std::vector<signed char> img(U::KEY_BYTES, 0);
-        memcpy(img.data(), all.data(), 3 * C::ENTRY4 * 16);
-        std::vector<signed char> k7(C::K7);
-        to_k7<C>(e_mu, k7);
-        umma_cm_table<C, 1>(k7.data(), true, img.data() + (U::OFF_CMH - U::OFF_CONST));
-        to_k7<C>(e_nt, k7);
-        umma_cm_table<C, 1>(k7.data(), false, img.data() + (U::OFF_CML - U::OFF_CONST));
-        CUW(cudaMalloc(&key->d_wuconsts, img.size()));
-        CUW(cudaMemcpyAsync(key->d_wuconsts, img.data(), img.size(), cudaMemcpyHostToDevice, st));
-        CUW(cudaStreamSynchronize(st));
+        CUW((upload_u_image<C, 1, true>(&key->d_wuconsts, kc, st)));
         key->wdev.uconsts = key->d_wuconsts;
         key->has_wu = !getenv("PB200_NO_UMMA_WITNESS");
     }
@@ -1839,12 +1723,9 @@ cudaError_t block28_encrypt(Block28Key* key, const u64* d_m, const u64* d_r, siz
 }
 cudaError_t block28_pow_prepare(Block28Key* key, const BigInt& e, cudaStream_t st) {
     std::vector<int2> ops;
-    const int first_idx = window_schedule(e, ops);
     if (key->d_pow_ops) { cudaFree(key->d_pow_ops); key->d_pow_ops = nullptr; }
-    CUW(cudaMalloc(&key->d_pow_ops, (ops.size() + 1) * sizeof(int2)));
-    if (!ops.empty()) CUW(cudaMemcpyAsync(key->d_pow_ops, ops.data(), ops.size() * sizeof(int2), cudaMemcpyHostToDevice, st));
+    CUW(upload_schedule(e, ops, &key->d_pow_ops, &key->pow, st));
     CUW(cudaStreamSynchronize(st));
-    key->pow.ops = key->d_pow_ops; key->pow.n_ops = (int)ops.size(); key->pow.first_idx = first_idx;
     key->pow_ready = true;
     return cudaSuccess;
 }
@@ -2039,10 +1920,7 @@ cudaError_t block28_trace_chain(Block28Key* key, const u64* d_init, const u64* d
 
 // ---- matvec: planner and driver (DESIGN.md §9b) ---------------------------------------------------------------------------------
 // multiplications of k_scalar's chain for k_bits-bit scalars (table, windows, finalize)
-static uint64_t scalar_chain(uint32_t k_bits) {
-    const int w = scalar_window(k_bits);
-    return ((1u << w) - 2) + ((k_bits + w - 1) / w - 1) * (uint64_t)(w + 1) + 1;
-}
+static uint64_t scalar_chain(uint32_t k_bits) { return scalar_cost(k_bits, scalar_window(k_bits)) + 1; }
 // slice length of a k_bucket_fold launch over n entries: one wave of lanes, at least 8 entries (the carry list shrinks 4x per level)
 static int fold_ls(size_t n, size_t lanes) { const size_t l = cdiv(n, lanes); return (int)(l < 8 ? 8 : l); }
 // mulmods (upper bound) and sequential chain of the fold of n entries, every carry level included
