@@ -41,8 +41,9 @@ typedef enum pb200_status {
     PB200_OK = 0,
     PB200_ERR_INVALID_ARG = -1,   /* null pointer, zero sizes, n_bits % limb_bits != 0 (assign_integer's assert) */
     PB200_ERR_ZERO_MODULUS = -2,  /* n == 0: num-bigint modpow / % panic (src/paillier.rs:89-91,96) */
-    PB200_ERR_EVEN_MODULUS = -3,  /* reserved (never returned): even n is accepted, as in the reference, whose tests draw
-                                     n = rng.gen_biguint(bits) (src/paillier.rs:173,251) */
+    PB200_ERR_EVEN_MODULUS = -3,  /* only from pb200_inverse_batch*, pb200_sub_batch* and pb200_scalar_mul_signed_batch* with signs
+                                     (their algorithm needs an odd n); every other entry point accepts an even n, as the reference
+                                     does, whose tests draw n = rng.gen_biguint(bits) (src/paillier.rs:173,251) */
     PB200_ERR_RANGE = -4,         /* an input does not fit its declared bit width (range check would fail) */
     PB200_ERR_UNSUPPORTED = -5,   /* key size larger than the largest compiled engine */
     PB200_ERR_CUDA = -6,          /* CUDA runtime failure; pb200_last_cuda_error() has the text */
@@ -50,7 +51,8 @@ typedef enum pb200_status {
     PB200_ERR_SINK = -8,          /* the witness sink callback returned non-zero */
     PB200_ERR_CONSTRAINT = -9,    /* a supplied (q, rem) does not satisfy a*b = q*n^2 + rem (mul_mod's equality would fail) */
     PB200_ERR_PEER = -10,         /* multi-GPU tally: a peer's partial did not arrive within the kernel's time-out */
-    PB200_ERR_DECRYPT = -11       /* c^lambda mod n^2 is not 1 modulo n: not a valid ciphertext for this key */
+    PB200_ERR_DECRYPT = -11,      /* c^lambda mod n^2 is not 1 modulo n: not a valid ciphertext for this key */
+    PB200_ERR_NOT_INVERTIBLE = -12 /* gcd(c mod n^2, n) != 1: the value has no inverse mod n^2 (0, n, a multiple of p or q) */
 } pb200_status;
 
 /* bits of the per-key device flag word (pb200_key_take_flags) */
@@ -58,6 +60,7 @@ typedef enum pb200_status {
 #define PB200_FLAG_CONSTRAINT 2u  /* -> PB200_ERR_CONSTRAINT */
 #define PB200_FLAG_PEER_TIMEOUT 4u /* a peer GPU's tally partial did not arrive (pb200_tally_peer_dev / pb200_tally_multi) */
 #define PB200_FLAG_DECRYPT 8u     /* -> PB200_ERR_DECRYPT */
+#define PB200_FLAG_NOT_INVERTIBLE 16u /* -> PB200_ERR_NOT_INVERTIBLE */
 
 typedef struct pb200_key pb200_key;
 
@@ -237,6 +240,34 @@ int pb200_scalar_mul_batch_dev(pb200_key* key, const uint64_t* d_c_le, const uin
 int pb200_tally_weighted(pb200_key* key, const uint64_t* c_le, const uint64_t* k_le, uint32_t k_bits, size_t count, uint64_t* out_le);
 int pb200_tally_weighted_dev(pb200_key* key, const uint64_t* d_c_le, const uint64_t* d_k_le, uint32_t k_bits, size_t count,
                              uint64_t* d_out_le);
+
+/* ---- ciphertext inverse, homomorphic subtraction and signed scalars -----------------------------------------------------
+ * c^-1 mod n^2 encrypts -Dec(c), so negation, subtraction and negative scalars cost one inversion instead of a full-width exponent
+ * n - 1.  The inverse is a per-ciphertext Bernstein-Yang safegcd mod n (a fixed number of batches of 62 divsteps, so no warp diverges
+ * on data) followed by one Hensel step to n^2, one thread per ciphertext, on every engine; it needs no private part.
+ *
+ *   pb200_inverse_batch:            out_i = c_i^-1 mod n^2                      Dec(out_i) = -Dec(c_i) mod n
+ *   pb200_sub_batch:                out_i = c1_i * c2_i^-1 mod n^2              Dec(out_i) = Dec(c1_i) - Dec(c2_i) mod n
+ *   pb200_scalar_mul_signed_batch:  out_i = c_i^(k_i) mod n^2, k_i = (k_neg[i] ? -1 : +1) * mag_i, c^-s = (c^-1)^s
+ *                                                                               Dec(out_i) = k_i * Dec(c_i) mod n
+ * c, c1, c2: count * words_out words, any value (reduced mod n^2); out: count * words_out words, canonical.  k_mag: count *
+ * PB200_WORDS(k_bits) words, 1 <= k_bits <= n_bits; k_neg: nullable, one byte per unit, non-zero = negative.  k_neg == NULL gives
+ * exactly pb200_scalar_mul_batch; a negative sign with magnitude 0 is k = 0 (output 1, no error, even for c = 0).  The scalars are
+ * not reduced mod n: the output is c^k mod n^2 exactly.
+ * A unit whose inverse does not exist (gcd(c mod n^2, n) != 1; for sub the c2 operand) gets 0; the others are still computed.  The host
+ * variants copy every output back and then return PB200_ERR_NOT_INVERTIBLE; _dev raises PB200_FLAG_NOT_INVERTIBLE in the flag word.
+ * PB200_ERR_EVEN_MODULUS for an even n (pb200_scalar_mul_signed_batch* only when k_neg is non-null).  PB200_ERR_INVALID_ARG for null
+ * pointers where data is needed, k_bits == 0 or k_bits > n_bits; PB200_ERR_RANGE (host variant) when a magnitude has a bit at or above
+ * k_bits.  count == 0 does nothing.  The first call prepares the per-key constants on the device (synchronises once).
+ * _dev: device pointers on the key's device, enqueued on the key's stream, no final synchronise, magnitudes are not range-checked. */
+int pb200_inverse_batch(pb200_key* key, const uint64_t* c_le, size_t count, uint64_t* out_le);
+int pb200_inverse_batch_dev(pb200_key* key, const uint64_t* d_c_le, size_t count, uint64_t* d_out_le);
+int pb200_sub_batch(pb200_key* key, const uint64_t* c1_le, const uint64_t* c2_le, size_t count, uint64_t* out_le);
+int pb200_sub_batch_dev(pb200_key* key, const uint64_t* d_c1_le, const uint64_t* d_c2_le, size_t count, uint64_t* d_out_le);
+int pb200_scalar_mul_signed_batch(pb200_key* key, const uint64_t* c_le, const uint64_t* k_mag_le, const uint8_t* k_neg, uint32_t k_bits,
+                                  size_t count, uint64_t* out_le);
+int pb200_scalar_mul_signed_batch_dev(pb200_key* key, const uint64_t* d_c_le, const uint64_t* d_k_mag_le, const uint8_t* d_k_neg,
+                                      uint32_t k_bits, size_t count, uint64_t* d_out_le);
 
 /* ---- encrypted matrix-vector product with a signed plaintext matrix ------------------------------------------------------
  * Enc(W m) from Enc(m): private scoring with a linear model, multi-question ballots, PIR-style selection.  On a block28 engine a

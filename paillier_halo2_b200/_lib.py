@@ -23,7 +23,8 @@ PB200_ERR_SINK = -8
 PB200_ERR_CONSTRAINT = -9
 PB200_ERR_PEER = -10
 PB200_ERR_DECRYPT = -11
-PB200_FLAG_RANGE, PB200_FLAG_CONSTRAINT, PB200_FLAG_PEER_TIMEOUT, PB200_FLAG_DECRYPT = 1, 2, 4, 8
+PB200_ERR_NOT_INVERTIBLE = -12
+PB200_FLAG_RANGE, PB200_FLAG_CONSTRAINT, PB200_FLAG_PEER_TIMEOUT, PB200_FLAG_DECRYPT, PB200_FLAG_NOT_INVERTIBLE = 1, 2, 4, 8, 16
 
 u64p = C.POINTER(C.c_uint64)
 u32p = C.POINTER(C.c_uint32)
@@ -86,6 +87,12 @@ SYMBOLS = {
     "pb200_scalar_mul_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
     "pb200_tally_weighted": (C.c_int, [C.c_void_p, u64p, u64p, C.c_uint32, C.c_size_t, u64p]),
     "pb200_tally_weighted_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
+    "pb200_inverse_batch": (C.c_int, [C.c_void_p, u64p, C.c_size_t, u64p]),
+    "pb200_inverse_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "pb200_sub_batch": (C.c_int, [C.c_void_p, u64p, u64p, C.c_size_t, u64p]),
+    "pb200_sub_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "pb200_scalar_mul_signed_batch": (C.c_int, [C.c_void_p, u64p, u64p, C.c_void_p, C.c_uint32, C.c_size_t, u64p]),
+    "pb200_scalar_mul_signed_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
     "pb200_matvec": (C.c_int, [C.c_void_p, u64p, C.c_size_t, u64p, C.c_void_p, C.c_uint32, C.c_size_t, u64p]),
     "pb200_matvec_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
     "pb200_matvec_plan": (C.c_int, [C.c_uint32, C.c_int, C.c_size_t, C.c_size_t, C.c_uint32, C.c_int, u64p]),

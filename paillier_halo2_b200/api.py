@@ -445,6 +445,78 @@ class PaillierKey(CellMixin):
         """Device-pointer variant (pb200_tally_weighted_dev): enqueues on the key's stream, no synchronise, no range check."""
         check(self._lib.pb200_tally_weighted_dev(self._h, d_c, d_k, k_bits, count, d_out), "pb200_tally_weighted_dev")
 
+    # -- inverse mod n^2: Dec(c^-1) = -Dec(c), Dec(c1 c2^-1) = Dec(c1) - Dec(c2), c^-s = (c^-1)^s ----------------------------------
+    def invert_words(self, c_w: np.ndarray) -> np.ndarray:
+        """c_w: (count, words_out) any values -> (count, words_out) c^-1 mod n^2 (pb200_inverse_batch); a unit without an inverse gets 0
+        and the call raises PB200_ERR_NOT_INVERTIBLE (Pb200Error.outputs holds the outputs)."""
+        c_w = np.ascontiguousarray(c_w, dtype="<u8").reshape(-1, self.words_out)
+        out = np.empty_like(c_w)
+        _check_out(self._lib.pb200_inverse_batch(self._h, _p(c_w), c_w.shape[0], _p(out)), "pb200_inverse_batch", out)
+        return out
+
+    def invert_dev(self, d_c: int, count: int, d_out: int) -> None:
+        """Device-pointer variant (pb200_inverse_batch_dev): enqueues on the key's stream, no synchronise; a unit without an inverse
+        raises PB200_FLAG_NOT_INVERTIBLE in the flag word (take_flags)."""
+        check(self._lib.pb200_inverse_batch_dev(self._h, d_c, count, d_out), "pb200_inverse_batch_dev")
+
+    def invert(self, cs: Sequence[int]) -> List[int]:
+        """c^-1 mod n^2 for every ciphertext: the ciphertext of -m mod n."""
+        return words_to_ints(self.invert_words(self._ciphertexts(cs, "invert"))) if len(cs) else []
+
+    def sub_words(self, c1_w: np.ndarray, c2_w: np.ndarray) -> np.ndarray:
+        """(count, words_out) each, any values -> c1 * c2^-1 mod n^2 (pb200_sub_batch); PB200_ERR_NOT_INVERTIBLE as invert_words."""
+        c1_w = np.ascontiguousarray(c1_w, dtype="<u8").reshape(-1, self.words_out)
+        c2_w = np.ascontiguousarray(c2_w, dtype="<u8").reshape(-1, self.words_out)
+        assert c1_w.shape == c2_w.shape
+        out = np.empty_like(c1_w)
+        _check_out(self._lib.pb200_sub_batch(self._h, _p(c1_w), _p(c2_w), c1_w.shape[0], _p(out)), "pb200_sub_batch", out)
+        return out
+
+    def sub_dev(self, d_c1: int, d_c2: int, count: int, d_out: int) -> None:
+        """Device-pointer variant (pb200_sub_batch_dev): enqueues on the key's stream, no synchronise."""
+        check(self._lib.pb200_sub_batch_dev(self._h, d_c1, d_c2, count, d_out), "pb200_sub_batch_dev")
+
+    def sub(self, c1s: Sequence[int], c2s: Sequence[int]) -> List[int]:
+        """c1 * c2^-1 mod n^2 for every pair: the ciphertext of m1 - m2 mod n."""
+        assert len(c1s) == len(c2s)
+        if not len(c1s):
+            return []
+        return words_to_ints(self.sub_words(self._ciphertexts(c1s, "sub"), self._ciphertexts(c2s, "sub")))
+
+    def scalar_mul_signed_words(self, c_w: np.ndarray, mag_w: np.ndarray, neg: Optional[np.ndarray], k_bits: int) -> np.ndarray:
+        """c_w: (count, words_out) any values; mag_w: (count, words(k_bits)) magnitudes below 2^k_bits; neg: None or (count,) non-zero
+        where the scalar is negative -> (count, words_out) c^k mod n^2 (pb200_scalar_mul_signed_batch)."""
+        c_w = np.ascontiguousarray(c_w, dtype="<u8").reshape(-1, self.words_out)
+        mag_w = np.ascontiguousarray(mag_w, dtype="<u8").reshape(-1, words(k_bits))
+        count = c_w.shape[0]
+        assert mag_w.shape[0] == count
+        if neg is not None:
+            neg = np.ascontiguousarray(neg, dtype=np.uint8)
+            assert neg.size == count
+        out = np.empty((count, self.words_out), dtype="<u8")
+        _check_out(self._lib.pb200_scalar_mul_signed_batch(self._h, _p(c_w), _p(mag_w), neg.ctypes.data_as(C.c_void_p) if neg is not None else None,
+                                                           k_bits, count, _p(out)), "pb200_scalar_mul_signed_batch", out)
+        return out
+
+    def scalar_mul_signed_dev(self, d_c: int, d_mag: int, d_neg: Optional[int], k_bits: int, count: int, d_out: int) -> None:
+        """Device-pointer variant (pb200_scalar_mul_signed_batch_dev): enqueues on the key's stream, no synchronise, no range check."""
+        check(self._lib.pb200_scalar_mul_signed_batch_dev(self._h, d_c, d_mag, d_neg or None, k_bits, count, d_out),
+              "pb200_scalar_mul_signed_batch_dev")
+
+    def scalar_mul_signed(self, cs: Sequence[int], ks: Sequence[int]) -> List[int]:
+        """c_i^(k_i) mod n^2 exactly, for scalars of any sign with |k_i| < 2^enc_bits (not reduced mod n; c^-s = (c^-1)^s): the
+        ciphertext of k_i * m_i mod n."""
+        assert len(cs) == len(ks)
+        if not len(cs):
+            return []
+        ks = [int(k) for k in ks]
+        k_bits = max([1] + [abs(k).bit_length() for k in ks])
+        if k_bits > self.enc_bits:
+            raise Pb200Error(_lib.PB200_ERR_RANGE, "scalar_mul_signed")
+        neg = np.array([k < 0 for k in ks], dtype=np.uint8)
+        mag_w = ints_to_words([abs(k) for k in ks], words(k_bits))
+        return words_to_ints(self.scalar_mul_signed_words(self._ciphertexts(cs, "scalar_mul_signed"), mag_w, neg if neg.any() else None, k_bits))
+
     # -- encrypted matrix-vector product: row r of the result encrypts sum_i W[r, i] * m_i mod n --------------------------------
     def matvec_words(self, c_w: np.ndarray, w_mag_w: np.ndarray, w_neg: Optional[np.ndarray], k_bits: int) -> np.ndarray:
         """c_w: (count, words_out) any values; w_mag_w: (rows, count, words(k_bits)) magnitudes below 2^k_bits; w_neg: None or
@@ -535,6 +607,15 @@ class PaillierKey(CellMixin):
         out = np.empty((len(vals), nl, 2), dtype="<u8")
         check(self._lib.pb200_repack_limbs(self._h, _p(v_w), len(vals), value_bits, limb_bits, _p(out)), "pb200_repack_limbs")
         return [[int(out[i, j, 0]) | (int(out[i, j, 1]) << 64) for j in range(nl)] for i in range(len(vals))]
+
+
+def _check_out(status: int, where: str, out: np.ndarray) -> None:
+    """check(), with the outputs attached to the error: a call that fails with PB200_ERR_NOT_INVERTIBLE has still written every unit
+    (0 where the inverse does not exist)."""
+    if status != _lib.PB200_OK:
+        err = Pb200Error(status, where)
+        err.outputs = out
+        raise err
 
 
 def matvec_weights(W, count: int) -> Tuple[np.ndarray, Optional[np.ndarray], int]:

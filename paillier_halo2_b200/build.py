@@ -18,7 +18,7 @@ LIB = os.path.join(HERE, "libpaillier_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC"]
-SOURCES = ["capi.cu", "simple64_kernels.cu", "block28_kernels.cu", "cells.cu"]
+SOURCES = ["capi.cu", "simple64_kernels.cu", "block28_kernels.cu", "cells.cu", "inverse_kernels.cu"]
 
 
 def _deps_hash(src: str) -> str:

@@ -73,6 +73,8 @@ struct pb200_key {
     DevBuf mv_arena, mv_neg, mv_nm1;        // matvec: temporary memory of the plan, staged signs, copies of n - 1 for the sign step
     size_t mv_nm1_units = 0;
     DevBuf tr_tmp;                          // running-tally trace: per-level chunk totals and the leaf chunks' carries
+    InvConsts* d_inv = nullptr;             // inverse mod n^2: per-key constants, prepared on first use
+    DevBuf sgn;                             // signed scalar multiplication: staged sign bytes
     std::string engine_name;
     // K4 cell expansion: per lookup_bits layout + device constants (n^2 limbs, word_max, q_acc, mod_acc), refresh spill vector
     struct CellCtx { CellLayout Y; u64* d_consts = nullptr; int* d_inc = nullptr; u64* d_mtab = nullptr; int n_out = 0; int n2_cells = 0; };
@@ -102,7 +104,7 @@ const char* pb200_strerror(int s) {
         case PB200_OK: return "ok";
         case PB200_ERR_INVALID_ARG: return "invalid argument";
         case PB200_ERR_ZERO_MODULUS: return "modulus n is zero (num-bigint would panic)";
-        case PB200_ERR_EVEN_MODULUS: return "modulus n is even (reserved; even n is accepted)";
+        case PB200_ERR_EVEN_MODULUS: return "modulus n is even (inverse, subtraction and signed scalars need an odd n; other entry points accept it)";
         case PB200_ERR_RANGE: return "input does not fit its declared bit width (range check fails)";
         case PB200_ERR_UNSUPPORTED: return "key size not supported by any compiled engine";
         case PB200_ERR_CUDA: return "CUDA failure";
@@ -111,6 +113,7 @@ const char* pb200_strerror(int s) {
         case PB200_ERR_PEER: return "a peer GPU's tally partial did not arrive (every rank of the group must make the same call)";
         case PB200_ERR_DECRYPT: return "not a valid ciphertext for this key: c^lambda mod n^2 is not 1 modulo n";
         case PB200_ERR_CONSTRAINT: return "(q, rem) do not satisfy a*b = q*n^2 + rem (the chip's equality constraint fails)";
+        case PB200_ERR_NOT_INVERTIBLE: return "a value has no inverse mod n^2: gcd(c, n) != 1 (that unit's output is zero)";
         default: return "unknown status";
     }
 }
@@ -140,7 +143,7 @@ int pb200_key_create(int device, uint32_t n_bits, uint32_t limb_bits, const uint
     BigInt n = BigInt::from_u64_le(n_le, win), g = BigInt::from_u64_le(g_le, win);
     if (n.is_zero()) return PB200_ERR_ZERO_MODULUS;
     // even n is accepted: the reference's own tests draw n = rng.gen_biguint(bits) (src/paillier.rs:173,251) and nothing in the
-    // Barrett engines needs an odd modulus (PB200_ERR_EVEN_MODULUS stays in the enum for ABI stability, never returned)
+    // Barrett engines needs an odd modulus (only the inverse mod n^2 does: its entry points return PB200_ERR_EVEN_MODULUS)
     int ndev = pb200_device_count();
     if (device < 0 || device >= ndev) { t_cuda_error = "no such CUDA device"; return PB200_ERR_CUDA; }
     DevGuard dev_guard_; CU(dev_guard_.set(device));
@@ -189,6 +192,8 @@ void pb200_key_destroy(pb200_key* k) {
     k->wt_chunk.release(); k->wt_part.release();
     k->mv_arena.release(); k->mv_neg.release(); k->mv_nm1.release();
     k->tr_tmp.release();
+    if (k->d_inv) cudaFree(k->d_inv);
+    k->sgn.release();
     k->cin_a.release(); k->cin_b.release(); k->cin_q.release(); k->cin_r.release();
     if (k->pipe.ready) {
         if (k->pipe.copy) { cudaStreamSynchronize(k->pipe.copy); cudaStreamDestroy(k->pipe.copy); }
@@ -268,6 +273,7 @@ static int take_flags(pb200_key* k) {
     int rc = read_flags(k, &f); if (rc) return rc;
     if (f & PB200_FLAG_CONSTRAINT) return PB200_ERR_CONSTRAINT;
     if (f & PB200_FLAG_DECRYPT) return PB200_ERR_DECRYPT;
+    if (f & PB200_FLAG_NOT_INVERTIBLE) return PB200_ERR_NOT_INVERTIBLE;
     if (f & ~(PB200_FLAG_CONSTRAINT | PB200_FLAG_DECRYPT)) return PB200_ERR_RANGE;
     return PB200_OK;
 }
@@ -644,6 +650,17 @@ int pb200_tally_multi(pb200_key* const* keys, int n_gpus, const uint64_t* const*
 } PB200_CATCH
 
 // ---- decryption (SURVEY.md 8f-4) -----------------------------------------------------------------------------------------
+// Barrett constants of the modulus n itself (k = words_in; g slot zero): the L function of decryption and c mod n of the inverse
+static void consts_mod_n(const pb200_key* k, SimpleConsts* h) {
+    const uint32_t win = k->words_in;
+    memset(h, 0, sizeof(SimpleConsts));
+    h->k = (int)win; h->kin = (int)win; h->n_bits = (int)k->n_bits; h->exp_bits = 0;
+    h->s = (int)(64 * win - k->n.bits());
+    BigInt Nt = BigInt::shl(k->n, h->s);
+    BigInt bmu = BigInt::div(BigInt::pow2(128 * (size_t)win), Nt);
+    Nt.to_u64_le(h->Nt, win); bmu.to_u64_le(h->mu, win + 1);
+    k->n.to_u64_le(h->n, win);
+}
 int pb200_key_set_private(pb200_key* k, const uint64_t* lambda_le, const uint64_t* mu_le) try {
     if (!k || !lambda_le || !mu_le) return PB200_ERR_INVALID_ARG;
     if (!fits(lambda_le, k->words_in, k->n_bits) || !fits(mu_le, k->words_in, k->n_bits)) return PB200_ERR_RANGE;
@@ -652,13 +669,7 @@ int pb200_key_set_private(pb200_key* k, const uint64_t* lambda_le, const uint64_
     const uint32_t win = k->words_in;
     BigInt lambda = BigInt::from_u64_le(lambda_le, win), mu = BigInt::from_u64_le(mu_le, win);
     std::unique_ptr<SimpleConsts> h(new SimpleConsts());
-    memset(h.get(), 0, sizeof(SimpleConsts));
-    h->k = (int)win; h->kin = (int)win; h->n_bits = (int)k->n_bits; h->exp_bits = 0;
-    h->s = (int)(64 * win - k->n.bits());
-    BigInt Nt = BigInt::shl(k->n, h->s);
-    BigInt bmu = BigInt::div(BigInt::pow2(128 * (size_t)win), Nt);
-    Nt.to_u64_le(h->Nt, win); bmu.to_u64_le(h->mu, win + 1);
-    k->n.to_u64_le(h->n, win);
+    consts_mod_n(k, h.get());
     BigInt::mod(mu, k->n).to_u64_le(h->g, win);                 // the L-function kernel multiplies by this slot
     if (!k->d_simple_n) CU(cudaMalloc(&k->d_simple_n, sizeof(SimpleConsts)));
     if (!k->d_lambda) CU(cudaMalloc(&k->d_lambda, win * sizeof(u64)));
@@ -771,6 +782,113 @@ int pb200_tally_weighted(pb200_key* k, const uint64_t* c, const uint64_t* ks, ui
     rc = tally_weighted_dev_impl(k, (const u64*)k->in_a.p, (const u64*)k->in_b.p, k_bits, count, (u64*)k->out_b.p);
     if (rc) return rc;
     CU(cudaMemcpyAsync(out, k->out_b.p, bout, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
+} PB200_CATCH
+
+// ---- inverse mod n^2, subtraction and signed scalars ------------------------------------------------------------------------
+// per-key constants of the inverse kernel, prepared (and synchronised) on the first call
+static int ensure_inverse(pb200_key* k) {
+    if (k->d_inv) return PB200_OK;
+    std::unique_ptr<InvConsts> h(new InvConsts());
+    memset(h.get(), 0, sizeof(InvConsts));
+    consts_mod_n(k, &h->n);
+    inverse_consts(k->n, k->n_bits, h.get());
+    InvConsts* d = nullptr;
+    CU(cudaMalloc(&d, sizeof(InvConsts)));
+    cudaError_t e = cudaMemcpyAsync(d, h.get(), sizeof(InvConsts), cudaMemcpyHostToDevice, k->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(k->stream);
+    if (e != cudaSuccess) { cudaFree(d); return cuda_fail(e, "ensure_inverse"); }
+    k->d_inv = d;
+    return PB200_OK;
+}
+// d_c1 null: out = c^-1; else out = c1 * c^-1.  d_neg non-null: in place on the units with a negative non-zero magnitude only
+static int inverse_dev_impl(pb200_key* k, const u64* d_c, const u64* d_c1, const uint8_t* d_neg, const u64* d_mag, int kw, size_t count, u64* d_out) {
+    int rc = ensure_inverse(k); if (rc) return rc;
+    CU(simple_inverse(k->d_simple, k->d_inv, d_c, d_c1, d_neg, d_mag, kw, count, d_out, k->d_flags, k->stream));
+    return PB200_OK;
+}
+// the scalar chain on the key's engine with the magnitudes, then (c^s)^-1 = (c^-1)^s in place where the sign is negative
+static int scalar_signed_dev_impl(pb200_key* k, const u64* d_c, const u64* d_mag, const uint8_t* d_neg, uint32_t k_bits, size_t count, u64* d_out) {
+    int rc = scalar_dev_impl(k, d_c, d_mag, k_bits, count, d_out); if (rc) return rc;
+    return d_neg ? inverse_dev_impl(k, d_out, nullptr, d_neg, d_mag, (int)PB200_WORDS(k_bits), count, d_out) : PB200_OK;
+}
+
+int pb200_inverse_batch_dev(pb200_key* k, const uint64_t* d_c, size_t count, uint64_t* d_out) try {
+    if (!k || (count && (!d_c || !d_out))) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    if (!k->n.is_odd()) return PB200_ERR_EVEN_MODULUS;
+    USE_DEVICE(k);
+    return inverse_dev_impl(k, (const u64*)d_c, nullptr, nullptr, nullptr, 0, count, (u64*)d_out);
+} PB200_CATCH
+int pb200_inverse_batch(pb200_key* k, const uint64_t* c, size_t count, uint64_t* out) try {
+    if (!k || (count && (!c || !out))) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    if (!k->n.is_odd()) return PB200_ERR_EVEN_MODULUS;
+    USE_DEVICE(k);
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bc = count * k->words_out * sizeof(u64);
+    CU(k->in_a.reserve(bc)); CU(k->out_a.reserve(bc));
+    CU(cudaMemcpyAsync(k->in_a.p, c, bc, cudaMemcpyHostToDevice, k->stream));
+    int rc = inverse_dev_impl(k, (const u64*)k->in_a.p, nullptr, nullptr, nullptr, 0, count, (u64*)k->out_a.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out, k->out_a.p, bc, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
+} PB200_CATCH
+int pb200_sub_batch_dev(pb200_key* k, const uint64_t* d_c1, const uint64_t* d_c2, size_t count, uint64_t* d_out) try {
+    if (!k || (count && (!d_c1 || !d_c2 || !d_out))) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    if (!k->n.is_odd()) return PB200_ERR_EVEN_MODULUS;
+    USE_DEVICE(k);
+    return inverse_dev_impl(k, (const u64*)d_c2, (const u64*)d_c1, nullptr, nullptr, 0, count, (u64*)d_out);
+} PB200_CATCH
+int pb200_sub_batch(pb200_key* k, const uint64_t* c1, const uint64_t* c2, size_t count, uint64_t* out) try {
+    if (!k || (count && (!c1 || !c2 || !out))) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    if (!k->n.is_odd()) return PB200_ERR_EVEN_MODULUS;
+    USE_DEVICE(k);
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bc = count * k->words_out * sizeof(u64);
+    CU(k->in_a.reserve(bc)); CU(k->in_b.reserve(bc)); CU(k->out_a.reserve(bc));
+    CU(cudaMemcpyAsync(k->in_a.p, c1, bc, cudaMemcpyHostToDevice, k->stream));
+    CU(cudaMemcpyAsync(k->in_b.p, c2, bc, cudaMemcpyHostToDevice, k->stream));
+    int rc = inverse_dev_impl(k, (const u64*)k->in_b.p, (const u64*)k->in_a.p, nullptr, nullptr, 0, count, (u64*)k->out_a.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out, k->out_a.p, bc, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
+} PB200_CATCH
+int pb200_scalar_mul_signed_batch_dev(pb200_key* k, const uint64_t* d_c, const uint64_t* d_mag, const uint8_t* d_neg, uint32_t k_bits, size_t count,
+                                      uint64_t* d_out) try {
+    if (!scalar_args_ok(k, k_bits) || (count && (!d_c || !d_mag || !d_out))) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    if (d_neg && !k->n.is_odd()) return PB200_ERR_EVEN_MODULUS;
+    USE_DEVICE(k);
+    return scalar_signed_dev_impl(k, (const u64*)d_c, (const u64*)d_mag, d_neg, k_bits, count, (u64*)d_out);
+} PB200_CATCH
+int pb200_scalar_mul_signed_batch(pb200_key* k, const uint64_t* c, const uint64_t* mag, const uint8_t* neg, uint32_t k_bits, size_t count,
+                                  uint64_t* out) try {
+    if (!scalar_args_ok(k, k_bits) || (count && (!c || !mag || !out))) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    if (neg && !k->n.is_odd()) return PB200_ERR_EVEN_MODULUS;
+    int rc = check_scalars(mag, k_bits, count); if (rc) return rc;
+    bool any_neg = false;                             // all signs positive: exactly pb200_scalar_mul_batch, nothing to stage or invert
+    if (neg) for (size_t u = 0; u < count && !any_neg; u++) any_neg = neg[u] != 0;
+    USE_DEVICE(k);
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bc = count * k->words_out * sizeof(u64), bk = count * PB200_WORDS(k_bits) * sizeof(u64);
+    CU(k->in_a.reserve(bc)); CU(k->in_b.reserve(bk)); CU(k->out_a.reserve(bc));
+    CU(cudaMemcpyAsync(k->in_a.p, c, bc, cudaMemcpyHostToDevice, k->stream));
+    CU(cudaMemcpyAsync(k->in_b.p, mag, bk, cudaMemcpyHostToDevice, k->stream));
+    if (any_neg) {
+        CU(k->sgn.reserve(count));
+        CU(cudaMemcpyAsync(k->sgn.p, neg, count, cudaMemcpyHostToDevice, k->stream));
+    }
+    rc = scalar_signed_dev_impl(k, (const u64*)k->in_a.p, (const u64*)k->in_b.p, any_neg ? (const uint8_t*)k->sgn.p : nullptr, k_bits, count,
+                                (u64*)k->out_a.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out, k->out_a.p, bc, cudaMemcpyDeviceToHost, k->stream));
     CU(cudaStreamSynchronize(k->stream));
     return take_flags(k);
 } PB200_CATCH

@@ -35,6 +35,23 @@ cudaError_t simple_pow(const SimpleConsts* dK, const u64* d_base, int base_words
                        u64* d_out, int* d_flags, cudaStream_t st);
 cudaError_t simple_lfunc(const SimpleConsts* dKn, const u64* d_x, size_t count, u64* d_m, int* d_flags, cudaStream_t st);
 
+// ---- inverse mod n^2 (inverse_kernels.cu): safegcd mod n, then one Hensel step --------------------------------------------
+#define PB200_INV_MAXL 67   // signed 62-bit limbs of the safegcd state at |n| = 4096 (n_bits / 62 + 1)
+struct InvConsts {
+    SimpleConsts n;         // Barrett constants of the modulus n (k = words_in): c mod n
+    int L, batches;         // limbs, batches of 62 divsteps (Bernstein-Yang's bound for an n_bits-bit modulus)
+    u64 ninv62;             // n^-1 mod 2^62
+    long long n62[PB200_INV_MAXL];
+    u64 n2[PB200_SIMPLE_MAXK];
+};
+// the safegcd fields of an odd n (the caller fills the Barrett constants of n)
+void inverse_consts(const BigInt& n, uint32_t n_bits, InvConsts* h);
+// out_u = c_u^-1 mod n^2, or c1_u * c_u^-1 mod n^2 when d_c1 is given; a unit with gcd(c_u, n) != 1 gets 0 and raises PB200_FLAG_NOT_INVERTIBLE.  d_neg
+// non-null: only units with d_neg[u] != 0 and a non-zero magnitude (kw words at d_mag + u kw) are inverted, the others keep their value
+// (d_c == d_out is allowed)
+cudaError_t simple_inverse(const SimpleConsts* dK, const InvConsts* dI, const u64* d_c, const u64* d_c1, const uint8_t* d_neg, const u64* d_mag,
+                           int kw, size_t count, u64* d_out, int* d_flags, cudaStream_t st);
+
 // running-tally trace (pb200_tally_trace): level l holds n[l] entries per chain in chunks of s[l]; n[l + 1] = ceil(n[l] / s[l]) and the
 // last level has one chunk per chain.  Level 0 is the steps themselves.
 struct TracePlan { std::vector<size_t> n, s; };

@@ -16,7 +16,7 @@ fn main() {
     }
     let root = PathBuf::from(env::var("CARGO_MANIFEST_DIR").unwrap()).join("../..");
     let csrc = root.join("paillier_halo2_b200/csrc");
-    let sources = ["capi.cu", "simple64_kernels.cu", "block28_kernels.cu", "cells.cu"];
+    let sources = ["capi.cu", "simple64_kernels.cu", "block28_kernels.cu", "cells.cu", "inverse_kernels.cu"];
     let mut build = cc::Build::new();
     build
         .cuda(true)

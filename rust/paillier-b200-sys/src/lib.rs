@@ -25,10 +25,12 @@ pub const PB200_ERR_SINK: c_int = -8;
 pub const PB200_ERR_CONSTRAINT: c_int = -9;
 pub const PB200_ERR_PEER: c_int = -10;
 pub const PB200_ERR_DECRYPT: c_int = -11;
+pub const PB200_ERR_NOT_INVERTIBLE: c_int = -12;
 pub const PB200_FLAG_RANGE: u32 = 1;
 pub const PB200_FLAG_CONSTRAINT: u32 = 2;
 pub const PB200_FLAG_PEER_TIMEOUT: u32 = 4;
 pub const PB200_FLAG_DECRYPT: u32 = 8;
+pub const PB200_FLAG_NOT_INVERTIBLE: u32 = 16;
 
 /// 64-byte handle of a key's tally mailbox (CUDA IPC), exchanged between the ranks of a multi-process tally group
 #[repr(C)]
@@ -115,6 +117,14 @@ extern "C" {
     pub fn pb200_scalar_mul_batch_dev(key: *mut pb200_key, d_c_le: *const u64, d_k_le: *const u64, k_bits: u32, count: usize, d_out_le: *mut u64) -> c_int;
     pub fn pb200_tally_weighted(key: *mut pb200_key, c_le: *const u64, k_le: *const u64, k_bits: u32, count: usize, out_le: *mut u64) -> c_int;
     pub fn pb200_tally_weighted_dev(key: *mut pb200_key, d_c_le: *const u64, d_k_le: *const u64, k_bits: u32, count: usize, d_out_le: *mut u64) -> c_int;
+    pub fn pb200_inverse_batch(key: *mut pb200_key, c_le: *const u64, count: usize, out_le: *mut u64) -> c_int;
+    pub fn pb200_inverse_batch_dev(key: *mut pb200_key, d_c_le: *const u64, count: usize, d_out_le: *mut u64) -> c_int;
+    pub fn pb200_sub_batch(key: *mut pb200_key, c1_le: *const u64, c2_le: *const u64, count: usize, out_le: *mut u64) -> c_int;
+    pub fn pb200_sub_batch_dev(key: *mut pb200_key, d_c1_le: *const u64, d_c2_le: *const u64, count: usize, d_out_le: *mut u64) -> c_int;
+    pub fn pb200_scalar_mul_signed_batch(key: *mut pb200_key, c_le: *const u64, k_mag_le: *const u64, k_neg: *const u8, k_bits: u32, count: usize,
+                                         out_le: *mut u64) -> c_int;
+    pub fn pb200_scalar_mul_signed_batch_dev(key: *mut pb200_key, d_c_le: *const u64, d_k_mag_le: *const u64, d_k_neg: *const u8, k_bits: u32,
+                                             count: usize, d_out_le: *mut u64) -> c_int;
     pub fn pb200_matvec(key: *mut pb200_key, c_le: *const u64, count: usize, w_mag_le: *const u64, w_neg: *const u8, k_bits: u32, rows: usize,
                         out_le: *mut u64) -> c_int;
     pub fn pb200_matvec_dev(key: *mut pb200_key, d_c_le: *const u64, count: usize, d_w_mag_le: *const u64, d_w_neg: *const u8, k_bits: u32,
@@ -229,6 +239,42 @@ impl Key {
         }
         let mut out = vec![0u64; wo];
         let rc = unsafe { pb200_tally_weighted(self.raw, c.as_ptr(), k.as_ptr(), k_bits, c.len() / wo, out.as_mut_ptr()) };
+        if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// c_i^-1 mod n^2 for `count * words_out` words of ciphertexts: the ciphertexts of -m_i mod n.  A unit without an inverse
+    /// (gcd(c_i, n) != 1) makes the call return `Err(PB200_ERR_NOT_INVERTIBLE)`; `PB200_ERR_EVEN_MODULUS` for an even n
+    pub fn inverse_batch(&mut self, c: &[u64]) -> Result<Vec<u64>, i32> {
+        let wo = self.words_out();
+        if wo == 0 || c.len() % wo != 0 {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let mut out = vec![0u64; c.len()];
+        let rc = unsafe { pb200_inverse_batch(self.raw, c.as_ptr(), c.len() / wo, out.as_mut_ptr()) };
+        if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// homomorphic subtraction: c1_i * c2_i^-1 mod n^2, the ciphertexts of m1_i - m2_i mod n (errors as `inverse_batch`)
+    pub fn sub_batch(&mut self, c1: &[u64], c2: &[u64]) -> Result<Vec<u64>, i32> {
+        let wo = self.words_out();
+        if wo == 0 || c1.len() != c2.len() || c1.len() % wo != 0 {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let mut out = vec![0u64; c1.len()];
+        let rc = unsafe { pb200_sub_batch(self.raw, c1.as_ptr(), c2.as_ptr(), c1.len() / wo, out.as_mut_ptr()) };
+        if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// scalar multiplication with signed scalars: `k_mag` as `k` of scalar_mul_batch, `k_neg` (empty, or one byte per ciphertext,
+    /// non-zero = negative); returns c_i^(k_i) mod n^2 exactly (c^-s = (c^-1)^s, scalars not reduced mod n), the ciphertext of k_i * m_i
+    pub fn scalar_mul_signed_batch(&mut self, c: &[u64], k_mag: &[u64], k_neg: &[u8], k_bits: u32) -> Result<Vec<u64>, i32> {
+        let (wo, kw) = (self.words_out(), ((k_bits as usize) + 63) / 64);
+        if wo == 0 || kw == 0 || c.len() % wo != 0 || k_mag.len() != c.len() / wo * kw || (!k_neg.is_empty() && k_neg.len() != c.len() / wo) {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let mut out = vec![0u64; c.len()];
+        let neg = if k_neg.is_empty() { std::ptr::null() } else { k_neg.as_ptr() };
+        let rc = unsafe { pb200_scalar_mul_signed_batch(self.raw, c.as_ptr(), k_mag.as_ptr(), neg, k_bits, c.len() / wo, out.as_mut_ptr()) };
         if rc == PB200_OK { Ok(out) } else { Err(rc) }
     }
 
