@@ -41,8 +41,9 @@ typedef enum pb200_status {
     PB200_OK = 0,
     PB200_ERR_INVALID_ARG = -1,   /* null pointer, zero sizes, n_bits % limb_bits != 0 (assign_integer's assert) */
     PB200_ERR_ZERO_MODULUS = -2,  /* n == 0: num-bigint modpow / % panic (src/paillier.rs:89-91,96) */
-    PB200_ERR_EVEN_MODULUS = -3,  /* only from pb200_inverse_batch*, pb200_sub_batch* and pb200_scalar_mul_signed_batch* with signs
-                                     (their algorithm needs an odd n); every other entry point accepts an even n, as the reference
+    PB200_ERR_EVEN_MODULUS = -3,  /* only from pb200_inverse_batch*, pb200_sub_batch*, pb200_scalar_mul_signed_batch* with signs and
+                                     pb200_combine_shares_batch* with a negative coefficient (their algorithm needs an odd n); every
+                                     other entry point accepts an even n, as the reference
                                      does, whose tests draw n = rng.gen_biguint(bits) (src/paillier.rs:173,251) */
     PB200_ERR_RANGE = -4,         /* an input does not fit its declared bit width (range check would fail) */
     PB200_ERR_UNSUPPORTED = -5,   /* key size larger than the largest compiled engine */
@@ -268,6 +269,40 @@ int pb200_scalar_mul_signed_batch(pb200_key* key, const uint64_t* c_le, const ui
                                   size_t count, uint64_t* out_le);
 int pb200_scalar_mul_signed_batch_dev(pb200_key* key, const uint64_t* d_c_le, const uint64_t* d_k_mag_le, const uint8_t* d_k_neg,
                                       uint32_t k_bits, size_t count, uint64_t* d_out_le);
+
+/* ---- threshold decryption (Fouque-Poupard-Stern 2000, Shoup 2000, Damgard-Jurik 2001) --------------------------------------------
+ * The decryption key is split among l = parties trustees so that any t + 1 of them decrypt and t learn nothing; no party holds lambda.
+ * With M = n lambda, Delta = l! and L(x) = (x - 1) / n, a dealer (host key material, not in the library) takes d = lambda (lambda^-1 mod n)
+ * (d = 0 mod lambda, d = 1 mod n), a random polynomial f(X) = d + a_1 X + .. + a_t X^t mod M, the shares s_i = f(i) for i = 1 .. l, and
+ * phi = L(g^(4 Delta^2 d) mod n^2)^-1 mod n (for g = n + 1: (4 Delta^2)^-1 mod n).
+ *   pb200_partial_decrypt_batch:  trustee i, out_u = c_u^(2 Delta s_i) mod n^2
+ *   pb200_combine_shares_batch:   over a set S of distinct indices, mu_j = Delta prod_(j' in S, j' != j) j' / (j' - j) (an integer, may be
+ *                                 negative), P = prod_(mu_j > 0) c_j^(2 mu_j), N = prod_(mu_j < 0) c_j^(2 |mu_j|) mod n^2, m = L(P N^-1 mod n^2) phi mod n
+ * With |S| >= t + 1 honest shares m = Dec(c) for any g; with t shares or a corrupted one P N^-1 is not 1 mod n (except with negligible
+ * probability) and the unit raises PB200_ERR_DECRYPT.  Shares are not verified: a malicious trustee can shift m undetected.
+ *
+ * pb200_key_set_threshold: parties (1 .. 32) and phi (words_in words); clears any share set on the key.  PB200_ERR_INVALID_ARG for
+ * parties 0 or > 32, PB200_ERR_RANGE for phi >= 2^n_bits.  pb200_key_set_share: trustee `index` (1 .. parties, after set_threshold,
+ * else PB200_ERR_INVALID_ARG) and its share s (words_out words, any value); the library forms 2 Delta s and prepares its schedule.  A key
+ * can hold the private part and a share together.
+ * pb200_partial_decrypt_batch: c: count * words_out words (any value); out: count * words_out words, canonical.  Runs on the key's engine
+ * (block28: sliding window over the per-key exponent, as decryption).  PB200_ERR_INVALID_ARG when no share is set.
+ * pb200_combine_shares_batch: indices: k host integers (a host array in _dev too); shares: share-major, share j of unit u at
+ * (j * count + u) * words_out words; m_out: count * words_in words.  On a block28 key one multi-exponentiation per sign (Straus's
+ * method: one squaring chain for all the shares of a unit), then one inverse mod n^2 when some mu_j < 0, then L and phi.
+ * PB200_ERR_INVALID_ARG without set_threshold, for k == 0, an index 0 or > parties or an index given twice; PB200_ERR_EVEN_MODULUS for
+ * an even n when some mu_j < 0.  A unit whose N has no inverse gets m = 0 and raises PB200_FLAG_NOT_INVERTIBLE; an inexact L gives
+ * m = 0 and raises PB200_FLAG_DECRYPT.  The host variant copies every output back, then returns the status of the flags.  count == 0
+ * does nothing.  The first call on an index set prepares its schedules on the device (and, with a negative mu_j, the inverse's
+ * constants once per key); later _dev calls on the set enqueue without a synchronise.
+ * _dev: device pointers on the key's device, enqueued on the key's stream, no final synchronise; failures only raise flags. */
+int pb200_key_set_threshold(pb200_key* key, uint32_t parties, const uint64_t* phi_le);
+int pb200_key_set_share(pb200_key* key, uint32_t index, const uint64_t* s_le);
+int pb200_partial_decrypt_batch(pb200_key* key, const uint64_t* c_le, size_t count, uint64_t* out_le);
+int pb200_partial_decrypt_batch_dev(pb200_key* key, const uint64_t* d_c_le, size_t count, uint64_t* d_out_le);
+int pb200_combine_shares_batch(pb200_key* key, const uint32_t* indices, uint32_t k, const uint64_t* shares_le, size_t count, uint64_t* m_out_le);
+int pb200_combine_shares_batch_dev(pb200_key* key, const uint32_t* indices, uint32_t k, const uint64_t* d_shares_le, size_t count,
+                                   uint64_t* d_m_out_le);
 
 /* ---- encrypted matrix-vector product with a signed plaintext matrix ------------------------------------------------------
  * Enc(W m) from Enc(m): private scoring with a linear model, multi-question ballots, PIR-style selection.  On a block28 engine a

@@ -93,6 +93,12 @@ SYMBOLS = {
     "pb200_sub_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "pb200_scalar_mul_signed_batch": (C.c_int, [C.c_void_p, u64p, u64p, C.c_void_p, C.c_uint32, C.c_size_t, u64p]),
     "pb200_scalar_mul_signed_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
+    "pb200_key_set_threshold": (C.c_int, [C.c_void_p, C.c_uint32, u64p]),
+    "pb200_key_set_share": (C.c_int, [C.c_void_p, C.c_uint32, u64p]),
+    "pb200_partial_decrypt_batch": (C.c_int, [C.c_void_p, u64p, C.c_size_t, u64p]),
+    "pb200_partial_decrypt_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "pb200_combine_shares_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, u64p, C.c_size_t, u64p]),
+    "pb200_combine_shares_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_size_t, C.c_void_p]),
     "pb200_matvec": (C.c_int, [C.c_void_p, u64p, C.c_size_t, u64p, C.c_void_p, C.c_uint32, C.c_size_t, u64p]),
     "pb200_matvec_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t, C.c_void_p]),
     "pb200_matvec_plan": (C.c_int, [C.c_uint32, C.c_int, C.c_size_t, C.c_size_t, C.c_uint32, C.c_int, u64p]),

@@ -517,6 +517,65 @@ class PaillierKey(CellMixin):
         mag_w = ints_to_words([abs(k) for k in ks], words(k_bits))
         return words_to_ints(self.scalar_mul_signed_words(self._ciphertexts(cs, "scalar_mul_signed"), mag_w, neg if neg.any() else None, k_bits))
 
+    # -- threshold decryption: any t + 1 of `parties` trustees decrypt, t learn nothing (threshold_from_primes deals the shares) ------
+    def set_threshold(self, parties: int, phi: int) -> None:
+        """parties = l (1 .. 32, Delta = l!) and phi = L(g^(4 Delta^2 d) mod n^2)^-1 mod n; clears any share set on this key."""
+        try:
+            a = ints_to_words([phi], self.words_in)
+        except OverflowError:
+            raise Pb200Error(_lib.PB200_ERR_RANGE, "set_threshold")
+        check(self._lib.pb200_key_set_threshold(self._h, parties, _p(a)), "pb200_key_set_threshold")
+
+    def set_share(self, index: int, share: int) -> None:
+        """Trustee `index` (1 .. parties) and its share s_index (below 2^(64 words_out)); partial_decrypt then computes c^(2 Delta s)."""
+        try:
+            a = ints_to_words([share], self.words_out)
+        except OverflowError:
+            raise Pb200Error(_lib.PB200_ERR_RANGE, "set_share")
+        check(self._lib.pb200_key_set_share(self._h, index, _p(a)), "pb200_key_set_share")
+
+    def partial_decrypt_words(self, c_w: np.ndarray) -> np.ndarray:
+        """c_w: (count, words_out) any values -> (count, words_out) c^(2 Delta s) mod n^2 (pb200_partial_decrypt_batch)."""
+        c_w = np.ascontiguousarray(c_w, dtype="<u8").reshape(-1, self.words_out)
+        out = np.empty_like(c_w)
+        check(self._lib.pb200_partial_decrypt_batch(self._h, _p(c_w) if c_w.shape[0] else None, c_w.shape[0], _p(out)),
+              "pb200_partial_decrypt_batch")
+        return out
+
+    def partial_decrypt_dev(self, d_c: int, count: int, d_out: int) -> None:
+        """Device-pointer variant (pb200_partial_decrypt_batch_dev): enqueues on the key's stream, no synchronise."""
+        check(self._lib.pb200_partial_decrypt_batch_dev(self._h, d_c, count, d_out), "pb200_partial_decrypt_batch_dev")
+
+    def partial_decrypt(self, cs: Sequence[int]) -> List[int]:
+        """This trustee's decryption share c^(2 Delta s) mod n^2 of every ciphertext."""
+        return words_to_ints(self.partial_decrypt_words(self._ciphertexts(cs, "partial_decrypt"))) if len(cs) else []
+
+    def combine_shares_words(self, indices: Sequence[int], shares_w: np.ndarray) -> np.ndarray:
+        """indices: the k trustees; shares_w: (k, count, words_out), share j of unit u at [j, u] -> (count, words_in) plaintexts
+        (pb200_combine_shares_batch).  PB200_ERR_DECRYPT / PB200_ERR_NOT_INVERTIBLE carry the outputs (Pb200Error.outputs, 0 there)."""
+        idx = np.ascontiguousarray([int(i) for i in indices], dtype=np.uint32)
+        shares_w = np.ascontiguousarray(shares_w, dtype="<u8").reshape(idx.size, -1, self.words_out)
+        count = shares_w.shape[1]
+        out = np.empty((count, self.words_in), dtype="<u8")
+        _check_out(self._lib.pb200_combine_shares_batch(self._h, idx.ctypes.data_as(C.c_void_p), idx.size, _p(shares_w) if count else None,
+                                                        count, _p(out)), "pb200_combine_shares_batch", out)
+        return out
+
+    def combine_shares_dev(self, indices: Sequence[int], d_shares: int, count: int, d_m: int) -> None:
+        """Device-pointer variant (pb200_combine_shares_batch_dev; indices stay on the host): enqueues on the key's stream, no synchronise;
+        failures of units only raise PB200_FLAG_DECRYPT / PB200_FLAG_NOT_INVERTIBLE (take_flags)."""
+        idx = np.ascontiguousarray([int(i) for i in indices], dtype=np.uint32)
+        check(self._lib.pb200_combine_shares_batch_dev(self._h, idx.ctypes.data_as(C.c_void_p), idx.size, d_shares, count, d_m),
+              "pb200_combine_shares_batch_dev")
+
+    def combine_shares(self, indices: Sequence[int], shares: Sequence[Sequence[int]]) -> List[int]:
+        """shares[j][u]: trustee indices[j]'s partial decryption of ciphertext u -> the plaintexts m_u."""
+        assert len(indices) == len(shares)
+        count = len(shares[0]) if len(shares) else 0
+        assert all(len(s) == count for s in shares)
+        w = np.stack([self._ciphertexts(s, "combine_shares") for s in shares]) if count else np.empty((len(shares), 0, self.words_out), "<u8")
+        return words_to_ints(self.combine_shares_words(indices, w)) if count else []
+
     # -- encrypted matrix-vector product: row r of the result encrypts sum_i W[r, i] * m_i mod n --------------------------------
     def matvec_words(self, c_w: np.ndarray, w_mag_w: np.ndarray, w_neg: Optional[np.ndarray], k_bits: int) -> np.ndarray:
         """c_w: (count, words_out) any values; w_mag_w: (rows, count, words(k_bits)) magnitudes below 2^k_bits; w_neg: None or
@@ -704,3 +763,25 @@ def private_from_primes(p: int, q: int, g: int):
     lam = (p - 1) * (q - 1) // gcd(p - 1, q - 1)
     x = pow(g, lam, n * n)
     return lam, pow((x - 1) // n, -1, n)
+
+
+def threshold_from_primes(p: int, q: int, g: int, t: int, parties: int, rng=None):
+    """Dealer of threshold decryption (host key material, like private_from_primes): any t + 1 of `parties` trustees can decrypt.
+    d = lambda (lambda^-1 mod n), f(X) = d + a_1 X + .. + a_t X^t mod n lambda with random a_k, share s_i = f(i) for i = 1 .. parties,
+    phi = L(g^(4 Delta^2 d) mod n^2)^-1 mod n with Delta = parties!.  Returns ({i: s_i}, phi).  rng defaults to secrets.SystemRandom()."""
+    from math import factorial, gcd
+    if not 0 <= t < parties <= 32:
+        raise ValueError("need 0 <= t < parties <= 32")
+    if rng is None:
+        import secrets
+        rng = secrets.SystemRandom()
+    n = p * q
+    n2 = n * n
+    lam = (p - 1) * (q - 1) // gcd(p - 1, q - 1)
+    M = n * lam
+    d = lam * pow(lam, -1, n)
+    coeffs = [d] + [rng.randrange(M) for _ in range(t)]
+    shares = {i: sum(a * i ** k for k, a in enumerate(coeffs)) % M for i in range(1, parties + 1)}
+    delta = factorial(parties)
+    theta = (pow(g, 4 * delta * delta * d, n2) - 1) // n % n
+    return shares, pow(theta, -1, n)

@@ -350,6 +350,38 @@ __device__ __forceinline__ void slots_release(const SlotPool& P, const int* s_sl
     if (threadIdx.x == 0) for (int g = 0; g < LG; g++) slot_release(P, s_slot[g]);
 }
 
+// k_multipow's two halves of window_pow, with the table width a run-time value (window_pow keeps its own fixed-width copy: folding it
+// onto these changed the register allocation and spills of k_encrypt and k_pow).
+// The odd powers x, x^3, .., x^(2 h - 1) of the x in V (each lane its own) -> tab[0 .. h) of the CTA's scratch slot; x^2 passes
+// through the entry sq (h > 1).  V is left holding the last power.
+template <class C, int ENG, class SV>
+__device__ __forceinline__ void odd_powers(SV& S, int4* tab, int h, int4* sq, int role, int lane) {
+    copy_to_global<C>(tab, S.V, role, lane);                                        // tab[0] = x
+    if (h < 2) return;
+    mm<C, true, ENG>(S, nullptr, role, lane);                                   // x^2
+    copy_to_global<C>(sq, S.V, role, lane);
+    __syncthreads();
+    copy_from_global<C>(S.V, tab, role, lane);
+    for (int j = 1; j < h; j++) {
+        copy_from_global<C>(S.B, sq, role, lane);
+        mm<C, false, ENG>(S, S.B, role, lane);                                  // x^(2j+1)
+        copy_to_global<C>(tab + (size_t)j * C::VAL4, S.V, role, lane);
+    }
+}
+// V <- the product the schedule E describes over the table tab (multipow_schedule); an empty schedule gives 1
+template <class C, int ENG, class SV>
+__device__ __forceinline__ void pow_chain(SV& S, const PowSched& E, const int4* tab, int role, int lane) {
+    if (E.first_idx < 0) set_one_where<C>(S.V, true, role, lane);                   // e == 0
+    else copy_from_global<C>(S.V, tab + (size_t)E.first_idx * C::VAL4, role, lane);
+    for (int o = 0; o < E.n_ops; o++) {
+        const int2 op = E.ops[o];
+        for (int s_ = 0; s_ < op.x; s_++) mm<C, true, ENG>(S, nullptr, role, lane);
+        if (op.y >= 0) {
+            copy_from_global<C>(S.B, tab + (size_t)op.y * C::VAL4, role, lane);
+            mm<C, false, ENG>(S, S.B, role, lane);
+        }
+    }
+}
 // V <- x^e for the x in V (each lane its own), e given by its sliding-window schedule E; e == 0 gives 1.  The odd powers x, x^3, ..,
 // x^(2 TABN - 1) go to tab[0 .. TABN) of the CTA's scratch slot, x^2 to tab[TABN].
 template <class C, int ENG, class SV>
@@ -444,6 +476,35 @@ __global__ void __launch_bounds__(View<C, ENG>::THREADS, View<C, ENG>::PER_SM) k
     window_pow<C, ENG>(S, E, tab, role, lane);
     finalize<C, ENG>(S, K, out + unit * K.words_out, active, role, lane);
     slots_release<LG>(pool, s_slot);
+    cta_end(S);
+}
+
+// out_u = prod_j b_(j, u)^(e_j) mod n^2 over k <= MULTIPOW_MAXK bases per lane with exponents shared by the batch (Straus): one squaring
+// chain for all bases.  Base j of unit u is at base + (pos[j] * stride + u) * words_out (any words_out-word value).  Each lane puts the
+// odd powers of its k bases into the CTA's scratch slot, h = 2^(w - 1) per base (base j at entries [j h, j h + h), x^2 passing through
+// entry k h), then runs the merged schedule E (multipow_schedule), which every lane of the CTA shares.  Tally CTA shape (ENG 0 / 1 / 4).
+constexpr int MULTIPOW_MAXK = 32;
+struct MultiBases { const u64* base; size_t stride; const int* pos; int k; };      // pos: device array of k share positions
+
+template <class C, int ENG>
+__global__ void __launch_bounds__(C::THREADS, View<C, ENG>::PER_SM) k_multipow(B28Dev K, MultiBases B, int h, PowSched E, size_t count,
+                                                                         u64* __restrict__ out, int4* scratch, SlotPool pool) {
+    extern __shared__ int4 smem[];
+    __shared__ int s_slot[1];
+    typename View<C, ENG>::type S(smem);
+    const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
+    slots_acquire<1>(pool, s_slot);
+    cta_begin(S, smem, K);
+    const auto [unit, active] = lane_unit(count, lane);
+    int4* tab = scratch + (size_t)s_slot[0] * SCRATCH_ENTRIES * C::VAL4;
+    for (int j = 0; j < B.k; j++) {
+        load_value<C>(S.V, B.base + ((size_t)B.pos[j] * B.stride + unit) * K.words_out, K.words_out, role, lane);
+        odd_powers<C, ENG>(S, tab + (size_t)j * h * C::VAL4, h, tab + (size_t)B.k * h * C::VAL4, role, lane);
+        __syncthreads();
+    }
+    pow_chain<C, ENG>(S, E, tab, role, lane);
+    finalize<C, ENG>(S, K, out + unit * K.words_out, active, role, lane);
+    slots_release<1>(pool, s_slot);
     cta_end(S);
 }
 
@@ -1241,8 +1302,8 @@ struct Block28Key {
     TallyPeer peer{};                                        // world <= 1 until block28_tally_peer_connect
     void* ipc_opened[TALLY_MAXW] = {};                       // peer mailboxes opened with cudaIpcOpenMemHandle
     int device = 0;
-    int2* d_pow_ops = nullptr; PowSched pow{};               // decryption exponent (block28_pow_prepare)
-    bool pow_ready = false;
+    int2* d_pow_ops[POW_SLOTS] = {}; PowSched pow[POW_SLOTS] = {};   // per-key exponents of k_pow (block28_pow_prepare)
+    bool pow_ready[POW_SLOTS] = {};
     int sms = 148;
     uint64_t n_sqr = 0, n_mul = 0;   // modular squarings / multiplications per encryption
     int eng = 1;                     // 0: all phases on IMAD (block28), 1: phases B, C on mma.sync (block28t), 2: on tcgen05, 32 ciphertexts per
@@ -1296,24 +1357,31 @@ static void to_rtab(const std::vector<int>& entry, std::vector<int>& out_words) 
     memcpy(out_words.data(), tab.data(), tab.size());
 }
 
-// left-to-right sliding window (width WIN) over a fixed exponent: returns the table index the chain starts from (-1 for e == 0)
-// and the list of (squarings, table index to multiply by or -1)
-static int window_schedule(const BigInt& e, std::vector<int2>& ops) {
-    int first_idx = -1;
-    int i = (int)e.bits() - 1, pending = 0; bool first = true;
-    while (i >= 0) {
-        if (!e.bit(i)) { pending++; i--; continue; }
-        int j = i - WIN + 1; if (j < 0) j = 0;
-        while (!e.bit(j)) j++;
-        int val = 0; for (int b = i; b >= j; b--) val = (val << 1) | (e.bit(b) ? 1 : 0);
-        int len = i - j + 1;
-        if (first) { first_idx = (val - 1) / 2; first = false; }
-        else ops.push_back(make_int2(pending + len, (val - 1) / 2));
-        pending = 0; i = j - 1;
+// Straus's merged left-to-right sliding-window schedule of k exponents e_j (windows of w bits, h = 2^(w - 1) odd powers per base,
+// exponent j's at table entries [j h, j h + h)): one squaring chain, each window multiplied in where its lowest bit falls.  Returns the
+// table entry the chain starts from (-1: every exponent is 0) and the list of (squarings, table entry to multiply by or -1).
+static int multipow_schedule(const std::vector<BigInt>& e, int w, std::vector<int2>& ops) {
+    struct Win { int low, j, idx; };
+    std::vector<Win> wins;
+    for (int j = 0; j < (int)e.size(); j++) {
+        int i = (int)e[j].bits() - 1;
+        while (i >= 0) {
+            if (!e[j].bit(i)) { i--; continue; }
+            int lo = i - w + 1; if (lo < 0) lo = 0;
+            while (!e[j].bit(lo)) lo++;
+            int val = 0; for (int b = i; b >= lo; b--) val = (val << 1) | (e[j].bit(b) ? 1 : 0);
+            wins.push_back({lo, j, j * (1 << (w - 1)) + (val - 1) / 2});
+            i = lo - 1;
+        }
     }
-    if (pending) ops.push_back(make_int2(pending, -1));
-    return first_idx;
+    std::stable_sort(wins.begin(), wins.end(), [](const Win& a, const Win& b) { return a.low > b.low || (a.low == b.low && a.j < b.j); });
+    if (wins.empty()) return -1;
+    for (size_t t = 1; t < wins.size(); t++) ops.push_back(make_int2(wins[t - 1].low - wins[t].low, wins[t].idx));
+    if (wins.back().low) ops.push_back(make_int2(wins.back().low, -1));
+    return wins[0].idx;
 }
+// left-to-right sliding window (width WIN) over one fixed exponent
+static int window_schedule(const BigInt& e, std::vector<int2>& ops) { return multipow_schedule({e}, WIN, ops); }
 
 #define CUW(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return e_; } while (0)
 #define CUK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { *cuda_err = e_; block28_destroy(key); return nullptr; } } while (0)
@@ -1505,11 +1573,11 @@ static cudaError_t encrypt_cfg(Block28Key* key, const u64* d_m, const u64* d_r, 
 }
 
 template <class C>
-static cudaError_t pow_cfg(Block28Key* key, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st) {
+static cudaError_t pow_cfg(Block28Key* key, int slot, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st) {
     CUW(ensure_slots<C>(key, st));
     const SlotPool pool{key->d_slot_masks, key->enc_per_sm};
     return with_eng<View, C, 0, 1, 2, 3>(key->eng, [&](auto e) {
-        return launch<View<C, e>>(k_pow<C, e>, cdiv(count, 32 * View<C, e>::LG), st, key->dev, key->pow, d_base, base_words, count, d_out,
+        return launch<View<C, e>>(k_pow<C, e>, cdiv(count, 32 * View<C, e>::LG), st, key->dev, key->pow[slot], d_base, base_words, count, d_out,
                                   key->d_scratch, pool);
     });
 }
@@ -1690,7 +1758,7 @@ void block28_destroy(Block28Key* key) {
     if (key->d_gwords) cudaFree(key->d_gwords);
     if (key->d_scratch) cudaFree(key->d_scratch);
     if (key->d_slot_masks) cudaFree(key->d_slot_masks);
-    if (key->d_pow_ops) cudaFree(key->d_pow_ops);
+    for (int i = 0; i < POW_SLOTS; i++) if (key->d_pow_ops[i]) cudaFree(key->d_pow_ops[i]);
     if (key->d_nodes) cudaFree(key->d_nodes);
     if (key->d_node_cnt) cudaFree(key->d_node_cnt);
     for (int i = 0; i < TALLY_MAXW; i++) if (key->ipc_opened[i]) cudaIpcCloseMemHandle(key->ipc_opened[i]);
@@ -1721,18 +1789,59 @@ void block28_chain_counts(const Block28Key* key, uint64_t* n_sqr, uint64_t* n_mu
 cudaError_t block28_encrypt(Block28Key* key, const u64* d_m, const u64* d_r, size_t count, u64* d_c, cudaStream_t st) {
     return with_cfg(key, [&](auto c) { return encrypt_cfg<decltype(c)>(key, d_m, d_r, count, d_c, st); });
 }
-cudaError_t block28_pow_prepare(Block28Key* key, const BigInt& e, cudaStream_t st) {
+cudaError_t block28_pow_prepare(Block28Key* key, int slot, const BigInt& e, cudaStream_t st) {
+    if (slot < 0 || slot >= POW_SLOTS) return cudaErrorInvalidValue;
     std::vector<int2> ops;
-    if (key->d_pow_ops) { cudaFree(key->d_pow_ops); key->d_pow_ops = nullptr; }
-    CUW(upload_schedule(e, ops, &key->d_pow_ops, &key->pow, st));
+    key->pow_ready[slot] = false;
+    if (key->d_pow_ops[slot]) { CUW(cudaStreamSynchronize(st)); cudaFree(key->d_pow_ops[slot]); key->d_pow_ops[slot] = nullptr; }
+    CUW(upload_schedule(e, ops, &key->d_pow_ops[slot], &key->pow[slot], st));
     CUW(cudaStreamSynchronize(st));
-    key->pow_ready = true;
+    key->pow_ready[slot] = true;
     return cudaSuccess;
 }
-cudaError_t block28_pow(Block28Key* key, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st) {
+cudaError_t block28_pow(Block28Key* key, int slot, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st) {
     if (!count) return cudaSuccess;
-    if (!key->pow_ready) return cudaErrorInvalidValue;
-    return with_cfg(key, [&](auto c) { return pow_cfg<decltype(c)>(key, d_base, base_words, count, d_out, st); });
+    if (slot < 0 || slot >= POW_SLOTS || !key->pow_ready[slot]) return cudaErrorInvalidValue;
+    return with_cfg(key, [&](auto c) { return pow_cfg<decltype(c)>(key, slot, d_base, base_words, count, d_out, st); });
+}
+// the table width of k_multipow for these exponents: the w whose table (k h entries and x^2, within the CTA's scratch slot) and merged
+// chain take the fewest multiplications
+cudaError_t block28_multipow_prepare(const std::vector<BigInt>& e, const std::vector<int>& pos, MultiPow* P, cudaStream_t st) {
+    const int k = (int)e.size();
+    if (k < 1 || k > MULTIPOW_MAXK || (int)pos.size() != k) return cudaErrorInvalidValue;
+    uint64_t best = ~0ull;
+    for (int w = 1; w <= WIN && k * (1 << (w - 1)) + 1 <= SCRATCH_ENTRIES; w++) {
+        std::vector<int2> ops;
+        const int first = multipow_schedule(e, w, ops);
+        uint64_t sqr = 0, mul = w > 1 ? (uint64_t)k * (1u << (w - 1)) : 0;      // table: one squaring and h - 1 products per base
+        for (const int2& o : ops) { sqr += (uint64_t)o.x; mul += o.y >= 0; }
+        if (sqr + mul < best) { best = sqr + mul; P->h = 1 << (w - 1); P->first_idx = first; P->ops = ops; P->n_sqr = sqr; P->n_mul = mul; }
+    }
+    P->k = k;
+    P->pos = pos;
+    block28_multipow_free(P);
+    CUW(upload(&P->d_ops, P->ops, st));
+    return upload(&P->d_pos, P->pos, st);
+}
+void block28_multipow_free(MultiPow* P) {
+    if (P->d_ops) cudaFree(P->d_ops);
+    if (P->d_pos) cudaFree(P->d_pos);
+    P->d_ops = nullptr; P->d_pos = nullptr;
+}
+template <class C>
+static cudaError_t multipow_cfg(Block28Key* key, const MultiPow& P, const u64* d_base, size_t stride, size_t count, u64* d_out, cudaStream_t st) {
+    CUW(ensure_slots<C>(key, st));
+    const SlotPool pool{key->d_slot_masks, key->enc_per_sm};
+    const MultiBases B{d_base, stride, P.d_pos, P.k};
+    const PowSched E{P.d_ops, (int)P.ops.size(), P.first_idx};
+    return with_eng<View, C, 0, 1, 4>(tally_eng(key), [&](auto e) {
+        return launch<View<C, e>>(k_multipow<C, e>, cdiv(count, 32), st, key->dev, B, P.h, E, count, d_out, key->d_scratch, pool);
+    });
+}
+cudaError_t block28_multipow(Block28Key* key, const MultiPow& P, const u64* d_base, size_t stride, size_t count, u64* d_out, cudaStream_t st) {
+    if (!count) return cudaSuccess;
+    if (P.k < 1 || P.k > MULTIPOW_MAXK || !P.d_ops || !P.d_pos) return cudaErrorInvalidValue;
+    return with_cfg(key, [&](auto c) { return multipow_cfg<decltype(c)>(key, P, d_base, stride, count, d_out, st); });
 }
 cudaError_t block28_scalar(Block28Key* key, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out, cudaStream_t st) {
     if (!count) return cudaSuccess;

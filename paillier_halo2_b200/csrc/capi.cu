@@ -84,6 +84,20 @@ struct pb200_key {
     std::vector<pb200_key*> group;          // pb200_tally_multi: the peer group this key is connected to (single process)
     // private part (pb200_key_set_private): constants of the modulus n with mu in their g slot, lambda's words for the simple pow
     SimpleConsts* d_simple_n = nullptr; u64* d_lambda = nullptr; int lambda_bits = 0; bool has_private = false;
+    // threshold decryption (pb200_key_set_threshold / pb200_key_set_share): parties l (Delta = l!), constants of n with phi in their g
+    // slot, the share's exponent 2 Delta s for simple_pow, and one combination plan per index set
+    uint32_t parties = 0; BigInt delta; SimpleConsts* d_simple_phi = nullptr;
+    u64* d_share_e = nullptr; int share_e_bits = 0; bool has_share = false;
+    struct Combine {
+        bool any_neg = false;
+        MultiPow pos, neg;                      // k_multipow plans of the positive and the negative Lagrange exponents (block28 keys)
+        std::vector<bool> is_neg;               // mu_j < 0, in the order of the index set
+        std::vector<int> e_bits;                // simple64: bits of 2 |mu_j| and their words (ew each) on the device
+        std::vector<u64> e_words; int ew = 0; u64* d_e = nullptr;
+        void release() { block28_multipow_free(&pos); block28_multipow_free(&neg); if (d_e) cudaFree(d_e); d_e = nullptr; }
+    };
+    std::map<std::vector<uint32_t>, Combine> combine;
+    DevBuf th_p, th_n, th_x;                // combination: P, N, P N^-1
     // witness delivery pipeline (pb200_encrypt_witness_batch): created on first use
     struct Pipe {
         static const int NS = 4;             // pinned staging slots
@@ -104,7 +118,7 @@ const char* pb200_strerror(int s) {
         case PB200_OK: return "ok";
         case PB200_ERR_INVALID_ARG: return "invalid argument";
         case PB200_ERR_ZERO_MODULUS: return "modulus n is zero (num-bigint would panic)";
-        case PB200_ERR_EVEN_MODULUS: return "modulus n is even (inverse, subtraction and signed scalars need an odd n; other entry points accept it)";
+        case PB200_ERR_EVEN_MODULUS: return "modulus n is even (inverse, subtraction, signed scalars and combining shares with a negative coefficient need an odd n; other entry points accept it)";
         case PB200_ERR_RANGE: return "input does not fit its declared bit width (range check fails)";
         case PB200_ERR_UNSUPPORTED: return "key size not supported by any compiled engine";
         case PB200_ERR_CUDA: return "CUDA failure";
@@ -188,6 +202,10 @@ void pb200_key_destroy(pb200_key* k) {
     if (k->d_flags) cudaFree(k->d_flags);
     if (k->d_simple_n) cudaFree(k->d_simple_n);
     if (k->d_lambda) cudaFree(k->d_lambda);
+    if (k->d_simple_phi) cudaFree(k->d_simple_phi);
+    if (k->d_share_e) cudaFree(k->d_share_e);
+    for (auto& kv : k->combine) kv.second.release();
+    k->th_p.release(); k->th_n.release(); k->th_x.release();
     k->in_a.release(); k->in_b.release(); k->out_a.release(); k->out_b.release(); k->scratch.release(); k->offs.release();
     k->wt_chunk.release(); k->wt_part.release();
     k->mv_arena.release(); k->mv_neg.release(); k->mv_nm1.release();
@@ -677,7 +695,7 @@ int pb200_key_set_private(pb200_key* k, const uint64_t* lambda_le, const uint64_
     CU(cudaMemcpyAsync(k->d_lambda, lambda_le, win * sizeof(u64), cudaMemcpyHostToDevice, k->stream));
     CU(cudaStreamSynchronize(k->stream));
     k->lambda_bits = (int)lambda.bits();
-    if (k->fast) CU(block28_pow_prepare(k->fast, lambda, k->stream));
+    if (k->fast) CU(block28_pow_prepare(k->fast, POW_LAMBDA, lambda, k->stream));
     k->has_private = true;
     return PB200_OK;
 } PB200_CATCH
@@ -689,7 +707,7 @@ int pb200_decrypt_batch_dev(pb200_key* k, const uint64_t* d_c, size_t count, uin
     USE_DEVICE(k);
     CU(k->scratch.reserve(count * k->words_out * sizeof(u64)));
     u64* d_x = (u64*)k->scratch.p;                               // x = c^lambda mod n^2
-    if (use_fast(k)) CU(block28_pow(k->fast, (const u64*)d_c, (int)k->words_out, count, d_x, k->stream));
+    if (use_fast(k)) CU(block28_pow(k->fast, POW_LAMBDA, (const u64*)d_c, (int)k->words_out, count, d_x, k->stream));
     else CU(simple_pow(k->d_simple, (const u64*)d_c, (int)k->words_out, k->d_lambda, k->lambda_bits, 0, count, d_x, k->d_flags, k->stream));
     CU(simple_lfunc(k->d_simple_n, d_x, count, (u64*)d_m, k->d_flags, k->stream));
     return PB200_OK;
@@ -889,6 +907,193 @@ int pb200_scalar_mul_signed_batch(pb200_key* k, const uint64_t* c, const uint64_
                                 (u64*)k->out_a.p);
     if (rc) return rc;
     CU(cudaMemcpyAsync(out, k->out_a.p, bc, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
+} PB200_CATCH
+
+// ---- threshold decryption: partial decryptions c^(2 Delta s_i) and their combination ---------------------------------------------
+static void drop_combine_plans(pb200_key* k) {
+    if (k->combine.empty()) return;
+    cudaStreamSynchronize(k->stream);                            // the plans' schedules may still be read by enqueued launches
+    for (auto& kv : k->combine) kv.second.release();
+    k->combine.clear();
+}
+int pb200_key_set_threshold(pb200_key* k, uint32_t parties, const uint64_t* phi_le) try {
+    if (!k || !phi_le || parties == 0 || parties > 32) return PB200_ERR_INVALID_ARG;
+    if (!fits(phi_le, k->words_in, k->n_bits)) return PB200_ERR_RANGE;
+    USE_DEVICE(k);
+    CU(cudaStreamSynchronize(k->stream));
+    const uint32_t win = k->words_in;
+    std::unique_ptr<SimpleConsts> h(new SimpleConsts());
+    consts_mod_n(k, h.get());
+    BigInt::mod(BigInt::from_u64_le(phi_le, win), k->n).to_u64_le(h->g, win);   // the L-function kernel multiplies by this slot
+    if (!k->d_simple_phi) CU(cudaMalloc(&k->d_simple_phi, sizeof(SimpleConsts)));
+    CU(cudaMemcpyAsync(k->d_simple_phi, h.get(), sizeof(SimpleConsts), cudaMemcpyHostToDevice, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    drop_combine_plans(k);
+    k->parties = parties;
+    k->delta = BigInt(1);
+    for (uint32_t i = 2; i <= parties; i++) k->delta = BigInt::mul(k->delta, BigInt(i));
+    k->has_share = false;
+    return PB200_OK;
+} PB200_CATCH
+
+int pb200_key_set_share(pb200_key* k, uint32_t index, const uint64_t* s_le) try {
+    if (!k || !s_le || k->parties == 0 || index < 1 || index > k->parties) return PB200_ERR_INVALID_ARG;
+    USE_DEVICE(k);
+    CU(cudaStreamSynchronize(k->stream));
+    const BigInt e = BigInt::mul(BigInt::shl(k->delta, 1), BigInt::from_u64_le(s_le, k->words_out));      // 2 Delta s
+    const uint32_t ew = e.bits() ? (uint32_t)PB200_WORDS(e.bits()) : 1;
+    std::vector<u64> words(ew);
+    e.to_u64_le(words.data(), ew);
+    k->has_share = false;
+    if (k->d_share_e) { cudaFree(k->d_share_e); k->d_share_e = nullptr; }
+    CU(cudaMalloc(&k->d_share_e, ew * sizeof(u64)));
+    CU(cudaMemcpyAsync(k->d_share_e, words.data(), ew * sizeof(u64), cudaMemcpyHostToDevice, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    k->share_e_bits = (int)e.bits();
+    if (k->fast) CU(block28_pow_prepare(k->fast, POW_SHARE, e, k->stream));
+    k->has_share = true;
+    return PB200_OK;
+} PB200_CATCH
+
+int pb200_partial_decrypt_batch_dev(pb200_key* k, const uint64_t* d_c, size_t count, uint64_t* d_out) try {
+    if (!k || (count && (!d_c || !d_out))) return PB200_ERR_INVALID_ARG;
+    if (!k->has_share) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    USE_DEVICE(k);
+    if (use_fast(k)) CU(block28_pow(k->fast, POW_SHARE, (const u64*)d_c, (int)k->words_out, count, (u64*)d_out, k->stream));
+    else CU(simple_pow(k->d_simple, (const u64*)d_c, (int)k->words_out, k->d_share_e, k->share_e_bits, 0, count, (u64*)d_out, k->d_flags, k->stream,
+                       true));
+    return PB200_OK;
+} PB200_CATCH
+int pb200_partial_decrypt_batch(pb200_key* k, const uint64_t* c, size_t count, uint64_t* out) try {
+    if (!k || (count && (!c || !out))) return PB200_ERR_INVALID_ARG;
+    if (!k->has_share) return PB200_ERR_INVALID_ARG;
+    if (!count) return PB200_OK;
+    USE_DEVICE(k);
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bc = count * k->words_out * sizeof(u64);
+    CU(k->in_a.reserve(bc)); CU(k->out_a.reserve(bc));
+    CU(cudaMemcpyAsync(k->in_a.p, c, bc, cudaMemcpyHostToDevice, k->stream));
+    int rc = pb200_partial_decrypt_batch_dev(k, (const uint64_t*)k->in_a.p, count, (uint64_t*)k->out_a.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out, k->out_a.p, bc, cudaMemcpyDeviceToHost, k->stream));
+    CU(cudaStreamSynchronize(k->stream));
+    return take_flags(k);
+} PB200_CATCH
+
+// The combination plan of an index set (in the order given): the Lagrange exponents 2 |mu_j|, mu_j = Delta prod_(j' != j) j' / (j' - j),
+// whose magnitude is the exact quotient Delta prod j' / prod |j' - j| and whose sign is the parity of the j' < j.  Plans are cached per
+// index set, so a _dev call on a known set enqueues without a synchronise; PB200_ERR_INVALID_ARG for a bad set.
+static const size_t COMBINE_PLANS = 64;
+static int combine_plan(pb200_key* k, const uint32_t* idx, uint32_t kk, pb200_key::Combine** out) {
+    if (k->parties == 0 || kk == 0 || kk > k->parties) return PB200_ERR_INVALID_ARG;
+    std::vector<uint32_t> set(idx, idx + kk);
+    for (uint32_t a = 0; a < kk; a++) {
+        if (set[a] < 1 || set[a] > k->parties) return PB200_ERR_INVALID_ARG;
+        for (uint32_t b = 0; b < a; b++) if (set[a] == set[b]) return PB200_ERR_INVALID_ARG;
+    }
+    auto it = k->combine.find(set);
+    if (it != k->combine.end()) { *out = &it->second; return PB200_OK; }
+    std::vector<BigInt> e(kk);
+    std::vector<bool> neg(kk);
+    for (uint32_t a = 0; a < kk; a++) {
+        BigInt num = k->delta, den(1);
+        int below = 0;
+        for (uint32_t b = 0; b < kk; b++) {
+            if (b == a) continue;
+            num = BigInt::mul(num, BigInt(set[b]));
+            den = BigInt::mul(den, BigInt(set[b] > set[a] ? set[b] - set[a] : set[a] - set[b]));
+            below += set[b] < set[a];
+        }
+        BigInt q, r;
+        BigInt::divmod(num, den, q, r);
+        if (!r.is_zero()) throw std::runtime_error("Lagrange coefficient is not an integer");
+        e[a] = BigInt::shl(q, 1);
+        neg[a] = below & 1;
+    }
+    bool any_neg = false;
+    for (uint32_t a = 0; a < kk; a++) any_neg |= neg[a];
+    if (any_neg && !k->n.is_odd()) return PB200_ERR_EVEN_MODULUS;
+    pb200_key::Combine P;
+    struct Guard { pb200_key::Combine* p; ~Guard() { if (p) p->release(); } } guard{&P};      // released unless it joins the cache
+    P.any_neg = any_neg;
+    P.is_neg = neg;
+    if (any_neg) { int rc = ensure_inverse(k); if (rc) return rc; }
+    if (k->fast) {
+        std::vector<BigInt> ep, en;
+        std::vector<int> pp, pn;
+        for (uint32_t a = 0; a < kk; a++) { (neg[a] ? en : ep).push_back(e[a]); (neg[a] ? pn : pp).push_back((int)a); }
+        if (!ep.empty()) CU(block28_multipow_prepare(ep, pp, &P.pos, k->stream));
+        if (!en.empty()) CU(block28_multipow_prepare(en, pn, &P.neg, k->stream));
+    }
+    size_t bits = 1;
+    for (const BigInt& v : e) bits = std::max(bits, v.bits());
+    P.ew = (int)PB200_WORDS(bits);
+    P.e_words.assign((size_t)kk * P.ew, 0);
+    for (uint32_t a = 0; a < kk; a++) {
+        e[a].to_u64_le(P.e_words.data() + (size_t)a * P.ew, P.ew);
+        P.e_bits.push_back((int)e[a].bits());
+    }
+    CU(cudaMalloc(&P.d_e, P.e_words.size() * sizeof(u64)));
+    CU(cudaMemcpyAsync(P.d_e, P.e_words.data(), P.e_words.size() * sizeof(u64), cudaMemcpyHostToDevice, k->stream));
+    if (k->combine.size() >= COMBINE_PLANS) drop_combine_plans(k);
+    guard.p = nullptr;
+    *out = &(k->combine[set] = std::move(P));
+    return PB200_OK;
+}
+
+// m = L(P N^-1 mod n^2) phi mod n with P / N the products of the shares' positive / negative Lagrange powers: k_multipow once per sign
+// on a block28 key, else simple_pow per share folded with simple_add; the inverse only when some coefficient is negative
+static int combine_dev_impl(pb200_key* k, pb200_key::Combine& P, uint32_t kk, const u64* d_shares, size_t count, u64* d_m) {
+    const size_t wo = k->words_out, bytes = count * wo * sizeof(u64);
+    CU(k->th_p.reserve(bytes)); CU(k->th_n.reserve(bytes)); CU(k->th_x.reserve(bytes));
+    u64 *dp = (u64*)k->th_p.p, *dn = (u64*)k->th_n.p, *dx = (u64*)k->th_x.p;
+    if (use_fast(k)) {
+        if (P.pos.k) CU(block28_multipow(k->fast, P.pos, d_shares, count, count, dp, k->stream));
+        if (P.neg.k) CU(block28_multipow(k->fast, P.neg, d_shares, count, count, dn, k->stream));
+    } else {
+        bool first[2] = {true, true};
+        for (uint32_t a = 0; a < kk; a++) {
+            const bool ng = P.is_neg[a];
+            u64* acc = ng ? dn : dp;
+            u64* dst = first[ng] ? acc : dx;
+            CU(simple_pow(k->d_simple, d_shares + (size_t)a * count * wo, (int)wo, P.d_e + (size_t)a * P.ew, P.e_bits[a], 0, count,
+                          dst, k->d_flags, k->stream, true));
+            if (!first[ng]) CU(simple_add(k->d_simple, acc, dx, (int)wo, count, acc, nullptr, k->d_flags, k->stream));
+            first[ng] = false;
+        }
+    }
+    const u64* x = dp;
+    if (P.any_neg) {
+        int rc = inverse_dev_impl(k, dn, dp, nullptr, nullptr, 0, count, dx); if (rc) return rc;
+        x = dx;
+    }
+    CU(simple_lfunc(k->d_simple_phi, x, count, d_m, k->d_flags, k->stream));
+    return PB200_OK;
+}
+int pb200_combine_shares_batch_dev(pb200_key* k, const uint32_t* indices, uint32_t kk, const uint64_t* d_shares, size_t count, uint64_t* d_m) try {
+    if (!k || !indices || (count && (!d_shares || !d_m))) return PB200_ERR_INVALID_ARG;
+    USE_DEVICE(k);
+    pb200_key::Combine* P = nullptr;
+    int rc = combine_plan(k, indices, kk, &P); if (rc) return rc;
+    if (!count) return PB200_OK;
+    return combine_dev_impl(k, *P, kk, (const u64*)d_shares, count, (u64*)d_m);
+} PB200_CATCH
+int pb200_combine_shares_batch(pb200_key* k, const uint32_t* indices, uint32_t kk, const uint64_t* shares, size_t count, uint64_t* m_out) try {
+    if (!k || !indices || (count && (!shares || !m_out))) return PB200_ERR_INVALID_ARG;
+    USE_DEVICE(k);
+    pb200_key::Combine* P = nullptr;
+    int rc = combine_plan(k, indices, kk, &P); if (rc) return rc;
+    if (!count) return PB200_OK;
+    { int rc0_ = clear_flags(k); if (rc0_) return rc0_; }
+    const size_t bin = (size_t)kk * count * k->words_out * sizeof(u64), bout = count * k->words_in * sizeof(u64);
+    CU(k->in_a.reserve(bin)); CU(k->out_a.reserve(bout));
+    CU(cudaMemcpyAsync(k->in_a.p, shares, bin, cudaMemcpyHostToDevice, k->stream));
+    rc = combine_dev_impl(k, *P, kk, (const u64*)k->in_a.p, count, (u64*)k->out_a.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(m_out, k->out_a.p, bout, cudaMemcpyDeviceToHost, k->stream));
     CU(cudaStreamSynchronize(k->stream));
     return take_flags(k);
 } PB200_CATCH

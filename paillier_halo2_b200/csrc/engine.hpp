@@ -30,9 +30,9 @@ cudaError_t repack_limbs(const u64* d_vals, size_t count, int words_per_value, i
 // decryption pieces on the simple engine: x = base^e mod n^2 (exponent words on the device), and m = (x - 1) / n * mu mod n with
 // the constants of the modulus n (mu in their g slot); flag bit 3 when x != 1 (mod n).  e_stride = 0: one exponent for every unit
 // (decryption's lambda); e_stride > 0: unit u's exponent starts at word u * e_stride, and the base is reduced mod n^2 first (scalar
-// multiplication accepts any words_out-word value)
+// multiplication accepts any words_out-word value); reduce: the base is reduced with e_stride = 0 too (partial decryption)
 cudaError_t simple_pow(const SimpleConsts* dK, const u64* d_base, int base_words, const u64* d_e, int e_bits, int e_stride, size_t count,
-                       u64* d_out, int* d_flags, cudaStream_t st);
+                       u64* d_out, int* d_flags, cudaStream_t st, bool reduce = false);
 cudaError_t simple_lfunc(const SimpleConsts* dKn, const u64* d_x, size_t count, u64* d_m, int* d_flags, cudaStream_t st);
 
 // ---- inverse mod n^2 (inverse_kernels.cu): safegcd mod n, then one Hensel step --------------------------------------------
@@ -79,9 +79,24 @@ bool block28_has_engine(const Block28Key*, int eng);
 void block28_chain_counts(const Block28Key*, uint64_t* n_sqr, uint64_t* n_mul);
 cudaError_t block28_encrypt(Block28Key*, const u64* d_m, const u64* d_r, size_t count, u64* d_c, cudaStream_t st);
 cudaError_t block28_tally(Block28Key*, const u64* d_c, size_t count, u64* d_out, cudaStream_t st);
-// out = base^e mod n^2 for a per-key exponent e (sliding-window schedule built by block28_pow_prepare): the decryption's c^lambda
-cudaError_t block28_pow_prepare(Block28Key*, const BigInt& e, cudaStream_t st);
-cudaError_t block28_pow(Block28Key*, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st);
+// out = base^e mod n^2 for a per-key exponent e (sliding-window schedule built by block28_pow_prepare), one schedule per slot:
+// POW_LAMBDA the decryption's c^lambda, POW_SHARE a trustee's partial decryption c^(2 Delta s_i)
+enum { POW_LAMBDA = 0, POW_SHARE = 1, POW_SLOTS = 2 };
+cudaError_t block28_pow_prepare(Block28Key*, int slot, const BigInt& e, cudaStream_t st);
+cudaError_t block28_pow(Block28Key*, int slot, const u64* d_base, int base_words, size_t count, u64* d_out, cudaStream_t st);
+// out_u = prod_j b_(j, u)^(e_j) mod n^2 for k <= 32 exponents shared by the batch (k_multipow, Straus): b_(j, u) at d_base +
+// (pos[j] * stride + u) * words_out.  block28_multipow_prepare builds the merged schedule and uploads it on st; the plan (and its
+// host copy of the schedule) must live until st has run every launch that uses it.
+struct MultiPow {
+    int k = 0, h = 0, first_idx = -1;   // bases, odd powers per base (2^(w - 1)), first table entry of the chain
+    std::vector<int> pos;               // share position of each base
+    std::vector<int2> ops;              // (squarings, table entry or -1), as PowSched
+    int2* d_ops = nullptr; int* d_pos = nullptr;
+    uint64_t n_sqr = 0, n_mul = 0;      // squarings / multiplications per unit (table and chain)
+};
+cudaError_t block28_multipow_prepare(const std::vector<BigInt>& e, const std::vector<int>& pos, MultiPow* P, cudaStream_t st);
+void block28_multipow_free(MultiPow* P);
+cudaError_t block28_multipow(Block28Key*, const MultiPow& P, const u64* d_base, size_t stride, size_t count, u64* d_out, cudaStream_t st);
 // out_i = c_i^(k_i) mod n^2 with a scalar per unit (PB200_WORDS(k_bits) words each; c_i: words_out words, any value): fixed-window
 // chain per lane, window width chosen from k_bits; no per-key preparation
 cudaError_t block28_scalar(Block28Key*, const u64* d_c, const u64* d_k, uint32_t k_bits, size_t count, u64* d_out, cudaStream_t st);

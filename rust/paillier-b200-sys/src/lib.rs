@@ -125,6 +125,14 @@ extern "C" {
                                          out_le: *mut u64) -> c_int;
     pub fn pb200_scalar_mul_signed_batch_dev(key: *mut pb200_key, d_c_le: *const u64, d_k_mag_le: *const u64, d_k_neg: *const u8, k_bits: u32,
                                              count: usize, d_out_le: *mut u64) -> c_int;
+    pub fn pb200_key_set_threshold(key: *mut pb200_key, parties: u32, phi_le: *const u64) -> c_int;
+    pub fn pb200_key_set_share(key: *mut pb200_key, index: u32, s_le: *const u64) -> c_int;
+    pub fn pb200_partial_decrypt_batch(key: *mut pb200_key, c_le: *const u64, count: usize, out_le: *mut u64) -> c_int;
+    pub fn pb200_partial_decrypt_batch_dev(key: *mut pb200_key, d_c_le: *const u64, count: usize, d_out_le: *mut u64) -> c_int;
+    pub fn pb200_combine_shares_batch(key: *mut pb200_key, indices: *const u32, k: u32, shares_le: *const u64, count: usize,
+                                      m_out_le: *mut u64) -> c_int;
+    pub fn pb200_combine_shares_batch_dev(key: *mut pb200_key, indices: *const u32, k: u32, d_shares_le: *const u64, count: usize,
+                                          d_m_out_le: *mut u64) -> c_int;
     pub fn pb200_matvec(key: *mut pb200_key, c_le: *const u64, count: usize, w_mag_le: *const u64, w_neg: *const u8, k_bits: u32, rows: usize,
                         out_le: *mut u64) -> c_int;
     pub fn pb200_matvec_dev(key: *mut pb200_key, d_c_le: *const u64, count: usize, d_w_mag_le: *const u64, d_w_neg: *const u8, k_bits: u32,
@@ -275,6 +283,50 @@ impl Key {
         let mut out = vec![0u64; c.len()];
         let neg = if k_neg.is_empty() { std::ptr::null() } else { k_neg.as_ptr() };
         let rc = unsafe { pb200_scalar_mul_signed_batch(self.raw, c.as_ptr(), k_mag.as_ptr(), neg, k_bits, c.len() / wo, out.as_mut_ptr()) };
+        if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// threshold decryption: `parties` trustees (1 ..= 32) and phi = L(g^(4 Delta^2 d) mod n^2)^-1 mod n (`words_in` words); clears
+    /// any share set on this key
+    pub fn set_threshold(&mut self, parties: u32, phi: &[u64]) -> Result<(), i32> {
+        if phi.len() != self.words_in() {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let rc = unsafe { pb200_key_set_threshold(self.raw, parties, phi.as_ptr()) };
+        if rc == PB200_OK { Ok(()) } else { Err(rc) }
+    }
+
+    /// this key's trustee: `index` (1 ..= parties) and its share s_index (`words_out` words)
+    pub fn set_share(&mut self, index: u32, share: &[u64]) -> Result<(), i32> {
+        if share.len() != self.words_out() {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let rc = unsafe { pb200_key_set_share(self.raw, index, share.as_ptr()) };
+        if rc == PB200_OK { Ok(()) } else { Err(rc) }
+    }
+
+    /// the trustee's partial decryptions c_i^(2 Delta s) mod n^2 of `count * words_out` words of ciphertexts
+    pub fn partial_decrypt_batch(&mut self, c: &[u64]) -> Result<Vec<u64>, i32> {
+        let wo = self.words_out();
+        if wo == 0 || c.len() % wo != 0 {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let mut out = vec![0u64; c.len()];
+        let rc = unsafe { pb200_partial_decrypt_batch(self.raw, c.as_ptr(), c.len() / wo, out.as_mut_ptr()) };
+        if rc == PB200_OK { Ok(out) } else { Err(rc) }
+    }
+
+    /// combination of the partial decryptions of the trustees `indices`: `shares` share-major (share j of ciphertext u at
+    /// `(j * count + u) * words_out`); returns `count * words_in` words of plaintexts.  `Err(PB200_ERR_DECRYPT)` when too few or wrong
+    /// shares leave some unit without an exact L (`PB200_ERR_NOT_INVERTIBLE` when its N has no inverse)
+    pub fn combine_shares_batch(&mut self, indices: &[u32], shares: &[u64]) -> Result<Vec<u64>, i32> {
+        let (wo, k) = (self.words_out(), indices.len());
+        if wo == 0 || k == 0 || shares.len() % (k * wo) != 0 {
+            return Err(PB200_ERR_INVALID_ARG);
+        }
+        let count = shares.len() / (k * wo);
+        let mut out = vec![0u64; count * self.words_in()];
+        let rc = unsafe { pb200_combine_shares_batch(self.raw, indices.as_ptr(), k as u32, shares.as_ptr(), count, out.as_mut_ptr()) };
         if rc == PB200_OK { Ok(out) } else { Err(rc) }
     }
 
